@@ -147,16 +147,14 @@ def run_reference(args, rank, world):
     sample = 48  # bounded sample: the first 48 frames of the C2 sequence, replayed
     s = Synth(SCENARIO, 2)
     frames = [s.frame(f) for f in range(sample)]
-    # keep the whole arm within a few minutes: the oracle needs ~0.1-0.3 s per frame on this sample
-    K_eff = min(K, 150)
+    # K timed steps after W untimed ones, in both figures; the oracle needs ~0.1-0.3 s per frame on this sample
     t_single = [0.0]
-    _oracle_worker(orc, frames, s.max_points, K_eff, min(W, 5), sample, t_single, 0, None)
-    value = K_eff / t_single[0]
+    _oracle_worker(orc, frames, s.max_points, K, W, sample, t_single, 0, None)
+    value = K / t_single[0]
     threads = max(1, min(os.cpu_count() or 1, 64))
-    K_all = min(K, sample)
     t_all = [0.0] * threads
     barrier = threading.Barrier(threads + 1)
-    ths = [threading.Thread(target=_oracle_worker, args=(orc, frames, s.max_points, K_all, 2, sample, t_all, t, barrier)) for t in range(threads)]
+    ths = [threading.Thread(target=_oracle_worker, args=(orc, frames, s.max_points, K, W, sample, t_all, t, barrier)) for t in range(threads)]
     for t in ths:
         t.start()
     barrier.wait()
@@ -165,17 +163,17 @@ def run_reference(args, rank, world):
     dt = time.perf_counter() - t0
     for t in ths:
         t.join()
-    all_cores = threads * K_all / dt
+    all_cores = threads * K / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": "frames/s", "n_gpus": world, "steps": K, "warmup": W,
-        "ms_per_step": 1e3 * t_single[0] / K_eff, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
+        "ms_per_step": 1e3 * t_single[0] / K, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": bench_config(world),
-        "reference_arm": {"timed_steps": K_eff, "note": "one sequence, one thread: the reference path is single-threaded per sensor stream"},
+        "reference_arm": {"timed_steps": K, "note": "one sequence, one thread: the reference path is single-threaded per sensor stream"},
         "cpu_baseline": {"value": value, "unit": "frames/s", "cores": 1, "kind": "port",
-                         "sample": f"{K_eff} frames replaying the first {sample} frames of C2, CPU oracle (PCL-semantics restatement, g++ -O2)",
+                         "sample": f"{K} frames replaying the first {sample} frames of C2, CPU oracle (PCL-semantics restatement, g++ -O2)",
                          "host_cpus": os.cpu_count()},
         "all_cores": {"value": all_cores, "unit": "frames/s", "cores": threads,
-                      "sample": f"{threads} independent sequences (one per host thread), {K_all} frames each from the same {sample}-frame sample"},
+                      "sample": f"{threads} independent sequences (one per host thread), {K} frames each from the same {sample}-frame sample"},
         "e2e": {"value": value, "unit": "frames/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }
     print(json.dumps(line), flush=True)
@@ -342,10 +340,10 @@ def run_product(args, rank, local_rank, world):
             assert b.device_download(local_rank, last.ctypes.data_as(C.c_void_p), C.c_void_p(mm.output_device()), last.nbytes) == 0
         crc_last = zlib.crc32(last.tobytes())
         mm.close()
-        return ms, n_launches, crc_last
+        return ms, n_launches, crc_last, last
 
-    one_ms, one_launches, crc_one_last = device_resident(False)   # one kernel per frame: k_frame
-    dev_ms, launches, crc_dev_last = device_resident(True)        # the headline: k_frame_pipe
+    one_ms, one_launches, crc_one_last, _ = device_resident(False)        # one kernel per frame: k_frame
+    dev_ms, launches, crc_dev_last, dev_last = device_resident(True)      # the headline: k_frame_pipe
     launches_all = sum_over_ranks(launches)
 
     # ------------------------------------------------------------------ multi-sequence (C5-style): S independent sequences per GPU
@@ -409,14 +407,13 @@ def run_product(args, rank, local_rank, world):
     if Se > 1:
         hs2 = [MovingObjectRemoval(CFG, 4, 3, device=local_rank, binding=b, max_points=maxp) for _ in range(Se)]
         outs2 = [pinned_array(b, (maxp, 8), np.float32) for _ in range(Se)]
-        Ke = max(20, K // 2)
         offs2 = [(si * F) // Se for si in range(Se)]
         gate = threading.Barrier(Se + 1)
 
         def drive(si):
             hh3, outp = hs2[si].h, C.c_void_p(outs2[si][0].ctypes.data)
             no = C.c_uint32(0)
-            for phase, cnt in (("warm", 5), ("timed", Ke)):
+            for phase, cnt in (("warm", 5), ("timed", K)):
                 if phase == "timed":
                     gate.wait()
                 for t in range(cnt):
@@ -435,7 +432,7 @@ def run_product(args, rank, local_rank, world):
         for th in ths:
             th.join()
         dt = max_over_ranks(dt)
-        multi_e2e = {"sequences_per_gpu": Se, "value": world * Se * Ke / dt, "unit": "frames/s",
+        multi_e2e = {"sequences_per_gpu": Se, "value": world * Se * K / dt, "unit": "frames/s",
                      "note": "host C ABI, one host thread + stream per sequence, pinned buffers, H2D and D2H inside; wall clock over all sequences"}
         for hh3 in hs2:
             hh3.close()
@@ -448,17 +445,16 @@ def run_product(args, rank, local_rank, world):
     frame_bytes_alg = 0.0
     if rank == 0:
         peak, which = measured_peak_gbs()
-        prof_frames = min(F, 64)
-        w0 = min(W, prof_frames)
+        # both passes time frames W .. F - 1, the K frames of the timed legs
         # pass 1: the fused kernel, one pair of CUDA events around every launch
         m2 = MovingObjectRemoval(CFG, 4, 3, device=local_rank, binding=b, max_points=maxp)
         m2.set_timing(True)
         kern_ms, alg_sum, nc_sum, nprof = 0.0, 0, 0, 0
         timeline = {}
-        for f in range(prof_frames):
+        for f in range(F):
             m2.push_device(d_frames.value + f * frame_bytes, int(npts[f]), poses[f])
             m2.filter_device(None, 0, want_count=True)
-            if f >= w0:
+            if f >= W:
                 kern_ms += m2.last_device_ms()[0]
                 for k, v in m2.phase_times().items():
                     timeline[k] = timeline.get(k, 0.0) + v
@@ -490,11 +486,11 @@ def run_product(args, rank, local_rank, world):
                                             "frac": frame_bytes_alg / (kern_us * 1e-6) / 1e9 / peak, "traffic": traffic}}
         # pass 2: one launch per phase (the same device functions), each between events
         m2 = MovingObjectRemoval(CFG, 4, 3, device=local_rank, binding=b, max_points=maxp)
-        for f in range(w0):
+        for f in range(W):
             m2.push_device(d_frames.value + f * frame_bytes, int(npts[f]), poses[f])
             m2.filter_device(None, 0, want_count=True)
         m2.set_kernel_profiling(True)
-        for f in range(w0, prof_frames):
+        for f in range(W, F):
             m2.push_device(d_frames.value + f * frame_bytes, int(npts[f]), poses[f])
             m2.filter_device(None, 0, want_count=True)
         prof = m2.kernel_profile()
@@ -514,36 +510,34 @@ def run_product(args, rank, local_rank, world):
         orc = MorBinding(C.CDLL(str(ROOT / "oracle" / "libmor_oracle.so")), "oracle_")
         mo = MovingObjectRemoval(CFG, 4, 3, binding=orc)
         out_o = np.empty((maxp, 8), np.float32)
-        budget, t_used, nf = 20.0, 0.0, 0
+        t_used = 0.0
         crcs_o = []
         for f in range(F):
             t0 = time.perf_counter()
             mo.push_raw_cloud_and_pose(pts[f, : npts[f]], poses[f])
             oo = mo.filter_cloud(out_o)
-            t_used += time.perf_counter() - t0
+            if f >= W:
+                t_used += time.perf_counter() - t0
             crcs_o.append((zlib.crc32(oo.tobytes()), zlib.crc32(mo.tap("removed_mask").tobytes())))
-            nf += 1
-            if t_used > budget:
-                break
-        cpu = {"value": nf / t_used, "unit": "frames/s", "cores": 1, "kind": "port",
-               "sample": f"first {nf} frames of the same C2 sequence, single thread, CPU oracle (PCL-semantics restatement, -O2)", "host_cpus": os.cpu_count()}
+        cpu = {"value": K / t_used, "unit": "frames/s", "cores": 1, "kind": "port",
+               "sample": f"frames {W}..{F - 1} of the same C2 sequence ({K} timed steps after {W} untimed), single thread, CPU oracle (PCL-semantics restatement, -O2)",
+               "host_cpus": os.cpu_count()}
         # the same frames through the product, untimed: output cloud and removal mask of every frame against the oracle's
         mg = MovingObjectRemoval(CFG, 4, 3, device=local_rank, binding=b, max_points=maxp)
         equal = 0
         first_bad = None
-        for f in range(nf):
+        for f in range(F):
             mg.push_raw_cloud_and_pose(pts[f, : npts[f]], poses[f])
             og = mg.filter_cloud(out_host)
             ok = (zlib.crc32(og.tobytes()), zlib.crc32(mg.tap("removed_mask").tobytes())) == crcs_o[f]
             equal += 1 if ok else 0
             if not ok and first_bad is None:
                 first_bad = f
-        spot = {"frames": nf, "crc_equal": equal == nf, "frames_equal": equal, "first_mismatch": first_bad,
+        spot = {"frames": F, "crc_equal": equal == F, "frames_equal": equal, "first_mismatch": first_bad,
                 "what": "crc32 of the filtered cloud bytes and of the removed-point mask, product vs oracle, frame by frame from the start of the timed sequence",
                 "timed_run_last_frame_crc_equal": crc_dev_last == crc_e2e_last,
-                "timed_run_note": "last output of the device-resident timed run == last output of the end-to-end timed run (two independent full passes)"}
-        if nf == F:
-            spot["timed_run_last_frame_equals_oracle"] = crcs_o[-1][0] == crc_dev_last
+                "timed_run_note": "last output of the device-resident timed run == last output of the end-to-end timed run (two independent full passes)",
+                "timed_run_last_frame_equals_oracle": crcs_o[-1][0] == crc_dev_last}
         mg.close()
         # north_star: "any tie-breaking divergence at the exact clustering radius counted and reported": point pairs within
         # 2 ulps of r^2 (the pairs a differently rounded distance or a pruned kd-tree search could classify the other way),
@@ -571,7 +565,8 @@ def run_product(args, rank, local_rank, world):
         import re
         import subprocess
         try:
-            r = subprocess.run([str(harness), str(CFG), "2", "2", "60", "--quiet"], capture_output=True, text=True, timeout=300,
+            # the harness leaves its first 5 callbacks out of its summary: 5 + K frames = K timed callbacks
+            r = subprocess.run([str(harness), str(CFG), "2", "2", str(5 + K), "--quiet"], capture_output=True, text=True, timeout=300,
                                env=dict(os.environ, CUDA_VISIBLE_DEVICES=str(local_rank)))
             m1 = re.search(r"summary frames (\d+) mean_ms ([\d.]+) p50_ms ([\d.]+) p99_ms ([\d.]+) fps ([\d.]+)", r.stdout)
             m2 = re.search(r"stages copy_ms ([\d.]+) push_ms ([\d.]+) filter_ms ([\d.]+)", r.stdout)
@@ -625,6 +620,12 @@ def run_product(args, rank, local_rank, world):
         "parity_spot_check": spot,
         "host": {"staged_frames": F, "staged_mb": F * frame_bytes / 1e6, "rank_cores": cores},
     }
+    if args.dump_outputs:
+        # what a caller of the headline path receives for its last timed frame (frame W + K - 1 of seed 2): the filtered
+        # cloud, float32 [n_out, 8] PointXYZI wire records (x, y, z, 1, intensity, 0, 0, 0); at most 133,312 x 32 B
+        out_dir = Path(args.dump_outputs)
+        out_dir.mkdir(parents=True, exist_ok=True)
+        np.save(out_dir / "filtered_cloud.npy", dev_last)
     print(json.dumps(line), flush=True)
 
 
@@ -714,14 +715,18 @@ def run_c5(b, local_rank, rank, world, per_gpu, T, S, maxp, max_over_ranks, sum_
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200, help="timed steps (frames per sequence) of every leg on the C2 workload; the C5 leg keeps its 32 frames per sequence")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--e2e-sequences", type=int, default=8, help="sequences (= host threads) of the multi-sequence end-to-end figure (1 = skip)")
     ap.add_argument("--sequences", type=int, default=37, help="independent sequences per launch for the multi_sequence figure and the batches of the C5 leg (37 = a group of 4 CTAs per sequence on 148 SMs; 1 = skip)")
     ap.add_argument("--c5-sequences", type=int, default=128, help="BASELINE config 5: sequences per GPU (128 x 8 GPUs = the full 1024), 32 frames each (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the headline path's output of its last step as DIR/filtered_cloud.npy "
+                                                          "(rank 0; the inputs depend on --steps and --warmup only)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
