@@ -94,8 +94,9 @@ struct mor_handle {
     cudaStream_t stream = nullptr;
     uint32_t spec_out = 0;        // speculative size of the output D2H copy (points), from the previous frame
     cudaStream_t last_stream = nullptr;  // stream that carries this handle's latest work (differs after a batched step)
-    // batched stepping (this handle as the leader of a batch): device array of per-sequence arguments + pinned ring
-    FramePtrs* d_batch = nullptr; FramePtrs* h_batch = nullptr; uint32_t batch_cap = 0; int batch_slot = 0;
+    // batched stepping (this handle as the leader of a batch): device array of per-sequence arguments + pinned ring; a slot
+    // holds S FramePtrs followed by S GroundPtrs (the latter used by the voxel ground modes only)
+    uint8_t* d_batch = nullptr; uint8_t* h_batch = nullptr; uint32_t batch_cap = 0; int batch_slot = 0;
     cudaEvent_t batch_ev[4] = {nullptr, nullptr, nullptr, nullptr};
     uint32_t nmax = 0, kmax = 0, momax = 0;
     int ring_depth = 0, pde_ring = 0;
@@ -500,6 +501,32 @@ int enqueue_push(mor_handle* h, const uint8_t* d_points, uint32_t n, uint32_t st
     return MOR_OK;
 }
 
+// The voxel ground stage of mor_batch_step_device: the nine kernels of enqueue_push, each launched once for all S
+// sequences (blockIdx.y = sequence, arguments P[s] / GP[s]). The point-indexed stages are sized for the largest frame
+// of the batch; the strided stages share the num_sms * 8 blocks of one single-handle launch among the sequences (C4 on
+// B200: as fast as or faster than 2, 8 or 16 blocks per sequence at S = 1 ... 37).
+int enqueue_ground_batch(mor_handle* h, const FramePtrs* P, const GroundPtrs* GP, uint32_t S, uint32_t n_max) {
+    cudaStream_t st = h->stream;
+    const dim3 pts(blocks_for(n_max), S), strided(((unsigned)h->num_sms * 8 + S - 1) / S, S), single(1, S);
+#define MOR_GLAUNCH(kernel, grid, block)                                                                                \
+    do {                                                                                                               \
+        cudaError_t le__ = launch_pdl(kernel, grid, dim3(block), 0, st, P, GP);                                        \
+        if (le__ != cudaSuccess) { h->last_error = std::string(#kernel) + ": " + cudaGetErrorString(le__); return MOR_ERR_CUDA; } \
+        h->launches++;                                                                                                 \
+    } while (0)
+    MOR_GLAUNCH(k_ingest_raw_batch, pts, kBlock);
+    MOR_GLAUNCH(k_ground_keys_batch, pts, kBlock);
+    MOR_GLAUNCH(k_scan_cells_batch, strided, kBlock);
+    MOR_GLAUNCH(k_scan_voxels_batch, strided, kBlock);
+    MOR_GLAUNCH(k_ground_scatter_batch, pts, kBlock);
+    MOR_GLAUNCH(k_voxel_eval_batch, strided, kBlock);
+    MOR_GLAUNCH(k_ground_mode_batch, single, kSingle);
+    MOR_GLAUNCH(k_ground_mark_batch, strided, kBlock);
+    MOR_GLAUNCH(k_ground_partition_batch, pts, kBlock);
+#undef MOR_GLAUNCH
+    return MOR_OK;
+}
+
 // ca = cb; cb = new frame (cpp:520-521), pose delta cb.ps^-1 * ca.ps (cpp:536)
 void advance_frame(mor_handle* h, uint32_t n, const double pose7[7]) {
     if (h->have_cur) { h->cur = (h->cur + 1) % 3; h->fpar ^= 1; std::memcpy(h->prev_pose, h->cur_pose, sizeof(h->cur_pose)); h->have_prev = true; h->n_prev_input = h->n_input; }
@@ -753,20 +780,23 @@ int mor_batch_step_device(mor_handle* const* hs, uint32_t S, const void* const* 
             h->last_error = "batched handles must share device, limits, config and frame count";
             return MOR_ERR_ARG;
         }
-        if (g->cfg.ground_mode != MOR_GROUND_CROP) { h->last_error = "batched stepping supports ground_mode 0 only"; return MOR_ERR_ARG; }
         { int fs = flush_back(g); if (fs != MOR_OK) return fs; }
         if (n[s] > g->nmax || (!d_data[s] && n[s]) || !d_out[s]) return n[s] > g->nmax ? MOR_ERR_CAPACITY : MOR_ERR_ARG;
         for (uint32_t t = 0; t < s; t++) if (hs[t] == g) return MOR_ERR_ARG;
     }
+    const bool ground = h->cfg.ground_mode != MOR_GROUND_CROP;  // (shared by every handle: part of the config compared above)
+    if (ground && S > 65535u) { h->last_error = "the voxel ground modes batch at most 65535 sequences per step"; return MOR_ERR_ARG; }
     MOR_CUDA(cudaSetDevice(h->device));
     cudaStream_t st = h->stream;
+    static_assert(sizeof(FramePtrs) % alignof(GroundPtrs) == 0, "GroundPtrs follow the FramePtrs of a ring slot");
+    const size_t per_seq = sizeof(FramePtrs) + sizeof(GroundPtrs);
     if (S > h->batch_cap) {
         MOR_CUDA(cudaStreamSynchronize(st));
         if (h->d_batch) cudaFree(h->d_batch);
         if (h->h_batch) cudaFreeHost(h->h_batch);
         h->d_batch = nullptr; h->h_batch = nullptr; h->batch_cap = 0;
-        MOR_CUDA(cudaMalloc(&h->d_batch, sizeof(FramePtrs) * S * 4));
-        MOR_CUDA(cudaMallocHost(&h->h_batch, sizeof(FramePtrs) * S * 4));
+        MOR_CUDA(cudaMalloc(&h->d_batch, per_seq * S * 4));
+        MOR_CUDA(cudaMallocHost(&h->h_batch, per_seq * S * 4));
         for (auto& e : h->batch_ev) if (!e) MOR_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
         h->batch_cap = S;
     }
@@ -775,8 +805,11 @@ int mor_batch_step_device(mor_handle* const* hs, uint32_t S, const void* const* 
     const int slot = h->batch_slot;
     h->batch_slot = (slot + 1) & 3;
     MOR_CUDA(cudaEventSynchronize(h->batch_ev[slot]));
-    FramePtrs* hp = h->h_batch + (size_t)slot * h->batch_cap;
-    FramePtrs* dp = h->d_batch + (size_t)slot * h->batch_cap;
+    FramePtrs* hp = reinterpret_cast<FramePtrs*>(h->h_batch + (size_t)slot * per_seq * h->batch_cap);
+    FramePtrs* dp = reinterpret_cast<FramePtrs*>(h->d_batch + (size_t)slot * per_seq * h->batch_cap);
+    GroundPtrs* hg = reinterpret_cast<GroundPtrs*>(hp + S);
+    const GroundPtrs* dg = reinterpret_cast<const GroundPtrs*>(dp + S);
+    uint32_t n_max = 0;
     // G CTAs per sequence; the groups run side by side, a group that has more than one sequence steps them in turn
     int G = h->frame_ctas / (int)S;
     if (const char* env = std::getenv("MOR_BATCH_G")) { const int v = std::atoi(env); if (v > 0) G = v; }
@@ -796,10 +829,15 @@ int mor_batch_step_device(mor_handle* const* hs, uint32_t S, const void* const* 
         g->frame.out = (float4*)d_out[s];
         set_segments(g, g->frame, G);
         hp[s] = g->frame;
+        if (ground) { hg[s] = g->ground; n_max = n[s] > n_max ? n[s] : n_max; }
         g->last_stream = st;
     }
-    MOR_CUDA(cudaMemcpyAsync(dp, hp, sizeof(FramePtrs) * S, cudaMemcpyHostToDevice, st));
+    MOR_CUDA(cudaMemcpyAsync(dp, hp, (ground ? per_seq : sizeof(FramePtrs)) * S, cudaMemcpyHostToDevice, st));
     MOR_CUDA(cudaEventRecord(h->batch_ev[slot], st));
+    if (ground) {  // voxel-covariance ground removal of all S frames: 9 launches, then the frame kernel takes over
+        int gs = enqueue_ground_batch(h, dp, dg, S, n_max);
+        if (gs != MOR_OK) return gs;
+    }
     {
         cudaError_t e = launch_coop(k_frame_batch, (unsigned)(groups * G), h->frame_smem, st, (const FramePtrs*)dp, (int)S, G);
         h->launches++;

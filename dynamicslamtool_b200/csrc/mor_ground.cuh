@@ -38,14 +38,14 @@ struct GroundPtrs {
 // ===================================================================================== G1
 // fromPCLPointCloud2 + PassThrough x,y (cpp:94-102): stable compaction of the in-range points into
 // raw_cloud, bounding box of raw_cloud, resets of the per-frame ground state.
-__global__ void __launch_bounds__(kBlock) k_ingest_raw(FramePtrs a, GroundPtrs gp) {
-    pdl_prologue();
+// `nblocks` blocks take part (one tile each): blocks_for(a.n).
+__device__ __forceinline__ void ingest_raw(const FramePtrs& a, const GroundPtrs& gp, unsigned nblocks) {
     __shared__ int s_tile;
     if (threadIdx.x == 0) s_tile = atomicAdd(&a.scratch->ticket_ingest, 1);
     __syncthreads();
     const int tile = s_tile;
     const uint32_t i = (uint32_t)tile * kBlock + threadIdx.x;
-    const uint32_t stride = gridDim.x * kBlock;
+    const uint32_t stride = nblocks * kBlock;
     for (uint32_t t = i; t < 65536u; t += stride) gp.bin_hist[t] = 0;
     float x = 0.f, y = 0.f, z = 0.f, w = 0.f;
     bool in = false;
@@ -91,12 +91,15 @@ __global__ void __launch_bounds__(kBlock) k_ingest_raw(FramePtrs a, GroundPtrs g
         a.track->frames += 1;
     }
 }
+__global__ void __launch_bounds__(kBlock) k_ingest_raw(FramePtrs a, GroundPtrs gp) {
+    pdl_prologue();
+    ingest_raw(a, gp, gridDim.x);
+}
 
 // ===================================================================================== G2
 // Ball-query grid (cell edge leaf*(1+2^-10) over the raw bounding box) and VoxelGrid index of every raw
 // point; both histograms. Every block derives the two descriptors from the reduced box.
-__global__ void __launch_bounds__(kBlock) k_ground_keys(FramePtrs a, GroundPtrs gp) {
-    pdl_prologue();
+__device__ __forceinline__ void ground_keys(const FramePtrs& a, const GroundPtrs& gp, int block) {
     __shared__ GridDesc s_g;
     __shared__ VoxDesc s_v;
     const int nraw = a.counts[MOR_CNT_NT];
@@ -122,13 +125,13 @@ __global__ void __launch_bounds__(kBlock) k_ground_keys(FramePtrs a, GroundPtrs 
         g.ncells = g.nx * g.ny * g.nz;
         v.ncells = v.div[0] * v.div[1] * v.div[2];
         s_g = g; s_v = v;
-        if (blockIdx.x == 0) {
+        if (block == 0) {
             *gp.ggrid = g; *gp.vdesc = v;
             if (too_big) atomicOr(&a.counts[MOR_CNT_ERRFLAGS], ERR_GROUND_CAP);
         }
     }
     __syncthreads();
-    const int r = blockIdx.x * kBlock + threadIdx.x;
+    const int r = block * kBlock + threadIdx.x;
     if (r >= nraw) return;
     const float4 p = gp.rpts[r];
     const GridDesc& g = s_g;
@@ -146,6 +149,10 @@ __global__ void __launch_bounds__(kBlock) k_ground_keys(FramePtrs a, GroundPtrs 
     gp.vkey[r] = vk;
     atomicAdd(&gp.vox_count[vk], 1);
 }
+__global__ void __launch_bounds__(kBlock) k_ground_keys(FramePtrs a, GroundPtrs gp) {
+    pdl_prologue();
+    ground_keys(a, gp, blockIdx.x);
+}
 
 // ===================================================================================== G2b
 // Exclusive scan of the ball grid's per-cell histogram (counting sort of the cell keys) -> cell_start[0..ncells]. The
@@ -154,10 +161,8 @@ __global__ void __launch_bounds__(kBlock) k_ground_keys(FramePtrs a, GroundPtrs 
 // so the launch does not depend on the (device-side) cell count.
 constexpr int kScanItems = 8;
 constexpr int kScanTile = kBlock * kScanItems;
-__global__ void __launch_bounds__(kBlock) k_scan_cells(FramePtrs a) {
-    pdl_prologue();
+__device__ __forceinline__ void scan_cells(const FramePtrs& a, int ncells) {
     __shared__ int s_tile;
-    const int ncells = a.dgrid->ncells;
     const int ntiles = (ncells + kScanTile - 1) / kScanTile;
     while (true) {
         __syncthreads();
@@ -184,12 +189,15 @@ __global__ void __launch_bounds__(kBlock) k_scan_cells(FramePtrs a) {
         if (tile == ntiles - 1 && threadIdx.x == 0) a.cell_start[ncells] = before + total;
     }
 }
+__global__ void __launch_bounds__(kBlock) k_scan_cells(FramePtrs a) {
+    pdl_prologue();
+    scan_cells(a, a.dgrid->ncells);
+}
 
 // ===================================================================================== G3
 // Occupancy scan of the voxel histogram: ordinal of every occupied voxel in ascending voxel index (the
 // order pcl::VoxelGrid emits its centroids in), point count per ordinal, total number of voxels.
-__global__ void __launch_bounds__(kBlock) k_scan_voxels(FramePtrs a, GroundPtrs gp) {
-    pdl_prologue();
+__device__ __forceinline__ void scan_voxels(const FramePtrs& a, const GroundPtrs& gp) {
     __shared__ int s_tile;
     const int ncells = gp.vdesc->ncells;
     const int ntiles = (ncells + kTile - 1) / kTile;
@@ -225,12 +233,15 @@ __global__ void __launch_bounds__(kBlock) k_scan_voxels(FramePtrs a, GroundPtrs 
         if (tile == ntiles - 1 && threadIdx.x == 0) { gp.gstate[1] = before + total; a.counts[MOR_CNT_NVOX] = before + total; }
     }
 }
+__global__ void __launch_bounds__(kBlock) k_scan_voxels(FramePtrs a, GroundPtrs gp) {
+    pdl_prologue();
+    scan_voxels(a, gp);
+}
 
 // ===================================================================================== G4
 // Raw points into ball-grid order; exact fixed-point coordinate sums per voxel.
-__global__ void __launch_bounds__(kBlock) k_ground_scatter(FramePtrs a, GroundPtrs gp) {
-    pdl_prologue();
-    const int r = blockIdx.x * kBlock + threadIdx.x;
+__device__ __forceinline__ void ground_scatter(const FramePtrs& a, const GroundPtrs& gp, int block) {
+    const int r = block * kBlock + threadIdx.x;
     const int nraw = a.counts[MOR_CNT_NT];
     if ((r & ~31) >= nraw) return;  // whole warps stay for the group reductions
     const bool in = r < nraw;
@@ -262,6 +273,10 @@ __global__ void __launch_bounds__(kBlock) k_ground_scatter(FramePtrs a, GroundPt
             atomicAdd(gp.vacc + (size_t)ord * 6 + q * 2 + 1, (unsigned long long)sl);
         }
     }
+}
+__global__ void __launch_bounds__(kBlock) k_ground_scatter(FramePtrs a, GroundPtrs gp) {
+    pdl_prologue();
+    ground_scatter(a, gp, blockIdx.x);
 }
 
 // Closed-form smallest eigenpair of a symmetric PSD 3x3 matrix (trigonometric method), same operation order
@@ -397,21 +412,24 @@ __device__ __forceinline__ void voxel_eval_one(const FramePtrs& a, const GroundP
 }
 // The number of voxels is only known on the device (and is far below the number of points): a fixed grid of warps
 // strides over them instead of launching one warp per point's worth of blocks that would mostly exit.
-__global__ void __launch_bounds__(kBlock) k_voxel_eval(FramePtrs a, GroundPtrs gp) {
-    pdl_prologue();
+// Blocks [0, nblocks) of a grid of any size take part.
+__device__ __forceinline__ void voxel_eval(const FramePtrs& a, const GroundPtrs& gp, int block, int nblocks) {
     const int lane = threadIdx.x & 31;
-    const int nvox = gp.gstate[1], warps = (gridDim.x * kBlock) >> 5;
+    const int nvox = gp.gstate[1], warps = (nblocks * kBlock) >> 5;
     const GridDesc g = *gp.ggrid;
     // (consecutive voxels stay in one block on purpose: their balls overlap, so the block shares them in L1; spreading
     // the dense voxels near the sensor over the SMs instead was measured 30 % slower)
-    for (int v = (blockIdx.x * kBlock + threadIdx.x) >> 5; v < nvox; v += warps) voxel_eval_one(a, gp, g, v, lane);
+    for (int v = (block * kBlock + threadIdx.x) >> 5; v < nvox; v += warps) voxel_eval_one(a, gp, g, v, lane);
+}
+__global__ void __launch_bounds__(kBlock) k_voxel_eval(FramePtrs a, GroundPtrs gp) {
+    pdl_prologue();
+    voxel_eval(a, gp, blockIdx.x, gridDim.x);
 }
 
 // ===================================================================================== G6
 // Mode bin (cpp:169-178, tie => smallest key) and the selection threshold; resets the look-back state that the
 // clustering stage reuses.
-__global__ void __launch_bounds__(kSingle) k_ground_mode(FramePtrs a, GroundPtrs gp) {
-    pdl_prologue();
+__device__ __forceinline__ void ground_mode(const FramePtrs& a, const GroundPtrs& gp) {
     __shared__ unsigned long long s_best[kSingle / 32];
     const bool ascending = !(gp.mode == MOR_GROUND_VOXEL_COV && gp.bin_gap < 0.f);
     unsigned long long best = 0ull;  // (count << 32) | (65535 - rank-of-key): max => largest count, then smallest key
@@ -438,16 +456,19 @@ __global__ void __launch_bounds__(kSingle) k_ground_mode(FramePtrs a, GroundPtrs
     for (int t = threadIdx.x; t < gp.tiles_vox; t += kSingle) gp.st_vox[t] = 0ull;
     if (threadIdx.x < 3) { a.scratch->box_inv_min[threadIdx.x] = 0u; a.scratch->box_max[threadIdx.x] = 0u; }
 }
+__global__ void __launch_bounds__(kSingle) k_ground_mode(FramePtrs a, GroundPtrs gp) {
+    pdl_prologue();
+    ground_mode(a, gp);
+}
 
 // ===================================================================================== G7
 // ground = union of the balls of the accepted voxels in the selected bins (cpp:184-191).
-__global__ void __launch_bounds__(kBlock) k_ground_mark(FramePtrs a, GroundPtrs gp) {
-    pdl_prologue();
+__device__ __forceinline__ void ground_mark(const FramePtrs& a, const GroundPtrs& gp, int block, int nblocks) {
     const int lane = threadIdx.x & 31;
-    const int nvox = gp.gstate[1], warps = (gridDim.x * kBlock) >> 5;
+    const int nvox = gp.gstate[1], warps = (nblocks * kBlock) >> 5;
     if (gp.gstate[2] < 0) return;
     const GridDesc g = *gp.ggrid;
-    for (int v = (blockIdx.x * kBlock + threadIdx.x) >> 5; v < nvox; v += warps) {
+    for (int v = (block * kBlock + threadIdx.x) >> 5; v < nvox; v += warps) {
         const float* info = gp.vox_info + (size_t)v * 8;
         if (info[3] == 0.f) continue;
         const int k = (int)info[4] + 32768;
@@ -456,12 +477,15 @@ __global__ void __launch_bounds__(kBlock) k_ground_mark(FramePtrs a, GroundPtrs 
         for_each_in_ball_warp(a, gp, g, info[0], info[1], info[2], lane, [&](const float4& p) { gp.is_ground[__float_as_int(p.w)] = 1; });
     }
 }
+__global__ void __launch_bounds__(kBlock) k_ground_mark(FramePtrs a, GroundPtrs gp) {
+    pdl_prologue();
+    ground_mark(a, gp, blockIdx.x, gridDim.x);
+}
 
 // ===================================================================================== G8
 // ExtractIndices(negative) (cpp:194-198): stable partition of raw_cloud into cloud / gp_indices. The frame kernel
 // takes over from here (phase_bin_cloud).
-__global__ void __launch_bounds__(kBlock) k_ground_partition(FramePtrs a, GroundPtrs gp) {
-    pdl_prologue();
+__device__ __forceinline__ void ground_partition(const FramePtrs& a, const GroundPtrs& gp) {
     __shared__ int s_tile;
     if (threadIdx.x == 0) s_tile = atomicAdd(&a.scratch->ticket_ingest, 1);
     __syncthreads();
@@ -498,6 +522,60 @@ __global__ void __launch_bounds__(kBlock) k_ground_partition(FramePtrs a, Ground
         a.counts[MOR_CNT_NC] = (int)(all & 0x7FFFFFFFull);
         a.counts[MOR_CNT_NG] = (int)((all >> 31) & 0x7FFFFFFFull);
     }
+}
+__global__ void __launch_bounds__(kBlock) k_ground_partition(FramePtrs a, GroundPtrs gp) {
+    pdl_prologue();
+    ground_partition(a, gp);
+}
+
+// ===================================================================================== batched forms
+// The same nine stages for S sequences per launch (mor_batch_step_device): blockIdx.y is the sequence, whose arguments
+// come from the device arrays P / GP. The point-indexed stages are sized for the largest frame of the batch; in the two
+// ticket stages the blocks beyond a sequence's own tile count leave before they draw a ticket, so every sequence sees
+// exactly the tickets, look-back tiles and zeroing stride of its single-handle launch. The strided stages accept any
+// x-size.
+__device__ __forceinline__ unsigned ground_blocks_for(uint32_t n) { return n ? (n + kBlock - 1) / kBlock : 1; }
+
+__global__ void __launch_bounds__(kBlock) k_ingest_raw_batch(const FramePtrs* __restrict__ P, const GroundPtrs* __restrict__ GP) {
+    pdl_prologue();
+    const FramePtrs& a = P[blockIdx.y];
+    const unsigned nb = ground_blocks_for(a.n);
+    if (blockIdx.x >= nb) return;
+    ingest_raw(a, GP[blockIdx.y], nb);
+}
+__global__ void __launch_bounds__(kBlock) k_ground_keys_batch(const FramePtrs* __restrict__ P, const GroundPtrs* __restrict__ GP) {
+    pdl_prologue();
+    ground_keys(P[blockIdx.y], GP[blockIdx.y], blockIdx.x);
+}
+__global__ void __launch_bounds__(kBlock) k_scan_cells_batch(const FramePtrs* __restrict__ P, const GroundPtrs* __restrict__ GP) {
+    pdl_prologue();
+    scan_cells(P[blockIdx.y], GP[blockIdx.y].ggrid->ncells);  // over the ball-query grid (k_scan_cells: a.dgrid = gp.ggrid)
+}
+__global__ void __launch_bounds__(kBlock) k_scan_voxels_batch(const FramePtrs* __restrict__ P, const GroundPtrs* __restrict__ GP) {
+    pdl_prologue();
+    scan_voxels(P[blockIdx.y], GP[blockIdx.y]);
+}
+__global__ void __launch_bounds__(kBlock) k_ground_scatter_batch(const FramePtrs* __restrict__ P, const GroundPtrs* __restrict__ GP) {
+    pdl_prologue();
+    ground_scatter(P[blockIdx.y], GP[blockIdx.y], blockIdx.x);
+}
+__global__ void __launch_bounds__(kBlock) k_voxel_eval_batch(const FramePtrs* __restrict__ P, const GroundPtrs* __restrict__ GP) {
+    pdl_prologue();
+    voxel_eval(P[blockIdx.y], GP[blockIdx.y], blockIdx.x, gridDim.x);
+}
+__global__ void __launch_bounds__(kSingle) k_ground_mode_batch(const FramePtrs* __restrict__ P, const GroundPtrs* __restrict__ GP) {
+    pdl_prologue();
+    ground_mode(P[blockIdx.y], GP[blockIdx.y]);
+}
+__global__ void __launch_bounds__(kBlock) k_ground_mark_batch(const FramePtrs* __restrict__ P, const GroundPtrs* __restrict__ GP) {
+    pdl_prologue();
+    ground_mark(P[blockIdx.y], GP[blockIdx.y], blockIdx.x, gridDim.x);
+}
+__global__ void __launch_bounds__(kBlock) k_ground_partition_batch(const FramePtrs* __restrict__ P, const GroundPtrs* __restrict__ GP) {
+    pdl_prologue();
+    const FramePtrs& a = P[blockIdx.y];
+    if (blockIdx.x >= ground_blocks_for(a.n)) return;
+    ground_partition(a, GP[blockIdx.y]);
 }
 
 }  // namespace mor

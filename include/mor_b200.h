@@ -129,10 +129,11 @@ int mor_get_output_device(mor_handle* h, const void** d_records);
 int mor_sync(mor_handle* h);
 
 /* Batched device-resident step (BASELINE config 5: many independent sequences per GPU): one pushRawCloudAndPose +
- * filterCloud for S sequences in ONE launch of the frame kernel (a group of CTAs per sequence). All handles must
- * live on the same device with the same config, limits and frame count, ground_mode 0. d_data[s] / d_out[s] are
- * device pointers (d_out[s] must hold n[s] records), poses7 = S x 7 doubles. Asynchronous on hs[0]'s stream;
- * mor_sync / mor_tap on any of the handles waits for it. */
+ * filterCloud for S sequences in ONE launch of the frame kernel (a group of CTAs per sequence). With the voxel ground
+ * modes (ground_mode 1 / 2) the ground stage of all S frames runs first, as 9 launches whatever S (S <= 65535). All
+ * handles must live on the same device with the same config (ground_mode included), limits and frame count.
+ * d_data[s] / d_out[s] are device pointers (d_out[s] must hold n[s] records), poses7 = S x 7 doubles. Asynchronous on
+ * hs[0]'s stream; mor_sync / mor_tap on any of the handles waits for it. */
 int mor_batch_step_device(mor_handle* const* hs, uint32_t S, const void* const* d_data, const uint32_t* n,
                           uint32_t point_step, uint32_t off_x, uint32_t off_y, uint32_t off_z, uint32_t off_i,
                           const double* poses7, void* const* d_out);
