@@ -135,6 +135,7 @@ class MorBinding:
         self.collect_frame = f("collect_frame", [vp, C.POINTER(u32)], True)
         self.frames_in_flight = f("frames_in_flight", [vp, C.POINTER(u32)], True)
         self.set_pipelining = f("set_pipelining", [vp, C.c_int], True)
+        self.set_output_records = f("set_output_records", [vp, C.c_int], True)
 
     def _fn(self, name, argtypes, optional=False, restype=C.c_int):
         try:
@@ -176,7 +177,8 @@ class MovingObjectRemoval:
     push_raw_cloud_and_pose(points, pose7): `points` is a C-contiguous numpy array; either float32
     [N, F] with x,y,z,intensity in columns 0..3 (F >= 3; F == 3 => no intensity), or a uint8 blob with
     explicit point_step/offsets (PCLPointCloud2 semantics, reference cpp:523).
-    filter_cloud() returns float32 [N_out, 8] PointXYZI wire records (x,y,z,1,intensity,0,0,0), cpp:690.
+    filter_cloud() returns float32 [N_out, 8] PointXYZI wire records (x,y,z,1,intensity,0,0,0), cpp:690; with
+    set_output_records(True), uint8 [N_out, point_step] copies of the input records the points came from.
     """
 
     def __init__(self, config_path, n_bad: int = 4, n_good: int = 3, device: int = 0, binding: MorBinding | None = None,
@@ -190,6 +192,8 @@ class MovingObjectRemoval:
             raise MorError(st, "mor_create", str(config_path))
         self._out = None
         self.n_input = 0
+        self.output_records = False  # the setting (set_output_records)
+        self._rec_step = 0           # point_step of the last frame pushed in record mode, 0 for PointXYZI output
 
     def close(self):
         if getattr(self, "h", None) and self.h.value:
@@ -238,16 +242,28 @@ class MovingObjectRemoval:
         self._keep = points  # the copy is asynchronous: keep the buffer alive until the next sync
         self.n_input = n
         self._check(self.b.push(self.h, points.ctypes.data_as(C.c_void_p), n, step, *offs, pose), "push_raw_cloud_and_pose")
+        self._rec_step = step if self.output_records else 0
+
+    def _out_array(self, cap, step):
+        """Default output buffer: float32 [cap, 8] PointXYZI records, or uint8 [cap, step] input records."""
+        if self._out is None or self._out.shape[0] < cap or self._out.dtype != (np.uint8 if step else np.float32) \
+                or (step and self._out.shape[1] != step):
+            self._out = np.empty((cap, step), np.uint8) if step else np.empty((cap, 8), np.float32)
+        return self._out
 
     def filter_cloud(self, out: np.ndarray | None = None) -> np.ndarray:
         cap = max(self.n_input, 1)
         if out is None:
-            if self._out is None or self._out.shape[0] < cap:
-                self._out = np.empty((cap, 8), np.float32)
-            out = self._out
+            out = self._out_array(cap, self._rec_step)
         n_out = C.c_uint32(0)
         self._check(self.b.filter(self.h, out.ctypes.data_as(C.c_void_p), out.shape[0], C.byref(n_out)), "filter_cloud")
         return out[: n_out.value]
+
+    def set_output_records(self, enabled: bool):
+        """Deliver the filtered cloud as copies of the input records (every field kept) from the next push on; see
+        mor_set_output_records. filter_cloud / collect_frame then return uint8 [N_out, point_step] arrays."""
+        self._check(self.b.set_output_records(self.h, 1 if enabled else 0), "set_output_records")
+        self.output_records = bool(enabled)
 
     def cluster_collection(self) -> np.ndarray:
         """The reference's VISUALIZE debug cloud (cpp:226-229, :553-558): float32 [N_k, 8] PointXYZI records."""
@@ -311,8 +327,9 @@ class MovingObjectRemoval:
 
     # pipelined streaming (product only): copies of neighbouring frames overlap the frame kernel
     def submit_frame(self, points: np.ndarray, pose7, out: np.ndarray, point_step=None, offsets=None):
-        """push + filter of one frame, enqueued without waiting; `points` and `out` (float32 [cap, 8], both ideally views
-        of pinned memory) must stay untouched until collect_frame() has returned for this frame."""
+        """push + filter of one frame, enqueued without waiting; `points` and `out` (float32 [cap, 8], or uint8
+        [cap, point_step] with output records; both ideally views of pinned memory) must stay untouched until
+        collect_frame() has returned for this frame."""
         pose = (C.c_double * 7)(*[float(v) for v in pose7])
         if points.dtype == np.float32 and point_step is None:
             assert points.ndim == 2 and points.shape[1] >= 3 and points.flags.c_contiguous
@@ -321,7 +338,10 @@ class MovingObjectRemoval:
         else:
             assert points.flags.c_contiguous and point_step is not None and offsets is not None
             n, step, offs = points.nbytes // point_step, point_step, offsets
-        assert out.dtype == np.float32 and out.ndim == 2 and out.shape[1] == 8 and out.flags.c_contiguous
+        if self.output_records:
+            assert out.dtype == np.uint8 and out.ndim == 2 and out.shape[1] == step and out.flags.c_contiguous
+        else:
+            assert out.dtype == np.float32 and out.ndim == 2 and out.shape[1] == 8 and out.flags.c_contiguous
         self.n_input = n
         self._inflight = getattr(self, "_inflight", [])
         self._inflight.append((points, out))
@@ -406,6 +426,8 @@ class SequenceBatch:
         self._poses = (C.c_double * (7 * S))()
 
     def step_device(self, d_ptrs, ns, poses, d_outs, point_step=16, offsets=(0, 4, 8, 12)):
+        """d_outs[s] must hold ns[s] output points: 32-byte PointXYZI records, or ns[s] * point_step bytes when the
+        handles deliver output records (set_output_records)."""
         S = len(self.handles)
         for s in range(S):
             self._data[s] = d_ptrs[s]

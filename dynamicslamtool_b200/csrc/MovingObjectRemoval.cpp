@@ -61,6 +61,15 @@ void MovingObjectRemoval::pushRawCloudAndPose(pcl::PCLPointCloud2& cloud, geomet
     n_in_ = n;
     status_ = mor_push_raw_cloud_and_pose(h_, cloud.data.data(), n, cloud.point_step, ox, oy, oz, oi, p7);
     push_failed_ = status_ != MOR_OK;
+    rec_step_ = keep_fields_ ? cloud.point_step : 0;
+    if (keep_fields_) { rec_fields_ = cloud.fields; rec_bigendian_ = cloud.is_bigendian; }
+}
+
+bool MovingObjectRemoval::setKeepInputFields(bool keep) {
+    status_ = mor_set_output_records(h_, keep ? 1 : 0);
+    if (status_ != MOR_OK) return false;
+    keep_fields_ = keep;
+    return true;
 }
 
 bool MovingObjectRemoval::filterCloud(pcl::PCLPointCloud2& out_cloud, std::string f_id) {
@@ -71,13 +80,28 @@ bool MovingObjectRemoval::filterCloud(pcl::PCLPointCloud2& out_cloud, std::strin
     pin_output();
     if (output.data.size() < pinned_cap_) output.data.resize(pinned_cap_);
     uint32_t n_out = 0;
-    status_ = mor_filter_cloud(h_, output.data.data(), (uint32_t)(pinned_cap_ / 32), &n_out);
+    status_ = mor_filter_cloud(h_, output.data.data(), (uint32_t)(pinned_cap_ / (rec_step_ ? rec_step_ : 32)), &n_out);
     if (status_ != MOR_OK) return false;
+    output.header.seq = 0; output.header.frame_id = f_id;
+    if (rec_step_) {  // the input records: the pushed cloud's layout
+        const uint32_t st = rec_step_;
+        output.height = 1; output.width = n_out; output.is_bigendian = rec_bigendian_; output.point_step = st; output.row_step = st * n_out; output.is_dense = 1;
+        output.fields.resize(rec_fields_.size());
+        for (size_t i = 0; i < rec_fields_.size(); i++) {
+            output.fields[i].name = rec_fields_[i].name; output.fields[i].offset = rec_fields_[i].offset;
+            output.fields[i].datatype = rec_fields_[i].datatype; output.fields[i].count = rec_fields_[i].count;
+        }
+        output.data.resize((size_t)n_out * st);
+        out_cloud.header = pcl::PCLHeader();
+        out_cloud.height = 1; out_cloud.width = n_out; out_cloud.is_bigendian = rec_bigendian_; out_cloud.point_step = st; out_cloud.row_step = st * n_out; out_cloud.is_dense = 1;
+        out_cloud.fields = rec_fields_;
+        out_cloud.data.assign(output.data.begin(), output.data.end());
+        return true;
+    }
     // pcl::toPCLPointCloud2 of a pcl::PointCloud<PointXYZI> (cpp:690): 32-byte records, fields x@0 y@4 z@8 intensity@16
     static const char* const names[4] = {"x", "y", "z", "intensity"};
     static const uint32_t offs[4] = {0, 4, 8, 16};
     // pcl_conversions::fromPCL(out_cloud, output); output.header.frame_id = f_id (cpp:691-692)
-    output.header.seq = 0; output.header.frame_id = f_id;
     output.height = 1; output.width = n_out; output.is_bigendian = 0; output.point_step = 32; output.row_step = 32 * n_out; output.is_dense = 1;
     output.fields.resize(4);
     for (int i = 0; i < 4; i++) { output.fields[i].name = names[i]; output.fields[i].offset = offs[i]; output.fields[i].datatype = 7; output.fields[i].count = 1; }

@@ -8,6 +8,8 @@
 // Throughput paths on top of that: mor_submit_frame / mor_collect_frame (copies of neighbouring frames on their own
 // streams, up to four frames in flight) and mor_set_pipelining (k_frame_pipe: the back half of frame f in one launch with
 // the front half of frame f+1; the frame products are triple-buffered for it, see fill_frame / launch_pipe).
+// mor_set_output_records: the filtered cloud as copies of the input records, by a gather kernel after the launch that ran
+// the frame's filter phase (mor_records.cuh); the frame kernels themselves do not change.
 // There is no CPU fallback: every entry point that computes needs the device.
 #include <cmath>
 #include <cstdio>
@@ -19,6 +21,7 @@
 #include "mor_kernels.cuh"
 #include "mor_ground.cuh"
 #include "mor_debug.cuh"
+#include "mor_records.cuh"
 
 using namespace mor;
 
@@ -116,6 +119,7 @@ struct mor_handle {
         uint8_t* d_in = nullptr; float4* d_out = nullptr; int32_t* h_counts = nullptr;
         cudaEvent_t h2d = nullptr, done = nullptr, d2h = nullptr;
         void* out = nullptr; uint32_t cap = 0, spec = 0, n = 0;
+        uint32_t rec_bytes = 32;  // bytes per output point of the frame in the slot: 32 (PointXYZI) or its point_step
         const int* d_counts = nullptr;
         bool used = false, d2h_enqueued = false;
     } slot[MOR_STREAM_DEPTH];
@@ -138,6 +142,11 @@ struct mor_handle {
     // of the next frame
     bool pipelining = false, back_pending = false;
     FramePtrs back_frame;
+    // output records (mor_set_output_records): the setting for frames pushed from now on, the mode of the current frame
+    // and of the pending back half, and where a batched step gathered the current frame's records (else frame.out)
+    bool out_records = false, frame_rec = false, back_rec = false;
+    void* rec_out = nullptr;
+    unsigned long long* rec_st = nullptr; int* rec_ctr = nullptr;  // the gather's tile states and counters (zero between launches)
     bool have_cur = false, have_prev = false, filtered = false;
     int mo_parity = 0;
     double cur_pose[7], prev_pose[7];
@@ -307,6 +316,7 @@ int allocate(mor_handle* h) {
         }
         b.track = carve<TrackState>(p, 1); b.mo_centroid = carve<float>(p, 2 * MO * 3); b.mo_conf = carve<int>(p, 2 * MO);
         b.res_ring = carve<uint8_t>(p, D * K); b.res_len = carve<int>(p, D); b.corr_ring = carve<int>(p, D * K); b.corr_len = carve<int>(p, D);
+        h->rec_st = carve<unsigned long long>(p, N / kRecT + 2); h->rec_ctr = carve<int>(p, 2);
         return p;
     };
     h->arena_bytes = (size_t)(plan(nullptr) - (uint8_t*)nullptr) + 256;
@@ -426,6 +436,28 @@ int launch_phase(mor_handle* h, const FramePtrs& a) {
     return MOR_OK;
 }
 
+// The gather of output records (mor_records.cuh) for the frame `a`, into its output buffer a.out (a batched step passes
+// d_out[s] to record_ptrs instead): enqueued after the launch that ran the frame's filter phase and before anything
+// rewrites what it reads (the frame's input, its parity buffers, cluster_removed).
+inline unsigned rec_blocks(uint32_t n) { return n ? (n + kRecT - 1) / kRecT : 1; }
+RecordPtrs record_ptrs(const mor_handle* h, const FramePtrs& a, void* dst) {
+    RecordPtrs r;
+    r.in = a.in; r.step = a.step;
+    const uintptr_t al = (uintptr_t)a.in | (uintptr_t)dst | a.step;
+    r.copy = al % 16 == 0 ? REC_VEC16 : al % 4 == 0 ? REC_WORD : REC_BYTES;
+    r.counts = a.counts; r.cid = a.cid; r.cluster_removed = a.cluster_removed; r.track = a.track;
+    r.cloud_src = a.cloud_src; r.gsrc = a.gsrc;
+    r.out = (uint8_t*)dst; r.st = h->rec_st; r.ctr = h->rec_ctr;
+    return r;
+}
+int launch_gather(mor_handle* h, const FramePtrs& a) {
+    k_gather_records<<<rec_blocks(a.n), kRecT, 0, h->stream>>>(record_ptrs(h, a, a.out));
+    h->launches++;
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) { h->last_error = std::string("k_gather_records: ") + cudaGetErrorString(e); return MOR_ERR_CUDA; }
+    return MOR_OK;
+}
+
 // Pipelined launches (k_frame_pipe): the front half of `front` on most CTAs beside the pending back half, or either alone.
 int launch_pipe(mor_handle* h, const FramePtrs* front, const FramePtrs* back) {
     const int G = h->frame_ctas;
@@ -456,7 +488,8 @@ int launch_pipe(mor_handle* h, const FramePtrs* front, const FramePtrs* back) {
 int flush_back(mor_handle* h) {
     if (!h->back_pending) return MOR_OK;
     h->back_pending = false;
-    return launch_pipe(h, nullptr, &h->back_frame);
+    const int s = launch_pipe(h, nullptr, &h->back_frame);
+    return s != MOR_OK || !h->back_rec ? s : launch_gather(h, h->back_frame);
 }
 
 int enqueue_push(mor_handle* h, const uint8_t* d_points, uint32_t n, uint32_t step, uint32_t ox, uint32_t oy, uint32_t oz, uint32_t oi, bool allow_pipe) {
@@ -485,18 +518,22 @@ int enqueue_push(mor_handle* h, const uint8_t* d_points, uint32_t n, uint32_t st
             (s = launch_phase<PH_JUMP>(h, a)) || (s = launch_phase<PH_CROSS>(h, a)) || (s = launch_phase<PH_ROOTS>(h, a)) || (s = launch_phase<PH_SELECT>(h, a)) || (s = launch_phase<PH_STATS>(h, a)) || 
             (s = launch_phase<PH_MOVING>(h, a)) || (s = launch_phase<PH_FILTER>(h, a)))
             return s;
+        if (h->frame_rec) return launch_gather(h, a);
     } else if (allow_pipe && h->pipelining && h->cfg.method_choice == 2 && h->cfg.ground_mode == MOR_GROUND_CROP) {
         // front half of this frame, beside the back half of the frame before if that one has been filtered already
         const bool fused = h->back_pending;
         h->back_pending = false;
         int s = launch_pipe(h, &a, fused ? &h->back_frame : nullptr);
         if (s != MOR_OK) return s;
+        if (fused && h->back_rec && (s = launch_gather(h, h->back_frame)) != MOR_OK) return s;
         h->back_frame = a;  // this frame's back half: beside the next frame's front half, or alone as soon as somebody needs its results
+        h->back_rec = h->frame_rec;
         h->back_pending = true;
     } else {
         cudaError_t e = launch_coop(k_frame, (unsigned)h->frame_ctas, h->frame_smem, st, a);
         h->launches++;
         if (e != cudaSuccess) { h->last_error = std::string("k_frame: ") + cudaGetErrorString(e); return MOR_ERR_CUDA; }
+        if (h->frame_rec) return launch_gather(h, a);
     }
     return MOR_OK;
 }
@@ -537,6 +574,7 @@ void advance_frame(mor_handle* h, uint32_t n, const double pose7[7]) {
     if (h->two_frames) pose_delta_affine(h->prev_pose, h->cur_pose, h->M);
     h->have_cur = true;
     h->filtered = false;
+    h->frame_rec = h->out_records; h->rec_out = nullptr;
 }
 
 // Work of a handle may have been enqueued on another handle's stream by mor_batch_step_device.
@@ -554,6 +592,7 @@ int do_push(mor_handle* h, const void* data, bool on_device, uint32_t n, uint32_
     if (validate_layout(step, ox, oy, oz, oi) != MOR_OK) { h->last_error = "point_step / field offsets do not describe a record with float32 x, y, z"; return MOR_ERR_ARG; }
     if (n > h->nmax) { h->last_error = "frame larger than mor_limits.max_points"; return MOR_ERR_CAPACITY; }
     if (h->inflight) { h->last_error = "submitted frames are in flight: collect them first"; return MOR_ERR_STATE; }
+    if (h->out_records && (size_t)n * step > h->d_in_bytes) { h->last_error = "output records: n * point_step exceeds the output buffer (32 B x max_points)"; return MOR_ERR_CAPACITY; }
     h->out_cur = h->slot[0].d_out;
     MOR_CUDA(cudaSetDevice(h->device));
     { int js = join_foreign_stream(h, on_device && h->pipelining && h->cfg.ground_mode == MOR_GROUND_CROP && !h->profiling); if (js != MOR_OK) return js; }
@@ -597,11 +636,18 @@ int do_filter(mor_handle* h, void* out, bool on_device, uint32_t cap_points, uin
         prof_end(h);
         h->launches++;
         MOR_CUDA(cudaGetLastError());
+        if (h->frame_rec) {  // (after a batched step this gathers into the handle's own buffer, no longer into d_out[s])
+            h->rec_out = nullptr;
+            int gs = launch_gather(h, a);
+            if (gs != MOR_OK) return gs;
+        }
         h->filtered = false;  // committed below like a first call
     }
     if (h->timing) MOR_CUDA(cudaEventRecord(h->ev[3], st));
+    const size_t rb = h->frame_rec ? a.step : 32;  // bytes per output point
+    const void* src = h->rec_out ? h->rec_out : a.out;
     if (on_device && !n_out && !h->profiling) {  // fully asynchronous device-resident mode
-        if (out && h->n_input) MOR_CUDA(cudaMemcpyAsync(out, a.out, (size_t)h->n_input * 32, cudaMemcpyDeviceToDevice, st));
+        if (out && h->n_input) MOR_CUDA(cudaMemcpyAsync(out, src, (size_t)h->n_input * rb, cudaMemcpyDeviceToDevice, st));
         h->mo_parity ^= 1; a.mo_parity = h->mo_parity; h->filtered = true;
         return MOR_OK;
     }
@@ -614,7 +660,7 @@ int do_filter(mor_handle* h, void* out, bool on_device, uint32_t cap_points, uin
         spec = h->spec_out ? h->spec_out + h->spec_out / 32 + 1024 : h->n_input;
         if (spec > h->n_input) spec = h->n_input;
         if (spec > cap_points) spec = cap_points;
-        if (spec) MOR_CUDA(cudaMemcpyAsync(out, a.out, (size_t)spec * 32, cudaMemcpyDeviceToHost, st));
+        if (spec) MOR_CUDA(cudaMemcpyAsync(out, src, (size_t)spec * rb, cudaMemcpyDeviceToHost, st));
     }
     MOR_CUDA(cudaStreamSynchronize(st));
     if (h->profiling) prof_harvest(h);
@@ -630,10 +676,10 @@ int do_filter(mor_handle* h, void* out, bool on_device, uint32_t cap_points, uin
     }
     if (no > cap_points && out) return MOR_ERR_CAPACITY;  // not committed: the call can be repeated with a larger buffer
     if (!on_device && out && no > spec) {
-        MOR_CUDA(cudaMemcpyAsync((uint8_t*)out + (size_t)spec * 32, (const uint8_t*)a.out + (size_t)spec * 32, (size_t)(no - spec) * 32, cudaMemcpyDeviceToHost, st));
+        MOR_CUDA(cudaMemcpyAsync((uint8_t*)out + (size_t)spec * rb, (const uint8_t*)src + (size_t)spec * rb, (size_t)(no - spec) * rb, cudaMemcpyDeviceToHost, st));
         MOR_CUDA(cudaStreamSynchronize(st));
     }
-    if (on_device && out && no) MOR_CUDA(cudaMemcpyAsync(out, a.out, (size_t)no * 32, cudaMemcpyDeviceToDevice, st));
+    if (on_device && out && no) MOR_CUDA(cudaMemcpyAsync(out, src, (size_t)no * rb, cudaMemcpyDeviceToDevice, st));
     h->mo_parity ^= 1; a.mo_parity = h->mo_parity; h->filtered = true;  // commit
     return MOR_OK;
 }
@@ -649,6 +695,7 @@ int reset_state(mor_handle* h) {
     MOR_CUDA(cudaStreamSynchronize(h->stream));
     h->cur = 0; h->fpar = 0; h->back_pending = false; h->have_cur = h->have_prev = h->filtered = h->two_frames = false;
     h->mo_parity = 0; h->n_input = h->n_prev_input = 0; h->spec_out = 0;
+    h->frame_rec = h->back_rec = false; h->rec_out = nullptr;  // (out_records, the setting, stays)
     h->last_stream = h->stream;
     return MOR_OK;
 }
@@ -762,7 +809,7 @@ int mor_filter_cloud_device(mor_handle* h, void* d_out, uint32_t cap_points, uin
 int mor_get_output_device(mor_handle* h, const void** d_records) {
     if (!h || !d_records) return MOR_ERR_ARG;
     if (!h->have_cur || !h->filtered) return MOR_ERR_STATE;
-    *d_records = h->frame.out;
+    *d_records = h->rec_out ? h->rec_out : h->frame.out;
     return MOR_OK;
 }
 
@@ -785,11 +832,21 @@ int mor_batch_step_device(mor_handle* const* hs, uint32_t S, const void* const* 
         for (uint32_t t = 0; t < s; t++) if (hs[t] == g) return MOR_ERR_ARG;
     }
     const bool ground = h->cfg.ground_mode != MOR_GROUND_CROP;  // (shared by every handle: part of the config compared above)
+    const bool rec = h->out_records;
+    if (rec && S > 65535u) { h->last_error = "output records: at most 65535 sequences per batched step"; return MOR_ERR_ARG; }
+    for (uint32_t s = 0; s < S; s++) {
+        if (hs[s]->out_records != rec) { h->last_error = "batched handles must agree on mor_set_output_records"; return MOR_ERR_ARG; }
+        if (rec && (size_t)n[s] * point_step > hs[s]->d_in_bytes) {
+            h->last_error = "output records: n * point_step exceeds the output buffer (32 B x max_points)";
+            return MOR_ERR_CAPACITY;
+        }
+    }
     if (ground && S > 65535u) { h->last_error = "the voxel ground modes batch at most 65535 sequences per step"; return MOR_ERR_ARG; }
     MOR_CUDA(cudaSetDevice(h->device));
     cudaStream_t st = h->stream;
     static_assert(sizeof(FramePtrs) % alignof(GroundPtrs) == 0, "GroundPtrs follow the FramePtrs of a ring slot");
-    const size_t per_seq = sizeof(FramePtrs) + sizeof(GroundPtrs);
+    static_assert((sizeof(FramePtrs) + sizeof(GroundPtrs)) % alignof(RecordPtrs) == 0, "RecordPtrs follow the GroundPtrs of a ring slot");
+    const size_t per_seq = sizeof(FramePtrs) + sizeof(GroundPtrs) + sizeof(RecordPtrs);
     if (S > h->batch_cap) {
         MOR_CUDA(cudaStreamSynchronize(st));
         if (h->d_batch) cudaFree(h->d_batch);
@@ -809,6 +866,7 @@ int mor_batch_step_device(mor_handle* const* hs, uint32_t S, const void* const* 
     FramePtrs* dp = reinterpret_cast<FramePtrs*>(h->d_batch + (size_t)slot * per_seq * h->batch_cap);
     GroundPtrs* hg = reinterpret_cast<GroundPtrs*>(hp + S);
     const GroundPtrs* dg = reinterpret_cast<const GroundPtrs*>(dp + S);
+    RecordPtrs* hr = reinterpret_cast<RecordPtrs*>(hg + S);
     uint32_t n_max = 0;
     // G CTAs per sequence; the groups run side by side, a group that has more than one sequence steps them in turn
     int G = h->frame_ctas / (int)S;
@@ -826,13 +884,18 @@ int mor_batch_step_device(mor_handle* const* hs, uint32_t S, const void* const* 
         advance_frame(g, n[s], poses7 + 7 * s);
         g->out_cur = g->slot[0].d_out;
         fill_frame(g, (const uint8_t*)d_data[s], n[s], point_step, off_x, off_y, off_z, off_i);
-        g->frame.out = (float4*)d_out[s];
+        if (rec) {  // the frame kernel's PointXYZI records go to the handle's own buffer, the gather alone writes d_out[s]
+            hr[s] = record_ptrs(g, g->frame, d_out[s]);
+            g->rec_out = d_out[s];
+        } else {
+            g->frame.out = (float4*)d_out[s];
+        }
         set_segments(g, g->frame, G);
         hp[s] = g->frame;
         if (ground) { hg[s] = g->ground; n_max = n[s] > n_max ? n[s] : n_max; }
         g->last_stream = st;
     }
-    MOR_CUDA(cudaMemcpyAsync(dp, hp, (ground ? per_seq : sizeof(FramePtrs)) * S, cudaMemcpyHostToDevice, st));
+    MOR_CUDA(cudaMemcpyAsync(dp, hp, (rec ? per_seq : ground ? sizeof(FramePtrs) + sizeof(GroundPtrs) : sizeof(FramePtrs)) * S, cudaMemcpyHostToDevice, st));
     MOR_CUDA(cudaEventRecord(h->batch_ev[slot], st));
     if (ground) {  // voxel-covariance ground removal of all S frames: 9 launches, then the frame kernel takes over
         int gs = enqueue_ground_batch(h, dp, dg, S, n_max);
@@ -842,6 +905,14 @@ int mor_batch_step_device(mor_handle* const* hs, uint32_t S, const void* const* 
         cudaError_t e = launch_coop(k_frame_batch, (unsigned)(groups * G), h->frame_smem, st, (const FramePtrs*)dp, (int)S, G);
         h->launches++;
         if (e != cudaSuccess) { h->last_error = std::string("k_frame_batch: ") + cudaGetErrorString(e); return MOR_ERR_CUDA; }
+    }
+    if (rec) {  // one gather launch for all S sequences
+        uint32_t nm = 0;
+        for (uint32_t s = 0; s < S; s++) nm = n[s] > nm ? n[s] : nm;
+        k_gather_records_batch<<<dim3(rec_blocks(nm), S), kRecT, 0, st>>>(reinterpret_cast<const RecordPtrs*>(reinterpret_cast<const GroundPtrs*>(dp + S) + S));
+        h->launches++;
+        const cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) { h->last_error = std::string("k_gather_records_batch: ") + cudaGetErrorString(e); return MOR_ERR_CUDA; }
     }
     for (uint32_t s = 0; s < S; s++) {  // push + filter in one call: the frame is committed
         hs[s]->mo_parity ^= 1;
@@ -894,7 +965,7 @@ static int enqueue_slot_d2h(mor_handle* h, mor_handle::StreamSlot& sl) {
     uint32_t spec = h->spec_out ? h->spec_out + h->spec_out / 32 + 1024 : sl.n;
     if (spec > sl.n) spec = sl.n;
     if (spec > sl.cap) spec = sl.cap;
-    if (spec) MOR_CUDA(cudaMemcpyAsync(sl.out, sl.d_out, (size_t)spec * 32, cudaMemcpyDeviceToHost, h->copy_out));
+    if (spec) MOR_CUDA(cudaMemcpyAsync(sl.out, sl.d_out, (size_t)spec * sl.rec_bytes, cudaMemcpyDeviceToHost, h->copy_out));
     MOR_CUDA(cudaEventRecord(sl.d2h, h->copy_out));
     sl.spec = spec; sl.d2h_enqueued = true;
     return MOR_OK;
@@ -931,6 +1002,7 @@ int mor_submit_frame(mor_handle* h, const void* data, uint32_t n, uint32_t step,
     int st = enqueue_push(h, sl.d_in, n, step, ox, oy, oz, oi, /*allow_pipe=*/true);
     if (st != MOR_OK) return st;
     sl.out = out; sl.cap = cap_points; sl.n = n; sl.d_counts = h->frame.counts; sl.used = true; sl.d2h_enqueued = false;
+    sl.rec_bytes = h->frame_rec ? step : 32;
     if (piped) {
         // the launch just enqueued carried the back half of the frame before (if one was waiting): that frame is complete now
         if (h->inflight) {
@@ -969,7 +1041,8 @@ int mor_collect_frame(mor_handle* h, uint32_t* n_out) {
     }
     if (no > sl.cap) { h->last_error = "output buffer of the submitted frame too small"; return MOR_ERR_CAPACITY; }
     if (no > sl.spec) {  // (the slot's device buffer is not rewritten before the frame after next is submitted)
-        MOR_CUDA(cudaMemcpyAsync((uint8_t*)sl.out + (size_t)sl.spec * 32, (const uint8_t*)sl.d_out + (size_t)sl.spec * 32, (size_t)(no - sl.spec) * 32,
+        const size_t rb = sl.rec_bytes;
+        MOR_CUDA(cudaMemcpyAsync((uint8_t*)sl.out + (size_t)sl.spec * rb, (const uint8_t*)sl.d_out + (size_t)sl.spec * rb, (size_t)(no - sl.spec) * rb,
                                  cudaMemcpyDeviceToHost, h->copy_out));
         MOR_CUDA(cudaStreamSynchronize(h->copy_out));
     }
@@ -982,6 +1055,13 @@ int mor_set_pipelining(mor_handle* h, int enabled) {
     { int js = join_foreign_stream(h); if (js != MOR_OK) return js; }
     if (h->inflight) { h->last_error = "submitted frames are in flight: collect them first"; return MOR_ERR_STATE; }
     h->pipelining = enabled != 0;
+    return MOR_OK;
+}
+
+int mor_set_output_records(mor_handle* h, int enabled) {
+    if (!h) return MOR_ERR_ARG;
+    if (h->inflight) { h->last_error = "submitted frames are in flight: collect them first"; return MOR_ERR_STATE; }
+    h->out_records = enabled != 0;  // (a frame already pushed, pending back half included, is delivered in its own mode)
     return MOR_OK;
 }
 

@@ -6,7 +6,7 @@
 // runs can be compared across implementations.
 //
 //   mov_harness <MOR_config.txt> <scenario 1..4> <seed> <frames> [n_bad=4] [n_good=3] [--quiet]
-//   mov_harness <MOR_config.txt> --replay <dir> [frames] [n_bad=4] [n_good=3] [--quiet] [--out <dir>]
+//   mov_harness <MOR_config.txt> --replay <dir> [frames] [n_bad=4] [n_good=3] [--quiet] [--out <dir>] [--keep-fields]
 //       (either form: --stream replays through mor_submit_frame / mor_collect_frame with pipelined launches: full rate, results three frames late)
 //       (either form: --debug also fetches the VISUALIZE debug cloud and bounding-box markers of every frame)
 //       recorded data: KITTI-style .bin clouds + poses.txt (+ calib.txt), see replay_io.h; --out writes the filtered clouds
@@ -139,10 +139,10 @@ int main(int argc, char** argv) {
         }
         return 0;
     }
-    if (argc < 4) { std::fprintf(stderr, "usage: %s <config> <scenario> <seed> <frames> [n_bad] [n_good] [--quiet]\n       %s <config> --replay <dir> [frames] [n_bad] [n_good] [--quiet] [--out <dir>]\n", argv[0], argv[0]); return 2; }
+    if (argc < 4) { std::fprintf(stderr, "usage: %s <config> <scenario> <seed> <frames> [n_bad] [n_good] [--quiet]\n       %s <config> --replay <dir> [frames] [n_bad] [n_good] [--quiet] [--out <dir>] [--keep-fields]\n", argv[0], argv[0]); return 2; }
     const std::string cfg = argv[1];
     const bool replay_mode = !std::strcmp(argv[2], "--replay");
-    bool quiet = false, debug = false, stream = false;  // --debug: also fetch the VISUALIZE outputs (debug cloud, markers) every frame
+    bool quiet = false, debug = false, stream = false, keep_fields = false;  // --debug: also fetch the VISUALIZE outputs (debug cloud, markers) every frame
     std::string out_dir;
     std::vector<std::string> pos;  // positional arguments after the source
     for (int i = replay_mode ? 4 : 2; i < argc; i++) {
@@ -150,6 +150,7 @@ int main(int argc, char** argv) {
         else if (!std::strcmp(argv[i], "--debug")) debug = true;
         else if (!std::strcmp(argv[i], "--stream")) stream = true;  // replay through the pipelined calls (results arrive three frames late)
         else if (!std::strcmp(argv[i], "--out") && i + 1 < argc) out_dir = argv[++i];
+        else if (!std::strcmp(argv[i], "--keep-fields")) keep_fields = true;  // output = the input records (mor_set_output_records)
         else pos.push_back(argv[i]);
     }
     FrameSource src;
@@ -185,6 +186,8 @@ int main(int argc, char** argv) {
         // be published - when frame f+3 has been submitted. Same per-frame lines as the callback loop below.
         mor_handle* h = mor.handle();
         if (mor_set_pipelining(h, 1) != MOR_OK) { std::fprintf(stderr, "mor_set_pipelining: %s\n", mor_last_error(h)); return 1; }
+        if (keep_fields && mor_set_output_records(h, 1) != MOR_OK) { std::fprintf(stderr, "mor_set_output_records: %s\n", mor_last_error(h)); return 1; }
+        const size_t rec_bytes = keep_fields ? 16 : 32;  // bytes per output point
         const size_t cap = lim.max_points;
         void* in[MOR_STREAM_DEPTH]; void* out[MOR_STREAM_DEPTH]; uint32_t n_of[MOR_STREAM_DEPTH];
         for (int q = 0; q < MOR_STREAM_DEPTH; q++)
@@ -201,9 +204,11 @@ int main(int argc, char** argv) {
             if (!out_dir.empty()) {
                 char name[32];
                 std::snprintf(name, sizeof name, "/%06d.bin", collected);
-                if (!replay::write_bin(out_dir + name, (const uint8_t*)out[q], n_out)) { std::fprintf(stderr, "cannot write %s%s\n", out_dir.c_str(), name); return false; }
+                const bool ok = keep_fields ? replay::write_records(out_dir + name, (const uint8_t*)out[q], (size_t)n_out * rec_bytes)
+                                            : replay::write_bin(out_dir + name, (const uint8_t*)out[q], n_out);
+                if (!ok) { std::fprintf(stderr, "cannot write %s%s\n", out_dir.c_str(), name); return false; }
             }
-            if (!quiet) std::printf("frame %d in %u out %u crc %08x ms 0\n", collected, n_of[q], n_out, crc32_buf((const uint8_t*)out[q], (size_t)n_out * 32));
+            if (!quiet) std::printf("frame %d in %u out %u crc %08x ms 0\n", collected, n_of[q], n_out, crc32_buf((const uint8_t*)out[q], (size_t)n_out * rec_bytes));
             collected++;
             return true;
         };
@@ -228,6 +233,7 @@ int main(int argc, char** argv) {
     cloud.height = 1; cloud.point_step = 16; cloud.is_dense = 1;
     const char* names[4] = {"x", "y", "z", "intensity"};
     for (int i = 0; i < 4; i++) { pcl::PCLPointField f; f.name = names[i]; f.offset = 4 * i; f.datatype = 7; f.count = 1; cloud.fields.push_back(f); }
+    if (keep_fields && !mor.setKeepInputFields(true)) { std::fprintf(stderr, "setKeepInputFields: %s\n", mor_status_string(mor.lastStatus())); return 1; }
     std::vector<double> ms;
     double stage_ms[3] = {0, 0, 0};  // callback copy, pushRawCloudAndPose, filterCloud (frames after the fifth)
     for (int f = 0; f < frames; f++) {
@@ -258,7 +264,9 @@ int main(int argc, char** argv) {
         if (!out_dir.empty()) {
             char name[32];
             std::snprintf(name, sizeof name, "/%06d.bin", f);
-            if (!replay::write_bin(out_dir + name, mor.output.data.data(), mor.output.width)) { std::fprintf(stderr, "cannot write %s%s\n", out_dir.c_str(), name); return 1; }
+            const bool ok = keep_fields ? replay::write_records(out_dir + name, mor.output.data.data(), mor.output.data.size())
+                                        : replay::write_bin(out_dir + name, mor.output.data.data(), mor.output.width);
+            if (!ok) { std::fprintf(stderr, "cannot write %s%s\n", out_dir.c_str(), name); return 1; }
         }
         if (debug) {
             std::vector<mor_marker> markers;

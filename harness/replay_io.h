@@ -186,4 +186,13 @@ inline bool write_bin(const std::string& path, const uint8_t* records32, uint32_
     return ok;
 }
 
+// Output records in the input's own layout (--keep-fields): written as they are.
+inline bool write_records(const std::string& path, const uint8_t* records, size_t bytes) {
+    FILE* f = std::fopen(path.c_str(), "wb");
+    if (!f) return false;
+    const bool ok = std::fwrite(records, 1, bytes, f) == bytes;
+    std::fclose(f);
+    return ok;
+}
+
 }  // namespace replay

@@ -86,6 +86,11 @@ public:
     // and to `output` with header.frame_id = f_id (cpp:613-696).
     bool filterCloud(pcl::PCLPointCloud2& cloud, std::string f_id);
 
+    // Off by default (PointXYZI output, cpp:690). On: from the next pushRawCloudAndPose, filterCloud publishes the kept
+    // points as copies of their input records, with the pushed cloud's fields, point_step and is_bigendian (ring, time
+    // and every other field kept; mor_set_output_records). Returns false (lastStatus()) while that cannot be changed.
+    bool setKeepInputFields(bool keep);
+
     // The reference's VISUALIZE outputs, on request (nothing is computed unless these are called):
     // cb->cluster_collection as published on the debug topic (cpp:553-558), valid after pushRawCloudAndPose ...
     bool clusterCollection(pcl::PCLPointCloud2& debug_cloud);
@@ -102,6 +107,9 @@ private:
     int status_ = MOR_OK;
     uint32_t n_in_ = 0;
     bool push_failed_ = false;    // the last pushRawCloudAndPose did not reach the device: filterCloud must not publish the frame before it
+    bool keep_fields_ = false;    // setKeepInputFields
+    // layout of the frame pushed last when it was pushed with keep_fields_ on (rec_step_ == 0: PointXYZI output)
+    uint32_t rec_step_ = 0; uint8_t rec_bigendian_ = 0; std::vector<pcl::PCLPointField> rec_fields_;
     void* pinned_out_ = nullptr;  // page-locked staging (clusterCollection)
     size_t pinned_cap_ = 0;
     void* registered_ = nullptr;  // storage of output.data, page-locked in place: the D2H copy of filterCloud lands in the message itself

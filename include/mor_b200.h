@@ -109,7 +109,7 @@ int mor_push_raw_cloud_and_pose(mor_handle* h, const void* data, uint32_t n, uin
                                 uint32_t off_x, uint32_t off_y, uint32_t off_z, uint32_t off_i,
                                 const double pose7[7]);
 
-/* Writes the filtered cloud as pcl::PointXYZI wire records (32 B/point: x@0 y@4 z@8 1.0f@12
+/* Writes the filtered cloud (or, with mor_set_output_records, copies of the input records) as pcl::PointXYZI wire records (32 B/point: x@0 y@4 z@8 1.0f@12
  * intensity@16, zero pad; pcl::toPCLPointCloud2, cpp:690) into `out` (capacity cap_points) and
  * the count into *n_out. Synchronous (the D2H copy completes before return).
  * Returns MOR_ERR_CAPACITY (and the needed count in *n_out) if cap_points is too small. */
@@ -133,7 +133,9 @@ int mor_sync(mor_handle* h);
  * modes (ground_mode 1 / 2) the ground stage of all S frames runs first, as 9 launches whatever S (S <= 65535). All
  * handles must live on the same device with the same config (ground_mode included), limits and frame count.
  * d_data[s] / d_out[s] are device pointers (d_out[s] must hold n[s] records), poses7 = S x 7 doubles. Asynchronous on
- * hs[0]'s stream; mor_sync / mor_tap on any of the handles waits for it. */
+ * hs[0]'s stream; mor_sync / mor_tap on any of the handles waits for it. With output records (mor_set_output_records,
+ * which all handles must agree on, else MOR_ERR_ARG) d_out[s] must hold n[s] * point_step bytes, S <= 65535, and d_data[s]
+ * must stay untouched until the step has completed. */
 int mor_batch_step_device(mor_handle* const* hs, uint32_t S, const void* const* d_data, const uint32_t* n,
                           uint32_t point_step, uint32_t off_x, uint32_t off_y, uint32_t off_z, uint32_t off_i,
                           const double* poses7, void* const* d_out);
@@ -163,6 +165,17 @@ int mor_collect_frame(mor_handle* h, uint32_t* n_out);
  * other. Results are identical; a call that needs a frame's results (count, taps, host output) runs its back half at
  * once. Applies to method_choice 2 with the crop ground mode; ignored otherwise. Off by default. */
 int mor_set_pipelining(mor_handle* h, int enabled);
+/* Output records, off by default: every output path above (mor_filter_cloud, mor_filter_cloud_device and
+ * mor_get_output_device, mor_submit_frame / mor_collect_frame, mor_batch_step_device) delivers output point o as a
+ * byte-for-byte copy of the input record it came from - point_step bytes, padding and every field (ring, time, ...)
+ * included - instead of a 32-byte pcl::PointXYZI record; order and count are those of the PointXYZI output, and
+ * cap_points counts records. Costs one more kernel launch per frame (per batched step). Takes effect from the next push,
+ * submit or batched step: a frame is delivered in the mode it was pushed with; mor_reset keeps the setting.
+ * MOR_ERR_STATE while submitted frames are in flight. In this mode a frame with n * point_step > 32 B x max_points is
+ * MOR_ERR_CAPACITY on every path. The records are copied from the caller's input after the frame's filter phase: with
+ * pipelining, a device-resident frame's input (d_data) must stay untouched until the next push or filter call that
+ * needs the frame's results has been enqueued. */
+int mor_set_output_records(mor_handle* h, int enabled);
 /* Frames submitted and not yet collected (0..MOR_STREAM_DEPTH). */
 int mor_frames_in_flight(const mor_handle* h, uint32_t* out);
 

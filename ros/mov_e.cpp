@@ -8,7 +8,9 @@
 //   * the VISUALIZE side outputs (IncludeAll.h:32) - the debug cloud the reference publishes from inside
 //     pushRawCloudAndPose (cpp:553-558) and the CUBE bounding-box markers it publishes from inside filterCloud
 //     (cpp:640-642, mark_cluster cpp:7-58: lifetime 2 s, alpha 0.5, zero extents widened to 0.1) - are published here,
-//     by the node, from clusterCollection() / movingMarkers(); the library never touches the caller's input cloud.
+//     by the node, from clusterCollection() / movingMarkers(); the library never touches the caller's input cloud;
+//   * `--keep-fields` publishes the filtered cloud in the input's own layout (ring, time ... kept: setKeepInputFields)
+//     instead of pcl::PointXYZI, for deskewing consumers downstream.
 // Build: only with ROS (catkin; -DMOR_WITH_ROS). Offline this file is type-checked against ros/stubs/ (tests/test_cpp_headers.py).
 #ifdef MOR_WITH_ROS
 #include <boost/bind.hpp>
@@ -79,8 +81,14 @@ void moving_object_test(const sensor_msgs::PointCloud2ConstPtr& input, const nav
 int main(int argc, char** argv) {
     ros::init(argc, argv, "test_moving_object");
     ros::NodeHandle nh;
-    const std::string config_path = argc > 1 ? argv[1] : "config/MOR_config.txt";
+    std::string config_path = "config/MOR_config.txt";
+    bool keep_fields = false;
+    for (int i = 1; i < argc; i++) {
+        if (std::string(argv[i]) == "--keep-fields") keep_fields = true;
+        else config_path = argv[i];
+    }
     mor.reset(new MovingObjectRemoval(nh, config_path, 4, 3));  // n_bad = 4, n_good = 3 as in external_sync_test.cpp:37
+    if (keep_fields && !mor->setKeepInputFields(true)) { ROS_ERROR("setKeepInputFields: %s", mor_status_string(mor->lastStatus())); return 1; }
     const mor_config& cfg = mor->config();
     pub = nh.advertise<sensor_msgs::PointCloud2>(cfg.output_topic, 10);
     debug_pub = nh.advertise<sensor_msgs::PointCloud2>(cfg.debug_topic, 10);
