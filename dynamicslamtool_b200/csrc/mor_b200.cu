@@ -137,6 +137,9 @@ struct mor_handle {
     // products of the front half that only the back half of the SAME frame reads: two, by frame parity
     int* scid2[2]; float4* gpts2[2]; int* gsrc2[2]; int* cloud_src2[2]; uint8_t* removed_mask2[2];
     unsigned long long* acc_sum2[2]; unsigned* acc_box2[2];
+    // method 1 only: the clustering grid by frame parity (a pipelined back half searches its frame's grid while the front
+    // half of the next frame builds the other one); otherwise both are base.table / base.cell_list
+    Cell* table2[2]; int* cell_list2[2];
     int cur = 0, fpar = 0;
     // pipelining (mor_set_pipelining): the back half of the last filtered frame waits to be launched beside the front half
     // of the next frame
@@ -297,11 +300,13 @@ int allocate(mor_handle* h) {
             h->scid2[f] = f ? carve<int>(p, N) : b.scid; h->gpts2[f] = f ? carve<float4>(p, N) : b.gpts; h->gsrc2[f] = f ? carve<int>(p, N) : b.gsrc;
             h->cloud_src2[f] = f ? carve<int>(p, N) : b.cloud_src; h->removed_mask2[f] = f ? carve<uint8_t>(p, N) : b.removed_mask;
             h->acc_sum2[f] = f ? carve<unsigned long long>(p, K * 6) : b.acc_sum; h->acc_box2[f] = f ? carve<unsigned>(p, K * 6) : b.acc_box;
+            const bool own_grid = f && h->cfg.method_choice == 1;
+            h->table2[f] = own_grid ? carve<Cell>(p, tab) : b.table; h->cell_list2[f] = own_grid ? carve<int>(p, N) : b.cell_list;
         }
         for (int f = 0; f < 3; f++) {
             h->pts[f] = carve<float4>(p, N); h->spts[f] = carve<float4>(p, N); h->cid[f] = carve<int>(p, N);
             h->cl_root[f] = carve<int>(p, K); h->cl_size[f] = carve<int>(p, K); h->cl_centroid[f] = carve<float>(p, K * 3);
-            h->cl_flags[f] = carve<uint8_t>(p, K); h->cl_bbox[f] = carve<float>(p, K * 6); h->counts[f] = carve<int>(p, MOR_NCOUNTS);
+            h->cl_flags[f] = carve<uint8_t>(p, K); h->cl_bbox[f] = carve<float>(p, K * 6); h->counts[f] = carve<int>(p, CNT_ALLOC);
         }
         if (ground) {  // dense ball-query grid and pcl::VoxelGrid index space over the bounding box of raw_cloud
             GroundPtrs& g = h->ground;
@@ -342,6 +347,9 @@ int configure_kernels(mor_handle* h) {
     MOR_CUDA(cudaFuncSetAttribute(k_frame, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
     MOR_CUDA(cudaFuncSetAttribute(k_frame_batch, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
     MOR_CUDA(cudaFuncSetAttribute(k_frame_pipe, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
+    MOR_CUDA(cudaFuncSetAttribute(k_frame_pipe_ground, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
+    MOR_CUDA(cudaFuncSetAttribute(k_frame_pipe_pde, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
+    MOR_CUDA(cudaFuncSetAttribute(k_frame_pipe_ground_pde, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
     int st = set_phase_smem<PH_SELECT>(h);
     if (st == MOR_OK) st = set_phase_smem<PH_LINK>(h);
     if (st == MOR_OK) st = set_phase_smem<PH_STATS>(h);
@@ -412,6 +420,7 @@ void fill_frame(mor_handle* h, const uint8_t* d_points, uint32_t n, uint32_t ste
     const int cur = h->cur, prev = (cur + 2) % 3;
     a.scid = h->scid2[h->fpar]; a.gpts = h->gpts2[h->fpar]; a.gsrc = h->gsrc2[h->fpar]; a.cloud_src = h->cloud_src2[h->fpar]; a.removed_mask = h->removed_mask2[h->fpar];
     a.acc_sum = h->acc_sum2[h->fpar]; a.acc_box = h->acc_box2[h->fpar];
+    a.table = h->table2[h->fpar]; a.cell_list = h->cell_list2[h->fpar];
     a.in = d_points; a.n = n; a.step = step; a.off_x = ox; a.off_y = oy; a.off_z = oz; a.off_i = oi;
     a.in_mode = input_mode(d_points, step, ox, oy, oz, oi);
     a.pts = h->pts[cur]; a.spts = h->spts[cur]; a.cid = h->cid[cur]; a.cl_root = h->cl_root[cur]; a.cl_size = h->cl_size[cur];
@@ -458,19 +467,31 @@ int launch_gather(mor_handle* h, const FramePtrs& a) {
     return MOR_OK;
 }
 
+// The pipelined launch of a handle's configuration (k_frame_pipe and its variants, mor_kernels.cuh), and the share of the
+// CTAs its back half gets, in 32nds.
+struct PipeVariant { void (*kernel)(FramePtrs, FramePtrs, int); const char* name; int back32; };
+PipeVariant pipe_variant(const mor_handle* h) {
+    const bool ground = h->cfg.ground_mode != MOR_GROUND_CROP, pde = h->cfg.method_choice == 1;
+    // 5/32 (23 of 148 CTAs): measured optimum on C2 (swept 100 ... 140: the front half holds two thirds of a frame's chain of
+    // phases and is tile-granular in its first one, the back half is three short phases over the points plus its
+    // single-CTA steps). The variants, swept with tools/pipe_modes_run.py on C4 / C1 / HDL-64 frames (BASELINE.md): the voxel
+    // ground modes have C2's front half after their ground stage and the same optimum; method 1's back half holds the
+    // point-distance search, one thread per point of the previous frame's clusters, and needs 11/32 (50 CTAs) - at 5/32 a
+    // pipelined HDL-64 frame is 30 % slower than one kernel per frame, at 11/32 it is faster on every configuration measured.
+    if (ground) return pde ? PipeVariant{k_frame_pipe_ground_pde, "k_frame_pipe_ground_pde", 11} : PipeVariant{k_frame_pipe_ground, "k_frame_pipe_ground", 5};
+    return pde ? PipeVariant{k_frame_pipe_pde, "k_frame_pipe_pde", 11} : PipeVariant{k_frame_pipe, "k_frame_pipe", 5};
+}
 // Pipelined launches (k_frame_pipe): the front half of `front` on most CTAs beside the pending back half, or either alone.
 int launch_pipe(mor_handle* h, const FramePtrs* front, const FramePtrs* back) {
     const int G = h->frame_ctas;
-    // the back half gets 5/32 of the CTAs (23 of 148): measured optimum on C2 (swept 100 ... 140: the front half holds two thirds
-    // of a frame's chain of phases and is tile-granular in its first one, the back half is three short phases over the
-    // points plus its single-CTA steps)
+    const PipeVariant v = pipe_variant(h);
     int Gf = G, Gb = 0;
     if (front && back && G < 8) {  // too few SMs to share: one half after the other
         int s0 = launch_pipe(h, nullptr, back);
         return s0 != MOR_OK ? s0 : launch_pipe(h, front, nullptr);
     }
     if (front && back) {
-        Gb = (G * 5) / 32;
+        Gb = (G * v.back32) / 32;
         if (Gb < 4) Gb = 4;
         Gf = G - Gb;
         if (const char* env = std::getenv("MOR_PIPE_GF")) { const int v = std::atoi(env); if (v > 0 && v < G) Gf = v; }  // (tuning)
@@ -479,9 +500,9 @@ int launch_pipe(mor_handle* h, const FramePtrs* front, const FramePtrs* back) {
     FramePtrs f = front ? *front : *back, b = back ? *back : *front;
     set_segments(h, f, Gf > 0 ? Gf : G);
     (void)Gb;
-    cudaError_t e = launch_coop(k_frame_pipe, (unsigned)G, h->frame_smem, h->stream, f, b, Gf);
+    cudaError_t e = launch_coop(v.kernel, (unsigned)G, h->frame_smem, h->stream, f, b, Gf);
     h->launches++;
-    if (e != cudaSuccess) { h->last_error = std::string("k_frame_pipe: ") + cudaGetErrorString(e); return MOR_ERR_CUDA; }
+    if (e != cudaSuccess) { h->last_error = std::string(v.name) + ": " + cudaGetErrorString(e); return MOR_ERR_CUDA; }
     return MOR_OK;
 }
 // The back half of the last filtered frame, if it is still waiting for a partner: alone.
@@ -519,8 +540,9 @@ int enqueue_push(mor_handle* h, const uint8_t* d_points, uint32_t n, uint32_t st
             (s = launch_phase<PH_MOVING>(h, a)) || (s = launch_phase<PH_FILTER>(h, a)))
             return s;
         if (h->frame_rec) return launch_gather(h, a);
-    } else if (allow_pipe && h->pipelining && h->cfg.method_choice == 2 && h->cfg.ground_mode == MOR_GROUND_CROP) {
-        // front half of this frame, beside the back half of the frame before if that one has been filtered already
+    } else if (allow_pipe && h->pipelining) {
+        // front half of this frame, beside the back half of the frame before if that one has been filtered already (voxel
+        // ground modes: the ground stage above ran first, see the audit at k_frame_pipe_ground)
         const bool fused = h->back_pending;
         h->back_pending = false;
         int s = launch_pipe(h, &a, fused ? &h->back_frame : nullptr);
@@ -595,7 +617,7 @@ int do_push(mor_handle* h, const void* data, bool on_device, uint32_t n, uint32_
     if (h->out_records && (size_t)n * step > h->d_in_bytes) { h->last_error = "output records: n * point_step exceeds the output buffer (32 B x max_points)"; return MOR_ERR_CAPACITY; }
     h->out_cur = h->slot[0].d_out;
     MOR_CUDA(cudaSetDevice(h->device));
-    { int js = join_foreign_stream(h, on_device && h->pipelining && h->cfg.ground_mode == MOR_GROUND_CROP && !h->profiling); if (js != MOR_OK) return js; }
+    { int js = join_foreign_stream(h, on_device && h->pipelining && !h->profiling); if (js != MOR_OK) return js; }
     if (h->timing) MOR_CUDA(cudaEventRecord(h->ev[0], h->stream));
     if (h->profiling && !h->prof_ids.empty()) { MOR_CUDA(cudaStreamSynchronize(h->stream)); prof_harvest(h); }
     const uint8_t* d_points = (const uint8_t*)data;
@@ -998,7 +1020,7 @@ int mor_submit_frame(mor_handle* h, const void* data, uint32_t n, uint32_t step,
     MOR_CUDA(cudaStreamWaitEvent(h->stream, sl.h2d, 0));
     advance_frame(h, n, pose7);
     h->out_cur = sl.d_out;
-    const bool piped = h->pipelining && h->cfg.method_choice == 2 && h->cfg.ground_mode == MOR_GROUND_CROP;
+    const bool piped = h->pipelining;
     int st = enqueue_push(h, sl.d_in, n, step, ox, oy, oz, oi, /*allow_pipe=*/true);
     if (st != MOR_OK) return st;
     sl.out = out; sl.cap = cap_points; sl.n = n; sl.d_counts = h->frame.counts; sl.used = true; sl.d2h_enqueued = false;

@@ -38,6 +38,9 @@ constexpr size_t kLinkSmem = (size_t)kStageLight * 8 + (size_t)kStageHeavy * 16;
 enum ErrBits { ERR_CLUSTER_CAP = 1, ERR_MOVING_CAP = 2, ERR_LATTICE_RANGE = 4, ERR_GROUND_CAP = 8, ERR_GRID_RANGE = 16, ERR_EDGE_CAP = 32 };
 // counts[] slots in which the filter phase parks its results until filterCloud commits the frame (mor_b200.cu, do_filter)
 enum { CNT_SPEC_NOUT = 21, CNT_SPEC_NMO = 22, CNT_SPEC_OVERFLOW = 23 };
+// A word after the public counts (never copied out): a pipelined method-1 frame's number of clustering cells, from its
+// front half to its back half, which empties the grid after the point-distance search (k_frame_pipe_pde)
+enum { CNT_PIPE_CELLS = MOR_NCOUNTS, CNT_ALLOC = MOR_NCOUNTS + 1 };
 
 // One occupied cell of the clustering grid: open-addressing hash table keyed by the packed cell coordinates.
 // key == 0 is "empty" (every real key has bit 63 set), so a zeroed table is a clean table.
@@ -461,8 +464,8 @@ __device__ __forceinline__ void phase_ingest(const FramePtrs& a, int cta, int G,
 }
 
 // Voxel ground modes: `cloud` already exists (k_ground_partition); only the binning is left to do.
-__device__ __forceinline__ void phase_bin_cloud(const FramePtrs& a, int cta, int G) {
-    frame_housekeeping(a, cta, G);
+__device__ __forceinline__ void phase_bin_cloud(const FramePtrs& a, int cta, int G, bool housekeep = true) {
+    if (housekeep) frame_housekeeping(a, cta, G);
     const int nc = a.counts[MOR_CNT_NC];
     for (int base = cta * kT; base < nc; base += G * kT) {
         const int c = base + threadIdx.x;
@@ -1869,11 +1872,35 @@ __device__ __forceinline__ void frame_body(const FramePtrs& a, int cta, int G, F
 // groups have their own barriers and counters and touch disjoint state: what the back half reads of frame f and f-1 is
 // triple-buffered (points, cluster ids, cluster tables, counts) or double-buffered (ground points, source indices, masks,
 // the clusters' coordinate sums and boxes)
-// on the host side (mor_b200.cu, fill_frame). Method 2 and the crop ground mode only (method 1 searches the clustering
-// grid of frame f in the back half, which the front half of f+1 rebuilds).
+// on the host side (mor_b200.cu, fill_frame).
+// Four instantiations of the same two bodies, picked per handle by mor_b200.cu (pipe_kernel):
+//  - k_frame_pipe: crop ground mode, method 2.
+//  - k_frame_pipe_ground (GROUND): voxel ground modes. Frame f+1's nine ground launches (mor_ground.cuh) run on the stream
+//    before this launch, i.e. after the launch that ran f's front half and before f's back half. What they write, against
+//    what the back half of f reads later:
+//      k_ingest_raw: counts of f+1 (zeroed and filled by its last tile; a slot of the triple-buffered counts, f's slot is
+//        another), track->frames (read by the ingest alone), point_class (per point; read by the front half and the taps of
+//        the current frame, never by a back half), removed_mask (parity of f+1; f's filter marks the other parity), the
+//        Scratch box words and ticket_ingest, st_ingest, bin_hist, rpts / rsrc / is_ground (ground stage only);
+//      k_ground_keys / k_scan_cells / k_ground_scatter: the dense cell_count / cell_start / cell_key / skey tables, vkey,
+//        vox_count, ggrid / vdesc, st_cells, ticket_cells (ground stage only), spts (f+1's slot of three), ERRFLAGS in
+//        the counts of f+1;
+//      k_scan_voxels / k_voxel_eval / k_ground_mode / k_ground_mark: vox_* , vacc, bin_hist, gstate, the scan states and
+//        Scratch tickets and box words they reset (ground stage only);
+//      k_ground_partition: point_class, pts (slot of f+1), cloud_src / gpts / gsrc (parity of f+1), counts of f+1.
+//    None of these is read by the back half of f (it reads f's and f-1's slots, f's parity, the tracking state, st_out
+//    and its own Scratch words), so f's back half sees what it would have seen without the ground stage in between. The
+//    front half starts at the binning (phase_bin_cloud, no housekeeping: the back half does that) and gives back the
+//    ticket that k_ground_partition leaves drawn.
+//  - k_frame_pipe_pde (PDE): method 1. Its moving test searches frame f's clustering grid in the back half, so a method-1
+//    handle keeps the grid (table, cell_list) per frame parity; the front half leaves it standing and hands its cell
+//    count over in counts[CNT_PIPE_CELLS]; the back half empties it after the search.
+//  - k_frame_pipe_ground_pde: both.
+template <bool GROUND = false, bool PDE = false>
 __device__ __forceinline__ void front_body(const FramePtrs& a, int cta, int G, FrameShared& sh, unsigned long long* dyn, unsigned& parity) {
     GroupBarrier bar{&a.scratch->bar, 0u, (unsigned)G};
-    phase_ingest(a, cta, G, dyn, &sh.mbar, parity, /*housekeep=*/false);
+    if (GROUND) phase_bin_cloud(a, cta, G, /*housekeep=*/false);
+    else phase_ingest(a, cta, G, dyn, &sh.mbar, parity, /*housekeep=*/false);
     bar.sync();
     load_frame_vars(a);
     phase_cells(a, cta, G); bar.sync();
@@ -1885,7 +1912,12 @@ __device__ __forceinline__ void front_body(const FramePtrs& a, int cta, int G, F
     if (group_last_arrival(&a.scratch->tail_centroids, (unsigned)G)) phase_select(a, dyn);  // (the last CTA in selects the clusters: no barrier in front of it)
     bar.sync();
     phase_stats(a, cta, G);  // (the sums it accumulates are double-buffered by frame parity: the back half turns them into centroids)
-    frame_cleanup(a, cta, G);
+    if (PDE) {  // the grid stays for the back half's search: only the scan states go back to zero here
+        for (int t = cta * kT + threadIdx.x; t < a.tiles_pts; t += G * kT) a.st_ingest[t] = 0ull;
+        if (cta == 0 && threadIdx.x == 0) a.counts[CNT_PIPE_CELLS] = frame_vars().n_cells;
+    } else {
+        frame_cleanup(a, cta, G);
+    }
     // last CTA of the group out: the front half's counters back to zero
     __shared__ int s_last_front;
     __syncthreads();
@@ -1899,9 +1931,13 @@ __device__ __forceinline__ void front_body(const FramePtrs& a, int cta, int G, F
         Scratch* sc = a.scratch;
         sc->bar = 0u; sc->blocks_done = 0; sc->n_cells = 0; sc->n_roots = 0; sc->n_light = 0; sc->n_heavy = 0; sc->n_sorted = 0; sc->tail_centroids = 0u;
         sc->ticket_light = 0; sc->ticket_heavy = 0; sc->err_early = 0;
+        if (GROUND) sc->ticket_ingest = 0;  // (drawn by k_ground_partition; frame_epilogue resets it in one kernel per frame)
     }
 }
 
+// (GROUND does not change the back half; it keeps every kernel's instantiations of the two bodies its own, so that their
+// static shared variables stay local to one kernel and k_frame_pipe's shared layout is what it was before the variants)
+template <bool GROUND = false, bool PDE = false>
 __device__ __forceinline__ void back_body(const FramePtrs& a, int cta, int G, FrameShared& sh, unsigned long long* dyn) {
     GroupBarrier bar{&a.scratch->bar_back, 0u, (unsigned)G};
     if (threadIdx.x == 0) {  // (the cell count belongs to the front half, which is busy with the next frame)
@@ -1918,9 +1954,14 @@ __device__ __forceinline__ void back_body(const FramePtrs& a, int cta, int G, Fr
     }
     if (group_last_arrival(&a.scratch->tail_match_back, (unsigned)G)) phase_match(a, dyn);
     bar.sync();
-    if (a.two_frames) phase_lattice_count(a, cta, G);
+    if (a.two_frames) { if (PDE) phase_pde_count(a, cta, G); else phase_lattice_count(a, cta, G); }
     if (group_last_arrival(&a.scratch->tail_chain, (unsigned)G)) phase_chain_tail(a);
     bar.sync();
+    if (PDE) {  // the search is over: this frame's clustering grid goes back to "all zero" (frame_cleanup's first loop)
+        const int n_cells = a.counts[CNT_PIPE_CELLS];
+        for (int i = cta * kT + threadIdx.x; i < n_cells; i += G * kT)
+            *reinterpret_cast<uint4*>(a.table + a.cell_list[i]) = make_uint4(0u, 0u, 0u, 0u);
+    }
     phase_filter(a, cta, G, sh.filter, /*cleanup=*/false);
     __shared__ int s_last_back;
     __syncthreads();
@@ -1947,6 +1988,27 @@ __global__ void __launch_bounds__(kT, 1) k_frame_pipe(const __grid_constant__ Fr
     unsigned parity = 0;
     if ((int)blockIdx.x < Gf) front_body(f, blockIdx.x, Gf, sh, dyn, parity);
     else back_body(b, (int)blockIdx.x - Gf, (int)gridDim.x - Gf, sh, dyn);
+}
+
+// The other configurations: the same launch with the variants of the two bodies described above.
+template <bool GROUND, bool PDE>
+__device__ __forceinline__ void frame_pipe_variant(const FramePtrs& f, const FramePtrs& b, int Gf) {
+    extern __shared__ __align__(128) unsigned long long dyn[];
+    __shared__ FrameShared sh;
+    if (threadIdx.x == 0) mbar_init(&sh.mbar, 1);
+    __syncthreads();
+    unsigned parity = 0;
+    if ((int)blockIdx.x < Gf) front_body<GROUND, PDE>(f, blockIdx.x, Gf, sh, dyn, parity);
+    else back_body<GROUND, PDE>(b, (int)blockIdx.x - Gf, (int)gridDim.x - Gf, sh, dyn);
+}
+__global__ void __launch_bounds__(kT, 1) k_frame_pipe_ground(const __grid_constant__ FramePtrs f, const __grid_constant__ FramePtrs b, int Gf) {
+    frame_pipe_variant<true, false>(f, b, Gf);
+}
+__global__ void __launch_bounds__(kT, 1) k_frame_pipe_pde(const __grid_constant__ FramePtrs f, const __grid_constant__ FramePtrs b, int Gf) {
+    frame_pipe_variant<false, true>(f, b, Gf);
+}
+__global__ void __launch_bounds__(kT, 1) k_frame_pipe_ground_pde(const __grid_constant__ FramePtrs f, const __grid_constant__ FramePtrs b, int Gf) {
+    frame_pipe_variant<true, true>(f, b, Gf);
 }
 
 // One sequence, the whole grid is its group; the frame's arguments travel in the constant bank.

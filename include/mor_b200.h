@@ -163,7 +163,9 @@ int mor_collect_frame(mor_handle* h, uint32_t* n_out);
  * frame f (pose transform, correspondences, moving test, chain, filterCloud's part) is launched together with the front
  * half of frame f+1 (ingest ... cluster statistics), in ONE kernel on disjoint groups of SMs, instead of one after the
  * other. Results are identical; a call that needs a frame's results (count, taps, host output) runs its back half at
- * once. Applies to method_choice 2 with the crop ground mode; ignored otherwise. Off by default. */
+ * once. Applies to every configuration: with ground_mode 1/2 the frame's nine ground-stage launches come first, then
+ * the one pipelined launch; with method_choice 1 the handle keeps a second clustering grid, so the back half of frame f
+ * can search f's grid while the front half of f+1 builds its own. Off by default. */
 int mor_set_pipelining(mor_handle* h, int enabled);
 /* Output records, off by default: every output path above (mor_filter_cloud, mor_filter_cloud_device and
  * mor_get_output_device, mor_submit_frame / mor_collect_frame, mor_batch_step_device) delivers output point o as a
