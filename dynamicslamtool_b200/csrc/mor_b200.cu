@@ -321,6 +321,9 @@ int allocate(mor_handle* h) {
         }
         b.track = carve<TrackState>(p, 1); b.mo_centroid = carve<float>(p, 2 * MO * 3); b.mo_conf = carve<int>(p, 2 * MO);
         b.res_ring = carve<uint8_t>(p, D * K); b.res_len = carve<int>(p, D); b.corr_ring = carve<int>(p, D * K); b.corr_len = carve<int>(p, D);
+        const size_t KL = K > (size_t)kSmallK ? K : 0;  // the large-K path's arrays: only where kmax allows such frames
+        b.sort_keys = KL ? carve<unsigned long long>(p, 2 * KL) : nullptr;
+        b.nn_cur = KL ? carve<int>(p, KL) : nullptr; b.nn_dist = KL ? carve<float>(p, KL) : nullptr; b.nn_prev = KL ? carve<int>(p, KL) : nullptr;
         h->rec_st = carve<unsigned long long>(p, N / kRecT + 2); h->rec_ctr = carve<int>(p, 2);
         return p;
     };
@@ -330,34 +333,46 @@ int allocate(mor_handle* h) {
     MOR_CUDA(cudaMallocHost(&h->h_counts, sizeof(int32_t) * MOR_NCOUNTS));
     for (int i = 0; i < 4; i++) MOR_CUDA(cudaEventCreate(&h->ev[i]));
     // dynamic shared memory of the frame kernel: the link phase's point tile + neighbour lists, or the cluster sort keys
-    // of the select phase
+    // of the select phase (at most kSmallK of them: a frame with more sorts runs of kSmallK keys, and its match and filter
+    // take candidate tiles of kNnTile centroids, 64 KB)
     int P = 1;
-    while (P < (int)K) P <<= 1;
+    while (P < (int)K && P < kSmallK) P <<= 1;
     h->frame_smem = (size_t)P * sizeof(unsigned long long);
     if (h->frame_smem < kLinkSmem) h->frame_smem = kLinkSmem;
     return MOR_OK;
 }
 
-template <int PH>
+// A handle whose max_clusters exceeds kSmallK runs the frame kernels' LK instantiations (the group-wide large-K steps);
+// every other handle the instantiations without them.
+inline bool large_k(const mor_handle* h) { return h->kmax > (uint32_t)kSmallK; }
+
+template <int PH, bool LK>
 int set_phase_smem(mor_handle* h) {
-    MOR_CUDA(cudaFuncSetAttribute(k_phase<PH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
+    MOR_CUDA(cudaFuncSetAttribute(k_phase<PH, LK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
     return MOR_OK;
 }
+template <bool LK>
+int configure_frame_kernels(mor_handle* h) {
+    MOR_CUDA(cudaFuncSetAttribute(k_frame<LK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
+    MOR_CUDA(cudaFuncSetAttribute(k_frame_batch<LK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
+    MOR_CUDA(cudaFuncSetAttribute(k_frame_pipe<LK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
+    MOR_CUDA(cudaFuncSetAttribute(k_frame_pipe_ground<LK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
+    MOR_CUDA(cudaFuncSetAttribute(k_frame_pipe_pde<LK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
+    MOR_CUDA(cudaFuncSetAttribute(k_frame_pipe_ground_pde<LK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
+    int st = set_phase_smem<PH_SELECT, LK>(h);
+    if (st == MOR_OK) st = set_phase_smem<PH_FILTER, LK>(h);
+    if (st == MOR_OK) st = set_phase_smem<PH_LINK, LK>(h);
+    if (st == MOR_OK) st = set_phase_smem<PH_STATS, LK>(h);
+    if (st == MOR_OK) st = set_phase_smem<PH_INGEST, LK>(h);
+    return st;
+}
 int configure_kernels(mor_handle* h) {
-    MOR_CUDA(cudaFuncSetAttribute(k_frame, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
-    MOR_CUDA(cudaFuncSetAttribute(k_frame_batch, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
-    MOR_CUDA(cudaFuncSetAttribute(k_frame_pipe, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
-    MOR_CUDA(cudaFuncSetAttribute(k_frame_pipe_ground, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
-    MOR_CUDA(cudaFuncSetAttribute(k_frame_pipe_pde, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
-    MOR_CUDA(cudaFuncSetAttribute(k_frame_pipe_ground_pde, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
-    int st = set_phase_smem<PH_SELECT>(h);
-    if (st == MOR_OK) st = set_phase_smem<PH_LINK>(h);
-    if (st == MOR_OK) st = set_phase_smem<PH_STATS>(h);
-    if (st == MOR_OK) st = set_phase_smem<PH_INGEST>(h);
+    if (large_k(h)) MOR_CUDA(cudaFuncSetAttribute(k_filter_markers, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kNnTile * sizeof(float4))));
+    const int st = large_k(h) ? configure_frame_kernels<true>(h) : configure_frame_kernels<false>(h);
     if (st != MOR_OK) return st;
     int sms = 0, per_sm = 0;
     if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device) == cudaSuccess && sms > 0) h->num_sms = sms;
-    MOR_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_frame, kT, h->frame_smem));
+    MOR_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, large_k(h) ? k_frame<true> : k_frame<false>, kT, h->frame_smem));
     if (per_sm < 1) { h->last_error = "the frame kernel does not fit on an SM of this device"; return MOR_ERR_CUDA; }
     h->frame_ctas = h->num_sms;  // one CTA per SM
     return MOR_OK;
@@ -437,8 +452,8 @@ void fill_frame(mor_handle* h, const uint8_t* d_points, uint32_t n, uint32_t ste
 template <int PH>
 int launch_phase(mor_handle* h, const FramePtrs& a) {
     prof_begin(h, KID_PHASE0 + PH);
-    const size_t smem = (PH == PH_INGEST || PH == PH_SELECT || PH == PH_LINK || PH == PH_STATS) ? h->frame_smem : 0;
-    cudaError_t e = launch_coop(k_phase<PH>, (unsigned)h->frame_ctas, smem, h->stream, a);
+    const size_t smem = (PH == PH_INGEST || PH == PH_SELECT || PH == PH_LINK || PH == PH_STATS || PH == PH_FILTER) ? h->frame_smem : 0;
+    cudaError_t e = launch_coop(large_k(h) ? k_phase<PH, true> : k_phase<PH, false>, (unsigned)h->frame_ctas, smem, h->stream, a);
     prof_end(h);
     h->launches++;
     if (e != cudaSuccess) { h->last_error = std::string("k_phase: ") + cudaGetErrorString(e); return MOR_ERR_CUDA; }
@@ -478,8 +493,11 @@ PipeVariant pipe_variant(const mor_handle* h) {
     // ground modes have C2's front half after their ground stage and the same optimum; method 1's back half holds the
     // point-distance search, one thread per point of the previous frame's clusters, and needs 11/32 (50 CTAs) - at 5/32 a
     // pipelined HDL-64 frame is 30 % slower than one kernel per frame, at 11/32 it is faster on every configuration measured.
-    if (ground) return pde ? PipeVariant{k_frame_pipe_ground_pde, "k_frame_pipe_ground_pde", 11} : PipeVariant{k_frame_pipe_ground, "k_frame_pipe_ground", 5};
-    return pde ? PipeVariant{k_frame_pipe_pde, "k_frame_pipe_pde", 11} : PipeVariant{k_frame_pipe, "k_frame_pipe", 5};
+    const bool lk = large_k(h);
+    if (ground) return pde ? PipeVariant{lk ? k_frame_pipe_ground_pde<true> : k_frame_pipe_ground_pde<false>, "k_frame_pipe_ground_pde", 11}
+                           : PipeVariant{lk ? k_frame_pipe_ground<true> : k_frame_pipe_ground<false>, "k_frame_pipe_ground", 5};
+    return pde ? PipeVariant{lk ? k_frame_pipe_pde<true> : k_frame_pipe_pde<false>, "k_frame_pipe_pde", 11}
+               : PipeVariant{lk ? k_frame_pipe<true> : k_frame_pipe<false>, "k_frame_pipe", 5};
 }
 // Pipelined launches (k_frame_pipe): the front half of `front` on most CTAs beside the pending back half, or either alone.
 int launch_pipe(mor_handle* h, const FramePtrs* front, const FramePtrs* back) {
@@ -552,7 +570,7 @@ int enqueue_push(mor_handle* h, const uint8_t* d_points, uint32_t n, uint32_t st
         h->back_rec = h->frame_rec;
         h->back_pending = true;
     } else {
-        cudaError_t e = launch_coop(k_frame, (unsigned)h->frame_ctas, h->frame_smem, st, a);
+        cudaError_t e = launch_coop(large_k(h) ? k_frame<true> : k_frame<false>, (unsigned)h->frame_ctas, h->frame_smem, st, a);
         h->launches++;
         if (e != cudaSuccess) { h->last_error = std::string("k_frame: ") + cudaGetErrorString(e); return MOR_ERR_CUDA; }
         if (h->frame_rec) return launch_gather(h, a);
@@ -654,7 +672,12 @@ int do_filter(mor_handle* h, void* out, bool on_device, uint32_t cap_points, uin
     if (h->filtered) {  // repeated call: the tracking update runs once more
         a.mo_parity = h->mo_parity;
         prof_begin(h, KID_FILTER_AGAIN);
-        k_filter_again<<<h->n_input ? (h->n_input + kOutTile - 1) / kOutTile : 1, kT, 0, st>>>(a);
+        if (large_k(h)) {  // (a frame with more than kSmallK clusters: markers and removal set first)
+            k_filter_markers<<<h->num_sms, kT, kNnTile * sizeof(float4), st>>>(a);
+            k_filter_mark<<<h->num_sms, kT, 0, st>>>(a);
+            h->launches += 2;
+        }
+        (large_k(h) ? k_filter_again<true> : k_filter_again<false>)<<<h->n_input ? (h->n_input + kOutTile - 1) / kOutTile : 1, kT, 0, st>>>(a);
         prof_end(h);
         h->launches++;
         MOR_CUDA(cudaGetLastError());
@@ -745,7 +768,8 @@ int mor_create_ex(const char* config_path, int n_bad, int n_good, int device, co
     h->kmax = limits && limits->max_clusters ? limits->max_clusters : 8192u;
     h->momax = limits && limits->max_moving ? limits->max_moving : 1024u;
     h->max_cells = limits && limits->max_cells ? (int)(limits->max_cells > 0x40000000u ? 0x40000000u : limits->max_cells) : (1 << 24);
-    if (h->kmax > 16384u) h->kmax = 16384u;  // the select phase sorts the clusters of a frame in shared memory (128 KB of keys)
+    // a frame has at most max_points clusters (values up to kSmallK are kept as they are, as before the large-K path)
+    if (h->kmax > (uint32_t)kSmallK && h->kmax > h->nmax) h->kmax = h->nmax > (uint32_t)kSmallK ? h->nmax : (uint32_t)kSmallK;
     h->ring_depth = (n_bad > 1 ? n_bad : 1) + 2;
     st = build_grid(h);
     if (st != MOR_OK) { delete h; return st; }
@@ -924,7 +948,7 @@ int mor_batch_step_device(mor_handle* const* hs, uint32_t S, const void* const* 
         if (gs != MOR_OK) return gs;
     }
     {
-        cudaError_t e = launch_coop(k_frame_batch, (unsigned)(groups * G), h->frame_smem, st, (const FramePtrs*)dp, (int)S, G);
+        cudaError_t e = launch_coop(large_k(h) ? k_frame_batch<true> : k_frame_batch<false>, (unsigned)(groups * G), h->frame_smem, st, (const FramePtrs*)dp, (int)S, G);
         h->launches++;
         if (e != cudaSuccess) { h->last_error = std::string("k_frame_batch: ") + cudaGetErrorString(e); return MOR_ERR_CUDA; }
     }

@@ -34,6 +34,10 @@ constexpr int kLightCnt = 32;    // ... and with at most this many points in eit
 #endif
 constexpr int kStageLight = MOR_STAGE_LIGHT, kStageHeavy = MOR_STAGE_HEAVY;  // pair records a CTA collects in shared memory before they go to the lists (24 + 8 KB)
 constexpr size_t kLinkSmem = (size_t)kStageLight * 8 + (size_t)kStageHeavy * 16;
+// Clusters per frame that the single-CTA steps take (select: sort keys in shared memory, 128 KB; filter: the removal
+// bitset). A frame with more runs the group-wide steps of the large-K path instead (phase_select_large, phase_match_large,
+// the LARGE filter).
+constexpr int kSmallK = 16384;
 
 enum ErrBits { ERR_CLUSTER_CAP = 1, ERR_MOVING_CAP = 2, ERR_LATTICE_RANGE = 4, ERR_GROUND_CAP = 8, ERR_GRID_RANGE = 16, ERR_EDGE_CAP = 32 };
 // counts[] slots in which the filter phase parks its results until filterCloud commits the frame (mor_b200.cu, do_filter)
@@ -66,7 +70,7 @@ struct Scratch {  // all zero between frames: every counter is put back by the f
     int ticket_light, ticket_heavy;   // next unclaimed record of the pair lists (test phase)
     int ticket_out, out_blocks_done;  // stand-alone filter kernel (repeated filterCloud on one frame)
     int err_early;           // error bits raised before the frame's counts exist
-    int pad0;
+    int n_sel;               // size-valid clusters found by the group-wide select (phase_select_large)
     // voxel ground modes only
     int ticket_ingest, ticket_cells;
     unsigned box_inv_min[3], box_max[3];  // bbox of raw_cloud (ordered keys; mins stored inverted so 0 is neutral)
@@ -141,6 +145,10 @@ struct FramePtrs {
     unsigned lattice_words16;    // lattice size in 16-byte units
     // ---- voxel ground modes only (mor_ground.cuh): dense ball-query grid
     int* cell_count; int* cell_start; int* cell_key; int* skey; GridDesc* dgrid; unsigned long long* st_cells; int tiles_cells; int max_cells;
+    // ---- frames with more than kSmallK clusters (handles with kmax > kSmallK only; null otherwise)
+    unsigned long long* sort_keys;  // [2 kmax] the select's keys, ping-pong of the merge rounds
+    int* nn_cur; float* nn_dist;    // [kmax] per previous cluster: nearest current cluster, its squared distance
+    int* nn_prev;                   // [kmax] per current cluster: nearest previous cluster
 };
 
 __device__ __forceinline__ unsigned long long global_ns() {
@@ -306,11 +314,20 @@ __device__ __forceinline__ void cell_list_append_warp(const FramePtrs& a, bool c
 // floor((p - anchor)/res) in double, anchored at its first point (PCL 1.8 adoptBoundingBoxToPoint + getKeyBitSize, see
 // DESIGN.md); the occupied leaves of every transformed previous cluster go into one global hash set keyed
 // (prev cluster, ix, iy, iz).
-__device__ __forceinline__ bool lattice_key(const double* anchor3, int k, float x, float y, float z, unsigned long long* key) {
+// A previous frame with more clusters than the 16-bit cluster field holds takes the wide key: 25 bits of cluster (any
+// K < 2^25 = the largest max_points) and 13 bits per axis, +-409.6 m around the anchor; beyond either range the frame is
+// flagged (ERR_LATTICE_RANGE).
+constexpr int kLatticeNarrowK = 65535;
+__device__ __forceinline__ bool lattice_key(const double* anchor3, int k, float x, float y, float z, unsigned long long* key, bool wide) {
     const double res = (double)0.1f;
     const long long ix = (long long)floor(((double)x - anchor3[0]) / res);
     const long long iy = (long long)floor(((double)y - anchor3[1]) / res);
     const long long iz = (long long)floor(((double)z - anchor3[2]) / res);
+    if (wide) {
+        *key = ((unsigned long long)(unsigned)k << 39) | ((unsigned long long)(ix + 4096) << 26) | ((unsigned long long)(iy + 4096) << 13) |
+               (unsigned long long)(iz + 4096);
+        return ix >= -4096 && ix < 4096 && iy >= -4096 && iy < 4096 && iz >= -4096 && iz < 4096;
+    }
     const bool ok = ix >= -32768 && ix < 32768 && iy >= -32768 && iy < 32768 && iz >= -32768 && iz < 32768;
     *key = ((unsigned long long)(unsigned)k << 48) | ((unsigned long long)(ix + 32768) << 32) | ((unsigned long long)(iy + 32768) << 16) |
            (unsigned long long)(iz + 32768);
@@ -605,7 +622,9 @@ __device__ __forceinline__ void block_cluster_accumulate(unsigned long long* acc
 // pcl_ros::transformPointCloud of every previous-frame cluster (cpp:544-551, A12), the bounding box of the transformed
 // points (getMinMax3D runs after the transform, cpp:272) and, for method 2, their octree leaves (cpp:319-324). Depends
 // on the previous frame only: it runs beside the single-CTA cluster selection, on the CTAs that one does not need.
+template <bool LK>
 __device__ __forceinline__ void transform_range(const FramePtrs& a, int lo, int hi) {
+    const bool wide = LK && a.p_counts[MOR_CNT_K] > kLatticeNarrowK;
     for (int base = lo; base < hi; base += kT) {
         const int s = base + threadIdx.x;
         int k = -1;
@@ -619,7 +638,7 @@ __device__ __forceinline__ void transform_range(const FramePtrs& a, int lo, int 
                 a.tpts[c] = make_float4(t.x, t.y, t.z, __int_as_float(k));
                 if (a.method == 2) {
                     unsigned long long key;
-                    if (lattice_key(a.anchorp + (size_t)k * 3, k, t.x, t.y, t.z, &key)) hset_insert(a.lattice, a.lattice_mask, key);
+                    if (lattice_key(a.anchorp + (size_t)k * 3, k, t.x, t.y, t.z, &key, wide)) hset_insert(a.lattice, a.lattice_mask, key);
                     else atomicOr(&a.scratch->err_early, ERR_LATTICE_RANGE);
                 }
             } else {
@@ -629,11 +648,12 @@ __device__ __forceinline__ void transform_range(const FramePtrs& a, int lo, int 
         block_cluster_accumulate<false>(nullptr, a.pacc_box, k, k >= 0, t.x, t.y, t.z);
     }
 }
+template <bool LK>
 __device__ __forceinline__ void phase_transform(const FramePtrs& a, int cta, int G) {
     if (!a.two_frames || (G > 1 && cta == 0)) return;  // CTA 0 selects the clusters meanwhile
     int lo, hi;
     cta_slice(a.p_counts[MOR_CNT_NC], G > 1 ? cta - 1 : 0, G > 1 ? G - 1 : 1, &lo, &hi);
-    transform_range(a, lo, hi);
+    transform_range<LK>(a, lo, hi);
 }
 
 
@@ -1106,6 +1126,22 @@ __device__ __forceinline__ void phase_roots(const FramePtrs& a, int cta, int G) 
     }
 }
 
+// Ascending sort of Pk (a power of two) keys in shared memory by the whole CTA.
+__device__ __forceinline__ void bitonic_sort_smem(unsigned long long* keys, int Pk) {
+    for (int size = 2; size <= Pk; size <<= 1) {
+        for (int stride = size >> 1; stride > 0; stride >>= 1) {
+            for (int t = threadIdx.x; t < (Pk >> 1); t += kT) {
+                const int lo = 2 * t - (t & (stride - 1));
+                const int hi = lo + stride;
+                const bool up = ((lo & size) == 0);
+                const unsigned long long A = keys[lo], B = keys[hi];
+                if ((A > B) == up) { keys[lo] = B; keys[hi] = A; }
+            }
+            __syncthreads();
+        }
+    }
+}
+
 MOR_OUTLINE void phase_select(const FramePtrs& a, unsigned long long* keys) {
     __shared__ int s_k;
     const int n_roots = __ldcg(&a.scratch->n_roots);
@@ -1132,18 +1168,7 @@ MOR_OUTLINE void phase_select(const FramePtrs& a, unsigned long long* keys) {
     while (Pk < K) Pk <<= 1;
     for (int t = K + threadIdx.x; t < Pk; t += kT) keys[t] = ~0ull;
     __syncthreads();
-    for (int size = 2; size <= Pk; size <<= 1) {
-        for (int stride = size >> 1; stride > 0; stride >>= 1) {
-            for (int t = threadIdx.x; t < (Pk >> 1); t += kT) {
-                const int lo = 2 * t - (t & (stride - 1));
-                const int hi = lo + stride;
-                const bool up = ((lo & size) == 0);
-                const unsigned long long A = keys[lo], B = keys[hi];
-                if ((A > B) == up) { keys[lo] = B; keys[hi] = A; }
-            }
-            __syncthreads();
-        }
-    }
+    bitonic_sort_smem(keys, Pk);
     int nk = 0;
     for (int k = threadIdx.x; k < K; k += kT) {
         const unsigned long long kk = keys[k];
@@ -1166,6 +1191,92 @@ MOR_OUTLINE void phase_select(const FramePtrs& a, unsigned long long* keys) {
     if (threadIdx.x == 0) {
         a.counts[MOR_CNT_K] = K;
         const int e = __ldcg(&a.scratch->err_early);
+        if (e) atomicOr(&a.counts[MOR_CNT_ERRFLAGS], e);
+    }
+}
+
+// ---- large-K path of the select (out of line, like the other large-K steps: the frame kernels run at their register
+// limit, and these rare steps should not add to it). Taken when the handle's kmax and the frame's root count (an upper bound on the
+// size-valid clusters; final after the roots barrier, so every CTA of the group reads the same value) both exceed kSmallK.
+template <bool LK>
+__device__ __forceinline__ bool select_large(const FramePtrs& a) {
+    return LK && __ldcg(&a.scratch->n_roots) > kSmallK;
+}
+// The same selection and order as phase_select, by the whole group: the size-valid keys go to a global array (capacity
+// exceeded: the first kmax found are kept and the frame is flagged, as in phase_select), runs of up to kSmallK keys are
+// sorted in shared memory (bitonic), then merged in pairs between group barriers - every key finds its place by a binary
+// search in the other run (the keys are unique: the labels are). Every CTA must call; writes what phase_select writes.
+__device__ __noinline__ void phase_select_large(const FramePtrs& a, int cta, int G, unsigned long long* dyn, GroupBarrier& bar) {
+    const int n_roots = __ldcg(&a.scratch->n_roots);
+    const int gtid = cta * kT + threadIdx.x, stride = G * kT;
+    unsigned long long* src = a.sort_keys;
+    unsigned long long* dst = a.sort_keys + a.kmax;
+    for (int t = gtid; t < n_roots; t += stride) {
+        const int i = __ldcg(&a.root_list[t]);
+        const int sz = __ldcg(&a.rsize[i]), lab = __ldcg(&a.rmin[i]);
+        if ((long long)sz >= a.min_cluster && (long long)sz <= a.max_cluster) {
+            const int slot = atomicAdd(&a.scratch->n_sel, 1);
+            if (slot < a.kmax) src[slot] = ((unsigned long long)(0xFFFFFFFFu - (unsigned)sz) << 32) | (unsigned)lab;
+            else a.cid_of_root[lab] = -1;
+        } else {
+            a.cid_of_root[lab] = -1;
+        }
+    }
+    bar.sync();
+    const int found = __ldcg(&a.scratch->n_sel);
+    const int K = min(found, a.kmax);
+    int R = kSmallK;  // run length: what the dynamic shared memory holds
+    while ((size_t)R * sizeof(unsigned long long) > (size_t)a.frame_smem) R >>= 1;
+    for (int r = cta; (long long)r * R < K; r += G) {
+        const int b0 = r * R, len = min(R, K - b0);
+        int Pk = 1;
+        while (Pk < len) Pk <<= 1;
+        for (int t = threadIdx.x; t < Pk; t += kT) dyn[t] = t < len ? __ldcg(&src[b0 + t]) : ~0ull;
+        __syncthreads();
+        bitonic_sort_smem(dyn, Pk);
+        for (int t = threadIdx.x; t < len; t += kT) src[b0 + t] = dyn[t];
+        __syncthreads();
+    }
+    for (int w = R; w < K; w <<= 1) {
+        bar.sync();
+        for (int e = gtid; e < K; e += stride) {
+            const unsigned long long x = __ldcg(&src[e]);
+            const int b = e / (2 * w) * (2 * w);
+            const bool in_a = e < b + w;
+            const int o0 = in_a ? min(b + w, K) : b, o1 = in_a ? min(b + 2 * w, K) : b + w;  // the other run
+            int lo = o0, hi = o1;
+            while (lo < hi) {
+                const int mid = (lo + hi) >> 1;
+                if (__ldcg(&src[mid]) < x) lo = mid + 1; else hi = mid;
+            }
+            dst[b + (e - (in_a ? b : b + w)) + (lo - o0)] = x;
+        }
+        unsigned long long* t = src; src = dst; dst = t;
+    }
+    bar.sync();
+    int nk = 0;
+    for (int k = gtid; k < K; k += stride) {
+        const unsigned long long kk = __ldcg(&src[k]);
+        const int root = (int)(unsigned)(kk & 0xFFFFFFFFull);
+        const int sz = (int)(0xFFFFFFFFu - (unsigned)(kk >> 32));
+        a.cl_root[k] = root; a.cl_size[k] = sz; a.cid_of_root[root] = k; a.cl_flags[k] = 0;
+        nk += sz;
+#pragma unroll
+        for (int q = 0; q < 6; q++) a.acc_sum[k * 6 + q] = 0ull;
+#pragma unroll
+        for (int q = 0; q < 3; q++) { a.acc_box[k * 6 + q] = 0xFFFFFFFFu; a.acc_box[k * 6 + 3 + q] = 0u; }
+    }
+    nk = __reduce_add_sync(kFull, nk);
+    if ((threadIdx.x & 31) == 0 && nk) atomicAdd(&a.counts[MOR_CNT_NK], nk);
+    bar.sync();
+    for (int t = gtid; t < n_roots; t += stride) {
+        const int i = __ldcg(&a.root_list[t]);
+        a.cid_of_pos[i] = __ldcg(&a.cid_of_root[__ldcg(&a.rmin[i])]);
+    }
+    if (gtid == 0) {
+        a.counts[MOR_CNT_K] = K;
+        int e = __ldcg(&a.scratch->err_early);
+        if (found > a.kmax) e |= ERR_CLUSTER_CAP;
         if (e) atomicOr(&a.counts[MOR_CNT_ERRFLAGS], e);
     }
 }
@@ -1385,13 +1496,137 @@ MOR_OUTLINE void phase_match(const FramePtrs& a, unsigned long long* dyn) {
     const int cap = (a.frame_smem - kSingle * 12) / kMatchBytesPerCluster;
     if (K <= cap && Kp <= cap) phase_match_impl<true>(a, dyn); else phase_match_impl<false>(a, dyn);
 }
+
+// ---- large-K path of the match: taken when either frame has more than kSmallK clusters (both counts are final before
+// the match, so the choice is the same in every CTA of the group).
+template <bool LK>
+__device__ __forceinline__ bool match_large(const FramePtrs& a) {
+    return LK && (__ldcg(&a.counts[MOR_CNT_K]) > kSmallK || (a.two_frames && __ldcg(&a.p_counts[MOR_CNT_K]) > kSmallK));
+}
+// Nearest neighbour of up to kNnQ queries (q0 ... q0 + nq - 1 of qpts, [.][3]) among the n points cand ([n][3]), by one
+// CTA: the candidates pass through shared memory in tiles of kNnTile, and each quarter of the CTA scans its own quarter of
+// every tile for all queries. Equal distances go to the lowest index, like nn_warp and the reference's linear scan (a
+// quarter scans its indices in ascending order, the quarters are merged by index); -1 / FLT_MAX if no candidate compares
+// below FLT_MAX. Results to out_k[q0 + u] (and out_d). tile: kNnTile float4 of shared memory. Every thread must call.
+constexpr int kNnQ = 256, kNnParts = kT / kNnQ, kNnTile = 4096;
+__device__ __forceinline__ void nn_chunk(const float* qpts, int q0, int nq, const float* cand, int n, float4* tile, int* out_k, float* out_d) {
+    const int u = threadIdx.x % kNnQ, part = threadIdx.x / kNnQ;
+    float qx = 0.f, qy = 0.f, qz = 0.f;
+    if (u < nq) { qx = __ldcg(qpts + (size_t)(q0 + u) * 3); qy = __ldcg(qpts + (size_t)(q0 + u) * 3 + 1); qz = __ldcg(qpts + (size_t)(q0 + u) * 3 + 2); }
+    int best = -1;
+    float bd = 3.402823466e+38f;
+    for (int t0 = 0; t0 < n; t0 += kNnTile) {
+        const int m = min(kNnTile, n - t0);
+        __syncthreads();  // the previous tile's readers are done
+        for (int t = threadIdx.x; t < m; t += kT) {
+            const float* c = cand + (size_t)(t0 + t) * 3;
+            tile[t] = make_float4(__ldcg(c), __ldcg(c + 1), __ldcg(c + 2), 0.f);
+        }
+        __syncthreads();
+        const int hi = min(m, (part + 1) * (kNnTile / kNnParts));
+        for (int i = part * (kNnTile / kNnParts); i < hi; i++) {
+            const float4 c = tile[i];
+            const float d = sqdist3(qx, qy, qz, c.x, c.y, c.z);
+            if (d < bd) { bd = d; best = t0 + i; }
+        }
+    }
+    __syncthreads();
+    int* const sk = reinterpret_cast<int*>(tile);
+    float* const sd = reinterpret_cast<float*>(tile) + kT;
+    sk[threadIdx.x] = best; sd[threadIdx.x] = bd;
+    __syncthreads();
+    if (part == 0 && u < nq) {
+        for (int p = 1; p < kNnParts; p++) {
+            const int ob = sk[p * kNnQ + u];
+            const float od = sd[p * kNnQ + u];
+            if (ob >= 0 && (best < 0 || od < bd || (od == bd && ob < best))) { bd = od; best = ob; }
+        }
+        out_k[q0 + u] = best;
+        if (out_d) out_d[q0 + u] = bd;
+    }
+    __syncthreads();
+}
+
+// phase_match_impl by the whole group: finalise centroids and boxes and transform the previous ones (spread over the
+// group), barrier, nearest current cluster of every previous one and nearest previous cluster of every current one
+// (chunks of queries dealt out over the CTAs), barrier, then one CTA keeps the reciprocal pairs in ascending query index
+// and applies the volume constraint in that order: the arrays and counts phase_match_impl writes. Every CTA must call;
+// the caller's barrier follows.
+__device__ __noinline__ void phase_match_large(const FramePtrs& a, int cta, int G, unsigned long long* dyn, GroupBarrier& bar) {
+    const int K = __ldcg(&a.counts[MOR_CNT_K]);
+    const int Kp = a.two_frames ? __ldcg(&a.p_counts[MOR_CNT_K]) : 0;
+    const int gtid = cta * kT + threadIdx.x, stride = G * kT;
+    for (int c = gtid; c < K; c += stride) {
+        const double n = (double)__ldcg(&a.cl_size[c]);
+#pragma unroll
+        for (int q = 0; q < 3; q++)
+            a.cl_centroid[c * 3 + q] = (float)join_fixed_mean((long long)__ldcg(&a.acc_sum[c * 6 + q * 2]), (long long)__ldcg(&a.acc_sum[c * 6 + q * 2 + 1]), n);
+#pragma unroll
+        for (int q = 0; q < 6; q++) a.cl_bbox[c * 6 + q] = fkey_inv(__ldcg(&a.acc_box[c * 6 + q]));
+    }
+    if (!a.two_frames) return;
+    for (int i = gtid; i < Kp; i += stride) {
+        const float3 t = xform(a.M, a.p_cl_centroid[i * 3], a.p_cl_centroid[i * 3 + 1], a.p_cl_centroid[i * 3 + 2]);
+        a.pct[i * 3] = t.x; a.pct[i * 3 + 1] = t.y; a.pct[i * 3 + 2] = t.z;
+#pragma unroll
+        for (int q = 0; q < 6; q++) a.pbbox[i * 6 + q] = fkey_inv(__ldcg(&a.pacc_box[i * 6 + q]));
+        a.match_of_prev[i] = -1; a.mid_of_prev[i] = -1;
+    }
+    for (int j = gtid; j < K; j += stride) a.mid_of_cur[j] = -1;
+    bar.sync();
+    float4* const tile = reinterpret_cast<float4*>(dyn);
+    const int chunks_prev = (Kp + kNnQ - 1) / kNnQ, chunks_cur = (K + kNnQ - 1) / kNnQ;
+    for (int c = cta; c < chunks_prev + chunks_cur; c += G) {
+        if (c < chunks_prev) nn_chunk(a.pct, c * kNnQ, min(kNnQ, Kp - c * kNnQ), a.cl_centroid, K, tile, a.nn_cur, a.nn_dist);
+        else { const int q0 = (c - chunks_prev) * kNnQ; nn_chunk(a.cl_centroid, q0, min(kNnQ, K - q0), a.pct, Kp, tile, a.nn_prev, nullptr); }
+    }
+    bar.sync();
+    if (cta != 0) return;
+    int n_recip = 0, n_match = 0;
+    for (int base = 0; base < Kp; base += kSingle) {
+        const int i = base + threadIdx.x;
+        bool ok = false, vok = false;
+        int j = -1;
+        float d = 0.f;
+        if (i < Kp) {
+            j = __ldcg(&a.nn_cur[i]); d = __ldcg(&a.nn_dist[i]);
+            ok = j >= 0 && __ldcg(&a.nn_prev[j]) == i;
+            if (ok) {
+                const float* bp = a.pbbox + i * 6; const float* bc = a.cl_bbox + j * 6;
+                const double volp = (double)__fmul_rn(__fmul_rn(__fsub_rn(__ldcg(bp + 3), __ldcg(bp)), __fsub_rn(__ldcg(bp + 4), __ldcg(bp + 1))), __fsub_rn(__ldcg(bp + 5), __ldcg(bp + 2)));
+                const double volc = (double)__fmul_rn(__fmul_rn(__fsub_rn(__ldcg(bc + 3), __ldcg(bc)), __fsub_rn(__ldcg(bc + 4), __ldcg(bc + 1))), __fsub_rn(__ldcg(bc + 5), __ldcg(bc + 2)));
+                vok = (fabs(volp - volc) / (volp + volc)) < (double)a.volume_constraint;  // NaN -> false
+            }
+        }
+        int tot;
+        const int r = single_block_rank(ok, &tot);
+        if (ok) { a.recip_q[n_recip + r] = i; a.recip_m[n_recip + r] = j; }
+        n_recip += tot;
+        const int rm = single_block_rank(vok, &tot);
+        if (vok) {
+            const int m = n_match + rm;
+            a.match_q[m] = i; a.match_m[m] = j; a.match_dist[m] = d;
+            a.match_of_prev[i] = j; a.mid_of_prev[i] = m; a.mid_of_cur[j] = m;
+            a.newcount[m] = 0; a.match_score[m] = 0.0;
+            atomicAdd(&a.counts[MOR_CNT_P1], a.p_cl_size[i]);
+            atomicAdd(&a.counts[MOR_CNT_P2], __ldcg(&a.cl_size[j]));
+        }
+        n_match += tot;
+    }
+    if (threadIdx.x == 0) {
+        a.counts[MOR_CNT_MU] = n_recip; a.counts[MOR_CNT_M] = n_match;
+        a.counts[MOR_CNT_NKPREV] = a.p_counts[MOR_CNT_NK];
+    }
+}
 // ===================================================================================== phase I: moving test
 // Method 2 (default): the score of a matched pair is the number of points of the current cluster whose octree leaf
 // holds no point of the transformed previous cluster (cpp:325-330).
+template <bool LK>
 __device__ __forceinline__ void phase_lattice_count(const FramePtrs& a, int cta, int G) {
     int lo, hi;
     cta_slice(frame_vars().nc, cta, G, &lo, &hi);
     const int lane = threadIdx.x & 31;
+    const bool wide = LK && a.p_counts[MOR_CNT_K] > kLatticeNarrowK;
     for (int base = lo; base < hi; base += kT) {
         const int s = base + threadIdx.x;
         int m = -1;
@@ -1403,7 +1638,7 @@ __device__ __forceinline__ void phase_lattice_count(const FramePtrs& a, int cta,
                 const float4 p = a.spts[s];
                 const int kp = a.match_q[m];
                 unsigned long long key;
-                if (lattice_key(a.anchorp + (size_t)kp * 3, kp, p.x, p.y, p.z, &key)) is_new = !hset_contains(a.lattice, a.lattice_mask, key);
+                if (lattice_key(a.anchorp + (size_t)kp * 3, kp, p.x, p.y, p.z, &key, wide)) is_new = !hset_contains(a.lattice, a.lattice_mask, key);
                 else { atomicOr(&a.counts[MOR_CNT_ERRFLAGS], ERR_LATTICE_RANGE); is_new = true; }
             }
         }
@@ -1605,7 +1840,7 @@ __device__ __forceinline__ void phase_chain_tail(const FramePtrs& a) {
 //  Output part: ExtractIndices(negative) of the moving points + append of the ground points (cpp:673-684), written as
 //  pcl::PointXYZI wire records (cpp:690); stable single-pass compaction over [cloud | ground].
 constexpr int kOutTile = kT;
-constexpr int kRemovedBits = 16384;  // = max kmax
+constexpr int kRemovedBits = kSmallK;  // a frame with more clusters takes the LARGE filter
 
 struct FilterShared {
     unsigned removed[kRemovedBits / 32];
@@ -1613,6 +1848,10 @@ struct FilterShared {
     int nn_k[kT]; float nn_d[kT];  // nearest cluster of one chunk of mo_vec entries
 };
 
+// LARGE (K > kRemovedBits): marker_cluster already holds every entry's nearest cluster and cluster_removed the removal
+// set (filter_markers_large, filter_mark_large); the distance is recomputed from the two centroids (the same sqdist3 as
+// the search: the same float).
+template <bool LARGE = false>
 __device__ __forceinline__ int filter_tracking(const FramePtrs& a, FilterShared& sh, bool writer) {
     const int mo_parity = a.mo_parity;
     const int K = a.counts[MOR_CNT_K];
@@ -1625,11 +1864,12 @@ __device__ __forceinline__ int filter_tracking(const FramePtrs& a, FilterShared&
     int* mo_f_out = a.mo_conf + (size_t)(mo_parity ^ 1) * a.momax;
     __syncthreads();
     if (threadIdx.x == 0) { sh.total = 0; sh.keep_base = 0; }
-    for (int t = threadIdx.x; t < (K + 31) / 32; t += kT) sh.removed[t] = 0u;
+    if (!LARGE)
+        for (int t = threadIdx.x; t < (K + 31) / 32; t += kT) sh.removed[t] = 0u;
     __syncthreads();
     // K == 0: un-built kd-tree in the reference (UB) -> entries untouched
     for (int base = 0; base < n_mo && K > 0; base += kT) {
-        {   // a warp per entry
+        if (!LARGE) {   // a warp per entry
             const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
             for (int u = warp; u < kT && base + u < n_mo; u += kWarps) {
                 const int e = base + u;
@@ -1645,10 +1885,17 @@ __device__ __forceinline__ int filter_tracking(const FramePtrs& a, FilterShared&
         if (t < n_mo) {
             cx = mo_c_in[t * 3]; cy = mo_c_in[t * 3 + 1]; cz = mo_c_in[t * 3 + 2];
             conf = mo_f_in[t];
-            const float d = sh.nn_d[threadIdx.x];
-            const int k = sh.nn_k[threadIdx.x];
-            if (writer) a.marker_cluster[t] = k;
-            atomicOr(&sh.removed[k >> 5], 1u << (k & 31));
+            float d;
+            int k;
+            if (LARGE) {
+                k = __ldcg(&a.marker_cluster[t]);
+                d = sqdist3(cx, cy, cz, __ldcg(&a.cl_centroid[k * 3]), __ldcg(&a.cl_centroid[k * 3 + 1]), __ldcg(&a.cl_centroid[k * 3 + 2]));
+            } else {
+                d = sh.nn_d[threadIdx.x];
+                k = sh.nn_k[threadIdx.x];
+                if (writer) a.marker_cluster[t] = k;
+                atomicOr(&sh.removed[k >> 5], 1u << (k & 31));
+            }
             atomicAdd(&sh.total, a.cl_size[k]);
             if (!a.cl_flags[k] || d > a.leave_off) {  // cpp:650
                 conf--;
@@ -1681,7 +1928,8 @@ __device__ __forceinline__ int filter_tracking(const FramePtrs& a, FilterShared&
                 mo_f_out[t] = mo_f_in[t];
             }
         }
-        for (int k = threadIdx.x; k < K; k += kT) a.cluster_removed[k] = (sh.removed[k >> 5] >> (k & 31)) & 1u;
+        if (!LARGE)
+            for (int k = threadIdx.x; k < K; k += kT) a.cluster_removed[k] = (sh.removed[k >> 5] >> (k & 31)) & 1u;
         if (threadIdx.x == 0) {
             const int kept = K > 0 ? sh.keep_base : n_mo;
             ts->n_mo[mo_parity ^ 1] = kept;  // the host flips the parity when filterCloud commits the frame
@@ -1694,6 +1942,24 @@ __device__ __forceinline__ int filter_tracking(const FramePtrs& a, FilterShared&
     return overflow;
 }
 
+// The LARGE filter's group-wide steps, each followed by a group barrier (k_filter_again: a launch each). 1: the nearest
+// current cluster of every mo_vec entry (chunks of entries dealt out over the CTAs) and an empty removal set.
+__device__ __forceinline__ void filter_markers_large(const FramePtrs& a, int cta, int G, float4* tile) {
+    const int K = __ldcg(&a.counts[MOR_CNT_K]);
+    const int n_mo = __ldcg(&a.track->n_mo[a.mo_parity]);
+    const float* mo_c_in = a.mo_centroid + (size_t)a.mo_parity * a.momax * 3;
+    for (int k = cta * kT + threadIdx.x; k < K; k += G * kT) a.cluster_removed[k] = 0;
+    for (int c = cta; c * kNnQ < n_mo; c += G) nn_chunk(mo_c_in, c * kNnQ, min(kNnQ, n_mo - c * kNnQ), a.cl_centroid, K, tile, a.marker_cluster, nullptr);
+}
+// 2: the clusters selected by the entries are removed (cpp:644-648).
+__device__ __forceinline__ void filter_mark_large(const FramePtrs& a, int cta, int G) {
+    const int n_mo = __ldcg(&a.track->n_mo[a.mo_parity]);
+    for (int e = cta * kT + threadIdx.x; e < n_mo; e += G * kT) {
+        const int k = __ldcg(&a.marker_cluster[e]);
+        if (k >= 0) a.cluster_removed[k] = 1;  // (-1: no centroid compared below FLT_MAX)
+    }
+}
+
 struct FilterTileIn { float4 p; int c; };  // a thread's item of a tile: the point and, for a cloud point, its cluster
 __device__ __forceinline__ FilterTileIn filter_tile_load(const FramePtrs& a, int tile) {
     const int nc = frame_vars().nc, ng = frame_vars().ng;
@@ -1704,6 +1970,10 @@ __device__ __forceinline__ FilterTileIn filter_tile_load(const FramePtrs& a, int
     else if (t < nc + ng) in.p = a.gpts[t - nc];
     return in;
 }
+__device__ __forceinline__ bool cluster_is_removed(const FramePtrs& a, const FilterShared& sh, int c, bool large) {
+    return large ? __ldcg(&a.cluster_removed[c]) != 0 : ((sh.removed[c >> 5] >> (c & 31)) & 1u) != 0;
+}
+template <bool LARGE = false>
 __device__ __forceinline__ void filter_tile(const FramePtrs& a, const FilterShared& sh, int overflow, int tile, int last_tile, const FilterTileIn& in) {
     const int nc = frame_vars().nc, ng = frame_vars().ng;
     const int t = tile * kOutTile + threadIdx.x;
@@ -1711,7 +1981,7 @@ __device__ __forceinline__ void filter_tile(const FramePtrs& a, const FilterShar
     const float4 p = in.p;
     if (t < nc) {
         const int c = in.c;
-        const bool removed = overflow || (c >= 0 && ((sh.removed[c >> 5] >> (c & 31)) & 1u));
+        const bool removed = overflow || (c >= 0 && cluster_is_removed(a, sh, c, LARGE));
         keep = !removed;
         if (removed) a.removed_mask[a.cloud_src[t]] = 2;
     } else if (t < nc + ng) {
@@ -1732,6 +2002,7 @@ __device__ __forceinline__ void filter_tile(const FramePtrs& a, const FilterShar
 // tiles per CTA (the back half of a pipelined launch on 23 CTAs, a sequence of a batch on 4) - a quarter of the rounds, each
 // a chain of scan, prefix round trip and stores.
 constexpr int kOutWide = 4;
+template <bool LARGE = false>
 __device__ __forceinline__ void filter_tile_wide(const FramePtrs& a, const FilterShared& sh, int overflow, int tile, int last_tile) {
     const int nc = frame_vars().nc, ng = frame_vars().ng;
     const int t0 = (tile * kOutTile + (int)threadIdx.x) * kOutWide;
@@ -1746,7 +2017,7 @@ __device__ __forceinline__ void filter_tile_wide(const FramePtrs& a, const Filte
         if (t < nc) {
             p[q] = a.pts[t];
             const int c = a.cid[t];
-            const bool removed = overflow || (c >= 0 && ((sh.removed[c >> 5] >> (c & 31)) & 1u));
+            const bool removed = overflow || (c >= 0 && cluster_is_removed(a, sh, c, LARGE));
             keep[q] = !removed;
             if (removed) a.removed_mask[a.cloud_src[t]] = 2;
         } else if (t < nc + ng) {
@@ -1769,27 +2040,46 @@ __device__ __forceinline__ void filter_tile_wide(const FramePtrs& a, const Filte
     if (tile == last_tile && threadIdx.x == 0) a.counts[CNT_SPEC_NOUT] = before + tot;
 }
 
-__device__ __forceinline__ void phase_filter(const FramePtrs& a, int cta, int G, FilterShared& sh, bool cleanup = true) {
+template <bool LARGE>
+__device__ __forceinline__ void phase_filter_tiles(const FramePtrs& a, int cta, int G, FilterShared& sh) {
     const int total_items = frame_vars().nc + frame_vars().ng;
-    if (cleanup) frame_cleanup(a, cta, G);
     if ((long long)total_items > 2ll * G * kOutTile) {  // several rounds per CTA: four items per thread
         const int last_wide = (total_items - 1) / (kOutTile * kOutWide);
         if (cta > last_wide) return;
-        const int overflow = filter_tracking(a, sh, cta == 0);
-        for (int tile = cta; tile <= last_wide; tile += G) filter_tile_wide(a, sh, overflow, tile, last_wide);
+        const int overflow = filter_tracking<LARGE>(a, sh, cta == 0);
+        for (int tile = cta; tile <= last_wide; tile += G) filter_tile_wide<LARGE>(a, sh, overflow, tile, last_wide);
         return;
     }
     const int last_tile = total_items ? (total_items - 1) / kOutTile : 0;
     if (cta > last_tile) return;  // nothing to compact here (CTA 0 always has tile 0: it owns the mo_vec update)
     FilterTileIn in = filter_tile_load(a, cta);  // the first tile's loads are in flight while the tracking part runs
-    const int overflow = filter_tracking(a, sh, cta == 0);
+    const int overflow = filter_tracking<LARGE>(a, sh, cta == 0);
     for (int tile = cta; tile <= last_tile; tile += G) {
         if (tile != cta) in = filter_tile_load(a, tile);
-        filter_tile(a, sh, overflow, tile, last_tile, in);
+        filter_tile<LARGE>(a, sh, overflow, tile, last_tile, in);
+    }
+}
+// (out of line: the frame kernels run at their register limit, and the rare large-K steps should not add to it)
+__device__ __noinline__ void phase_filter_large(const FramePtrs& a, int cta, int G, FilterShared& sh, unsigned long long* dyn, GroupBarrier& bar) {
+    filter_markers_large(a, cta, G, reinterpret_cast<float4*>(dyn));
+    bar.sync();
+    filter_mark_large(a, cta, G);
+    bar.sync();
+    phase_filter_tiles<true>(a, cta, G, sh);
+}
+// Every CTA must call (the LARGE filter has group barriers in front of the tiles); K is final since the match.
+template <bool LK>
+__device__ __forceinline__ void phase_filter(const FramePtrs& a, int cta, int G, FilterShared& sh, unsigned long long* dyn, GroupBarrier& bar, bool cleanup = true) {
+    if (cleanup) frame_cleanup(a, cta, G);
+    if (LK && __ldcg(&a.counts[MOR_CNT_K]) > kRemovedBits) {
+        phase_filter_large(a, cta, G, sh, dyn, bar);
+    } else {
+        phase_filter_tiles<false>(a, cta, G, sh);
     }
 }
 
 // Last CTA out: every counter of the frame back to zero.
+template <bool LK>
 __device__ __forceinline__ void frame_epilogue(const FramePtrs& a, int G) {
     __shared__ int s_last;
     __syncthreads();
@@ -1804,6 +2094,7 @@ __device__ __forceinline__ void frame_epilogue(const FramePtrs& a, int G) {
     if (threadIdx.x == 0) {
         Scratch* sc = a.scratch;
         sc->bar = 0u; sc->blocks_done = 0; sc->n_cells = 0; sc->n_roots = 0; sc->n_light = 0; sc->n_heavy = 0; sc->n_sorted = 0; sc->tail_match = 0u; sc->tail_chain = 0u; sc->ticket_light = 0; sc->ticket_heavy = 0; sc->err_early = 0;
+        if (LK) sc->n_sel = 0;
         sc->ticket_ingest = 0; sc->ticket_cells = 0;  // voxel ground modes (k_ground_partition leaves its tile tickets behind)
         for (int q = 0; q < 3; q++) { sc->box_inv_min[q] = 0u; sc->box_max[q] = 0u; }
     }
@@ -1817,8 +2108,8 @@ struct FrameShared {
     FilterShared filter;
 };
 
-template <int PH>
-__device__ __forceinline__ void run_phase(const FramePtrs& a, int cta, int G, FrameShared& sh, unsigned long long* dyn, unsigned& parity) {
+template <int PH, bool LK>
+__device__ __forceinline__ void run_phase(const FramePtrs& a, int cta, int G, FrameShared& sh, unsigned long long* dyn, unsigned& parity, GroupBarrier& bar) {
     if (PH == PH_INGEST) { if (a.skip_ingest) phase_bin_cloud(a, cta, G); else phase_ingest(a, cta, G, dyn, &sh.mbar, parity); }
     if (PH == PH_CELLS) phase_cells(a, cta, G);
     if (PH == PH_LINK) phase_link(a, cta, G, dyn);
@@ -1826,19 +2117,31 @@ __device__ __forceinline__ void run_phase(const FramePtrs& a, int cta, int G, Fr
     if (PH == PH_JUMP) phase_jump(a, cta, G);
     if (PH == PH_CROSS) phase_cross(a, cta, G);
     if (PH == PH_ROOTS) phase_roots(a, cta, G);
-    if (PH == PH_SELECT) { if (cta == 0) phase_select(a, dyn); phase_transform(a, cta, G); }
-    if (PH == PH_STATS) { phase_stats(a, cta, G); if (group_last_arrival(&a.scratch->tail_match, (unsigned)G)) phase_match(a, dyn); }
+    if (PH == PH_SELECT) {
+        if (select_large<LK>(a)) {
+            phase_select_large(a, cta, G, dyn, bar);
+            if (a.two_frames) { int lo, hi; cta_slice(a.p_counts[MOR_CNT_NC], cta, G, &lo, &hi); transform_range<LK>(a, lo, hi); }
+        } else {
+            if (cta == 0) phase_select(a, dyn);
+            phase_transform<LK>(a, cta, G);
+        }
+    }
+    if (PH == PH_STATS) {
+        phase_stats(a, cta, G);
+        if (match_large<LK>(a)) { bar.sync(); phase_match_large(a, cta, G, dyn, bar); }
+        else if (group_last_arrival(&a.scratch->tail_match, (unsigned)G)) phase_match(a, dyn);
+    }
     if (PH == PH_MOVING) {
-        if (a.two_frames) { if (a.method == 2) phase_lattice_count(a, cta, G); else phase_pde_count(a, cta, G); }
+        if (a.two_frames) { if (a.method == 2) phase_lattice_count<LK>(a, cta, G); else phase_pde_count(a, cta, G); }
         if (group_last_arrival(&a.scratch->tail_chain, (unsigned)G)) phase_chain_tail(a);
     }
-    if (PH == PH_FILTER) phase_filter(a, cta, G, sh.filter);
+    if (PH == PH_FILTER) phase_filter<LK>(a, cta, G, sh.filter, dyn, bar);
 }
 
 
-template <int PH>
+template <int PH, bool LK>
 __device__ __forceinline__ void frame_step(const FramePtrs& a, int cta, int G, FrameShared& sh, unsigned long long* dyn, unsigned& parity, GroupBarrier& bar) {
-    run_phase<PH>(a, cta, G, sh, dyn, parity);
+    run_phase<PH, LK>(a, cta, G, sh, dyn, parity, bar);
 #ifdef MOR_CTA_TRACE
     __syncthreads();
     if (threadIdx.x == 0 && cta < 256) a.cta_trace[PH * 256 + cta] = global_ns();
@@ -1847,22 +2150,23 @@ __device__ __forceinline__ void frame_step(const FramePtrs& a, int cta, int G, F
     if (cta == 0 && threadIdx.x == 0) a.phase_ts[PH + 1] = global_ns();  // a dozen stores per frame: the frame's own timeline
 }
 
+template <bool LK>
 __device__ __forceinline__ void frame_body(const FramePtrs& a, int cta, int G, FrameShared& sh, unsigned long long* dyn, unsigned& parity) {
     GroupBarrier bar{&a.scratch->bar, 0u, (unsigned)G};
     if (cta == 0 && threadIdx.x == 0) a.phase_ts[0] = global_ns();
-    frame_step<PH_INGEST>(a, cta, G, sh, dyn, parity, bar);
+    frame_step<PH_INGEST, LK>(a, cta, G, sh, dyn, parity, bar);
     load_frame_vars(a);
-    frame_step<PH_CELLS>(a, cta, G, sh, dyn, parity, bar);
-    frame_step<PH_LINK>(a, cta, G, sh, dyn, parity, bar);
-    frame_step<PH_TEST>(a, cta, G, sh, dyn, parity, bar);
-    frame_step<PH_JUMP>(a, cta, G, sh, dyn, parity, bar);
-    frame_step<PH_CROSS>(a, cta, G, sh, dyn, parity, bar);
-    frame_step<PH_ROOTS>(a, cta, G, sh, dyn, parity, bar);
-    frame_step<PH_SELECT>(a, cta, G, sh, dyn, parity, bar);
-    frame_step<PH_STATS>(a, cta, G, sh, dyn, parity, bar);
-    frame_step<PH_MOVING>(a, cta, G, sh, dyn, parity, bar);
-    frame_step<PH_FILTER>(a, cta, G, sh, dyn, parity, bar);
-    frame_epilogue(a, G);
+    frame_step<PH_CELLS, LK>(a, cta, G, sh, dyn, parity, bar);
+    frame_step<PH_LINK, LK>(a, cta, G, sh, dyn, parity, bar);
+    frame_step<PH_TEST, LK>(a, cta, G, sh, dyn, parity, bar);
+    frame_step<PH_JUMP, LK>(a, cta, G, sh, dyn, parity, bar);
+    frame_step<PH_CROSS, LK>(a, cta, G, sh, dyn, parity, bar);
+    frame_step<PH_ROOTS, LK>(a, cta, G, sh, dyn, parity, bar);
+    frame_step<PH_SELECT, LK>(a, cta, G, sh, dyn, parity, bar);
+    frame_step<PH_STATS, LK>(a, cta, G, sh, dyn, parity, bar);
+    frame_step<PH_MOVING, LK>(a, cta, G, sh, dyn, parity, bar);
+    frame_step<PH_FILTER, LK>(a, cta, G, sh, dyn, parity, bar);
+    frame_epilogue<LK>(a, G);
 }
 
 // ===================================================================================== pipelined launch
@@ -1896,7 +2200,7 @@ __device__ __forceinline__ void frame_body(const FramePtrs& a, int cta, int G, F
 //    handle keeps the grid (table, cell_list) per frame parity; the front half leaves it standing and hands its cell
 //    count over in counts[CNT_PIPE_CELLS]; the back half empties it after the search.
 //  - k_frame_pipe_ground_pde: both.
-template <bool GROUND = false, bool PDE = false>
+template <bool GROUND, bool PDE, bool LK>
 __device__ __forceinline__ void front_body(const FramePtrs& a, int cta, int G, FrameShared& sh, unsigned long long* dyn, unsigned& parity) {
     GroupBarrier bar{&a.scratch->bar, 0u, (unsigned)G};
     if (GROUND) phase_bin_cloud(a, cta, G, /*housekeep=*/false);
@@ -1909,8 +2213,10 @@ __device__ __forceinline__ void front_body(const FramePtrs& a, int cta, int G, F
     phase_jump(a, cta, G); bar.sync();
     phase_cross(a, cta, G); bar.sync();
     phase_roots(a, cta, G);
-    if (group_last_arrival(&a.scratch->tail_centroids, (unsigned)G)) phase_select(a, dyn);  // (the last CTA in selects the clusters: no barrier in front of it)
+    // (the last CTA in selects the clusters: no barrier in front of it; a large-K frame is selected by the whole group)
+    if (group_last_arrival(&a.scratch->tail_centroids, (unsigned)G) && !select_large<LK>(a)) phase_select(a, dyn);
     bar.sync();
+    if (select_large<LK>(a)) { phase_select_large(a, cta, G, dyn, bar); bar.sync(); }
     phase_stats(a, cta, G);  // (the sums it accumulates are double-buffered by frame parity: the back half turns them into centroids)
     if (PDE) {  // the grid stays for the back half's search: only the scan states go back to zero here
         for (int t = cta * kT + threadIdx.x; t < a.tiles_pts; t += G * kT) a.st_ingest[t] = 0ull;
@@ -1931,13 +2237,14 @@ __device__ __forceinline__ void front_body(const FramePtrs& a, int cta, int G, F
         Scratch* sc = a.scratch;
         sc->bar = 0u; sc->blocks_done = 0; sc->n_cells = 0; sc->n_roots = 0; sc->n_light = 0; sc->n_heavy = 0; sc->n_sorted = 0; sc->tail_centroids = 0u;
         sc->ticket_light = 0; sc->ticket_heavy = 0; sc->err_early = 0;
+        if (LK) sc->n_sel = 0;
         if (GROUND) sc->ticket_ingest = 0;  // (drawn by k_ground_partition; frame_epilogue resets it in one kernel per frame)
     }
 }
 
 // (GROUND does not change the back half; it keeps every kernel's instantiations of the two bodies its own, so that their
 // static shared variables stay local to one kernel and k_frame_pipe's shared layout is what it was before the variants)
-template <bool GROUND = false, bool PDE = false>
+template <bool GROUND, bool PDE, bool LK>
 __device__ __forceinline__ void back_body(const FramePtrs& a, int cta, int G, FrameShared& sh, unsigned long long* dyn) {
     GroupBarrier bar{&a.scratch->bar_back, 0u, (unsigned)G};
     if (threadIdx.x == 0) {  // (the cell count belongs to the front half, which is busy with the next frame)
@@ -1950,11 +2257,12 @@ __device__ __forceinline__ void back_body(const FramePtrs& a, int cta, int G, Fr
     if (a.two_frames) {
         int lo, hi;
         cta_slice(a.p_counts[MOR_CNT_NC], cta, G, &lo, &hi);
-        transform_range(a, lo, hi);
+        transform_range<LK>(a, lo, hi);
     }
-    if (group_last_arrival(&a.scratch->tail_match_back, (unsigned)G)) phase_match(a, dyn);
+    if (match_large<LK>(a)) { bar.sync(); phase_match_large(a, cta, G, dyn, bar); }
+    else if (group_last_arrival(&a.scratch->tail_match_back, (unsigned)G)) phase_match(a, dyn);
     bar.sync();
-    if (a.two_frames) { if (PDE) phase_pde_count(a, cta, G); else phase_lattice_count(a, cta, G); }
+    if (a.two_frames) { if (PDE) phase_pde_count(a, cta, G); else phase_lattice_count<LK>(a, cta, G); }
     if (group_last_arrival(&a.scratch->tail_chain, (unsigned)G)) phase_chain_tail(a);
     bar.sync();
     if (PDE) {  // the search is over: this frame's clustering grid goes back to "all zero" (frame_cleanup's first loop)
@@ -1962,7 +2270,7 @@ __device__ __forceinline__ void back_body(const FramePtrs& a, int cta, int G, Fr
         for (int i = cta * kT + threadIdx.x; i < n_cells; i += G * kT)
             *reinterpret_cast<uint4*>(a.table + a.cell_list[i]) = make_uint4(0u, 0u, 0u, 0u);
     }
-    phase_filter(a, cta, G, sh.filter, /*cleanup=*/false);
+    phase_filter<LK>(a, cta, G, sh.filter, dyn, bar, /*cleanup=*/false);
     __shared__ int s_last_back;
     __syncthreads();
     if (threadIdx.x == 0) {
@@ -1979,50 +2287,60 @@ __device__ __forceinline__ void back_body(const FramePtrs& a, int cta, int G, Fr
     }
 }
 
+// Every frame kernel below is a template on LK ("large-K"): the instantiation with LK = true serves handles whose
+// max_clusters exceeds kSmallK and carries the group-wide steps for frames with more clusters; LK = false is the code of
+// every other handle, with no trace of them (mor_b200.cu picks the instantiation per handle).
+//
 // Front half of `f` on the CTAs [0, Gf), back half of `b` on the rest; Gf = gridDim.x: front only, Gf = 0: back only.
+template <bool LK>
 __global__ void __launch_bounds__(kT, 1) k_frame_pipe(const __grid_constant__ FramePtrs f, const __grid_constant__ FramePtrs b, int Gf) {
     extern __shared__ __align__(128) unsigned long long dyn[];
     __shared__ FrameShared sh;
     if (threadIdx.x == 0) mbar_init(&sh.mbar, 1);
     __syncthreads();
     unsigned parity = 0;
-    if ((int)blockIdx.x < Gf) front_body(f, blockIdx.x, Gf, sh, dyn, parity);
-    else back_body(b, (int)blockIdx.x - Gf, (int)gridDim.x - Gf, sh, dyn);
+    if ((int)blockIdx.x < Gf) front_body<false, false, LK>(f, blockIdx.x, Gf, sh, dyn, parity);
+    else back_body<false, false, LK>(b, (int)blockIdx.x - Gf, (int)gridDim.x - Gf, sh, dyn);
 }
 
 // The other configurations: the same launch with the variants of the two bodies described above.
-template <bool GROUND, bool PDE>
+template <bool GROUND, bool PDE, bool LK>
 __device__ __forceinline__ void frame_pipe_variant(const FramePtrs& f, const FramePtrs& b, int Gf) {
     extern __shared__ __align__(128) unsigned long long dyn[];
     __shared__ FrameShared sh;
     if (threadIdx.x == 0) mbar_init(&sh.mbar, 1);
     __syncthreads();
     unsigned parity = 0;
-    if ((int)blockIdx.x < Gf) front_body<GROUND, PDE>(f, blockIdx.x, Gf, sh, dyn, parity);
-    else back_body<GROUND, PDE>(b, (int)blockIdx.x - Gf, (int)gridDim.x - Gf, sh, dyn);
+    if ((int)blockIdx.x < Gf) front_body<GROUND, PDE, LK>(f, blockIdx.x, Gf, sh, dyn, parity);
+    else back_body<GROUND, PDE, LK>(b, (int)blockIdx.x - Gf, (int)gridDim.x - Gf, sh, dyn);
 }
+template <bool LK>
 __global__ void __launch_bounds__(kT, 1) k_frame_pipe_ground(const __grid_constant__ FramePtrs f, const __grid_constant__ FramePtrs b, int Gf) {
-    frame_pipe_variant<true, false>(f, b, Gf);
+    frame_pipe_variant<true, false, LK>(f, b, Gf);
 }
+template <bool LK>
 __global__ void __launch_bounds__(kT, 1) k_frame_pipe_pde(const __grid_constant__ FramePtrs f, const __grid_constant__ FramePtrs b, int Gf) {
-    frame_pipe_variant<false, true>(f, b, Gf);
+    frame_pipe_variant<false, true, LK>(f, b, Gf);
 }
+template <bool LK>
 __global__ void __launch_bounds__(kT, 1) k_frame_pipe_ground_pde(const __grid_constant__ FramePtrs f, const __grid_constant__ FramePtrs b, int Gf) {
-    frame_pipe_variant<true, true>(f, b, Gf);
+    frame_pipe_variant<true, true, LK>(f, b, Gf);
 }
 
 // One sequence, the whole grid is its group; the frame's arguments travel in the constant bank.
+template <bool LK>
 __global__ void __launch_bounds__(kT, 1) k_frame(const __grid_constant__ FramePtrs a) {
     extern __shared__ __align__(128) unsigned long long dyn[];
     __shared__ FrameShared sh;
     if (threadIdx.x == 0) mbar_init(&sh.mbar, 1);
     __syncthreads();
     unsigned parity = 0;
-    frame_body(a, blockIdx.x, gridDim.x, sh, dyn, parity);
+    frame_body<LK>(a, blockIdx.x, gridDim.x, sh, dyn, parity);
 }
 
 // S sequences per launch: grid = groups x G CTAs; group g steps sequences g, g + groups, ... (each through all
 // phases, independently of the other groups), G CTAs per sequence.
+template <bool LK>
 __global__ void __launch_bounds__(kT, 1) k_frame_batch(const FramePtrs* __restrict__ P, int S, int G) {
     extern __shared__ __align__(128) unsigned long long dyn[];
     __shared__ FrameShared sh;
@@ -2030,24 +2348,42 @@ __global__ void __launch_bounds__(kT, 1) k_frame_batch(const FramePtrs* __restri
     if (threadIdx.x == 0) mbar_init(&sh.mbar, 1);
     __syncthreads();
     unsigned parity = 0;
-    for (int seq = group; seq < S; seq += groups) frame_body(P[seq], cta, G, sh, dyn, parity);
+    for (int seq = group; seq < S; seq += groups) frame_body<LK>(P[seq], cta, G, sh, dyn, parity);
 }
 
 // One phase per launch (per-phase timing; the kernel boundary is the barrier). Same grid, same striding.
-template <int PH>
+template <int PH, bool LK>
 __global__ void __launch_bounds__(kT, 1) k_phase(const __grid_constant__ FramePtrs a) {
     extern __shared__ __align__(128) unsigned long long dyn[];
     __shared__ FrameShared sh;
     if (threadIdx.x == 0) mbar_init(&sh.mbar, 1);
     __syncthreads();
     unsigned parity = 0;
+    GroupBarrier bar{&a.scratch->bar, 0u, gridDim.x};  // (the large-K steps of select, match and filter)
     if (PH != PH_INGEST) load_frame_vars(a);
-    run_phase<PH>(a, blockIdx.x, gridDim.x, sh, dyn, parity);
-    if (PH == PH_FILTER) frame_epilogue(a, gridDim.x);
+    run_phase<PH, LK>(a, blockIdx.x, gridDim.x, sh, dyn, parity, bar);
+    if (PH == PH_FILTER) frame_epilogue<LK>(a, gridDim.x);
+    if (LK && (PH == PH_SELECT || PH == PH_STATS)) {  // last CTA out: the barrier back to zero for the next launch
+        __shared__ int s_last;
+        __syncthreads();
+        if (threadIdx.x == 0) s_last = atomicAdd(&a.scratch->blocks_done, 1) == (int)gridDim.x - 1;
+        __syncthreads();
+        if (s_last && threadIdx.x == 0) { a.scratch->bar = 0u; a.scratch->blocks_done = 0; }
+    }
 }
 
 // filterCloud called again on a frame that was already filtered (the reference then runs the tracking update once
-// more on the updated mo_vec): the filter phase alone. Tiles by ticket, so a plain launch suffices.
+// more on the updated mo_vec): the filter phase alone. Tiles by ticket, so a plain launch suffices. A frame with more
+// than kRemovedBits clusters has its markers and removal set made first by k_filter_markers and k_filter_mark (launched
+// in front of it by handles whose kmax allows such frames; they do nothing for a smaller frame).
+__global__ void __launch_bounds__(kT, 1) k_filter_markers(const __grid_constant__ FramePtrs a) {
+    extern __shared__ __align__(128) unsigned long long dyn[];
+    if (__ldcg(&a.counts[MOR_CNT_K]) > kRemovedBits) filter_markers_large(a, blockIdx.x, gridDim.x, reinterpret_cast<float4*>(dyn));
+}
+__global__ void __launch_bounds__(kT, 1) k_filter_mark(const __grid_constant__ FramePtrs a) {
+    if (__ldcg(&a.counts[MOR_CNT_K]) > kRemovedBits) filter_mark_large(a, blockIdx.x, gridDim.x);
+}
+template <bool LK>
 __global__ void __launch_bounds__(kT, 1) k_filter_again(const __grid_constant__ FramePtrs a) {
     __shared__ FilterShared sh;
     __shared__ int s_tile, s_last;
@@ -2058,8 +2394,13 @@ __global__ void __launch_bounds__(kT, 1) k_filter_again(const __grid_constant__ 
     const int last_tile = total_items ? (total_items - 1) / kOutTile : 0;
     if (tile <= last_tile) {
         const FilterTileIn in = filter_tile_load(a, tile);
-        const int overflow = filter_tracking(a, sh, tile == 0);
-        filter_tile(a, sh, overflow, tile, last_tile, in);
+        if (LK && __ldcg(&a.counts[MOR_CNT_K]) > kRemovedBits) {
+            const int overflow = filter_tracking<true>(a, sh, tile == 0);
+            filter_tile<true>(a, sh, overflow, tile, last_tile, in);
+        } else {
+            const int overflow = filter_tracking(a, sh, tile == 0);
+            filter_tile(a, sh, overflow, tile, last_tile, in);
+        }
     }
     __syncthreads();
     if (threadIdx.x == 0) s_last = atomicAdd(&a.scratch->out_blocks_done, 1) == (int)gridDim.x - 1;

@@ -58,7 +58,10 @@ enum { MOR_GROUND_CROP = 0, MOR_GROUND_VOXEL_COV = 1, MOR_GROUND_VOXEL_EIGEN = 2
 /* Optional capacities; zero fields take defaults. */
 typedef struct mor_limits {
     uint32_t max_points;    /* largest frame accepted (default 300000) */
-    uint32_t max_clusters;  /* largest number of size-valid clusters per frame (default 8192, at most 16384) */
+    uint32_t max_clusters;  /* largest number of size-valid clusters per frame (default 8192). Values up to 16384 are
+                               taken as given; larger ones up to max_points (a larger value is clamped to it). A frame
+                               with more than 16384 clusters runs group-wide select, match and filter steps; a frame
+                               with more size-valid clusters than max_clusters is MOR_ERR_CAPACITY (ERR_CLUSTER_CAP) */
     uint32_t max_moving;    /* capacity of the confirmed-moving list mo_vec (default 1024) */
     uint32_t max_cells;     /* voxel ground modes only (ground_mode 1/2): largest dense voxel / ball-query table over the
                                bounding box of a frame's raw cloud (default 2^24 cells; a frame that needs more is
