@@ -4,5 +4,5 @@ The product is `libmor_b200.so` (CUDA kernels + C ABI, include/mor_b200.h) and t
 `MovingObjectRemoval` (include/MOR/MovingObjectRemoval.h). This Python package is only the ctypes
 binding used by the tests and bench.py, plus the build recipe.
 """
-from .binding import (MorBinding, MorConfig, MorError, MorLimits, MovingObjectRemoval, SequenceBatch, Synth, load_product,  # noqa: F401
+from .binding import (MixedBatch, MorBinding, MorConfig, MorError, MorLimits, MovingObjectRemoval, SequenceBatch, Synth, load_product,  # noqa: F401
                       parse_config, PRODUCT_LIB, SYNTH_LIB, REPO_ROOT, TAPS, COUNT_NAMES)

@@ -80,6 +80,11 @@ class MorLimits(C.Structure):
                 ("reserved", C.c_uint32 * 4)]
 
 
+class MorBatchFrame(C.Structure):
+    _fields_ = [("d_data", C.c_void_p), ("n", C.c_uint32), ("point_step", C.c_uint32), ("off_x", C.c_uint32), ("off_y", C.c_uint32),
+                ("off_z", C.c_uint32), ("off_i", C.c_uint32), ("pose7", C.c_double * 7), ("d_out", C.c_void_p)]
+
+
 MARKER_DTYPE = np.dtype([("position", np.float32, 3), ("scale", np.float32, 3), ("color", np.float32, 4), ("id", np.int32), ("cluster", np.int32)])
 
 
@@ -125,6 +130,7 @@ class MorBinding:
         self.last_error = f("last_error", [vp], True, C.c_char_p)
         self.batch_step_device = f("batch_step_device", [C.POINTER(vp), u32, C.POINTER(vp), C.POINTER(u32), u32, u32, u32, u32, u32,
                                                          C.POINTER(C.c_double), C.POINTER(vp)], True)
+        self.batch_step_device_mixed = f("batch_step_device_mixed", [C.POINTER(vp), u32, C.POINTER(MorBatchFrame)], True)
         self.event_record = f("event_record", [vp, C.c_int], True)
         self.event_elapsed_ms = f("event_elapsed_ms", [vp, C.c_int, C.c_int, C.POINTER(C.c_float)], True)
         self.set_kernel_profiling = f("set_kernel_profiling", [vp, C.c_int], True)
@@ -439,6 +445,33 @@ class SequenceBatch:
         st = self.b.batch_step_device(self._hs, S, self._data, self._n, point_step, *offsets, self._poses, self._out)
         if st:
             self.handles[0]._check(st, "batch_step_device")
+
+
+class MixedBatch:
+    """One step of S sequences that may differ in frame count, configuration, limits, record layout and output records
+    (mor_batch_step_device_mixed). The handles may change from one step to the next."""
+
+    def __init__(self, binding: MorBinding | None = None):
+        self.b = binding or load_product()
+
+    def step(self, handles: list[MovingObjectRemoval], d_ptrs, ns, poses, d_outs, point_steps=None, offsets=None):
+        """Per sequence s: device records d_ptrs[s] (ns[s] of point_steps[s] bytes, default 16, field offsets offsets[s],
+        default (0, 4, 8, 12)), pose poses[s]; d_outs[s] must hold ns[s] output records of the handle's output mode."""
+        S = len(handles)
+        hs = (C.c_void_p * S)(*[h.h.value for h in handles])
+        frames = (MorBatchFrame * S)()
+        for s in range(S):
+            fr = frames[s]
+            fr.d_data, fr.n, fr.d_out = d_ptrs[s], int(ns[s]), d_outs[s]
+            fr.point_step = int(point_steps[s]) if point_steps is not None else 16
+            fr.off_x, fr.off_y, fr.off_z, fr.off_i = offsets[s] if offsets is not None else (0, 4, 8, 12)
+            for k in range(7):
+                fr.pose7[k] = float(poses[s][k])
+        st = self.b.batch_step_device_mixed(hs, S, frames)
+        if st:
+            handles[0]._check(st, "batch_step_device_mixed")
+        for s in range(S):
+            handles[s].n_input = int(ns[s])
 
 
 class Synth:

@@ -15,6 +15,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <algorithm>
 #include <string>
 #include <vector>
 
@@ -24,6 +25,15 @@
 #include "mor_records.cuh"
 
 using namespace mor;
+
+namespace mor {  // mor_batch_mixed.cu: the kernels of mor_batch_step_device_mixed
+// k_frame_batch_mixed: sets its shared-memory limit to `smem`; launches it cooperatively on `grid` CTAs, the LK
+// instantiation if `lk`, over the FramePtrs array P and the group table T.
+cudaError_t configure_frame_batch_mixed(size_t smem);
+cudaError_t launch_frame_batch_mixed(bool lk, unsigned grid, size_t smem, cudaStream_t st, const void* P, const void* T, int groups);
+// k_gather_records_mixed over `seqs` sequences (RecordPtrs R[seqs], their block counts nb[seqs]), blocks_x blocks each.
+cudaError_t launch_gather_records_mixed(unsigned blocks_x, unsigned seqs, cudaStream_t st, const void* R, const void* nb);
+}  // namespace mor
 
 #define MOR_CUDA(call)                                                                              \
     do {                                                                                            \
@@ -97,9 +107,9 @@ struct mor_handle {
     cudaStream_t stream = nullptr;
     uint32_t spec_out = 0;        // speculative size of the output D2H copy (points), from the previous frame
     cudaStream_t last_stream = nullptr;  // stream that carries this handle's latest work (differs after a batched step)
-    // batched stepping (this handle as the leader of a batch): device array of per-sequence arguments + pinned ring; a slot
-    // holds S FramePtrs followed by S GroundPtrs (the latter used by the voxel ground modes only)
-    uint8_t* d_batch = nullptr; uint8_t* h_batch = nullptr; uint32_t batch_cap = 0; int batch_slot = 0;
+    // batched stepping (this handle as the leader of a batch): device array of per-sequence arguments + pinned ring of four
+    // slots of batch_bytes each (batch_ring_slot); what a slot holds is up to the step that fills it
+    uint8_t* d_batch = nullptr; uint8_t* h_batch = nullptr; size_t batch_bytes = 0; int batch_slot = 0;
     cudaEvent_t batch_ev[4] = {nullptr, nullptr, nullptr, nullptr};
     uint32_t nmax = 0, kmax = 0, momax = 0;
     int ring_depth = 0, pde_ring = 0;
@@ -342,6 +352,9 @@ int allocate(mor_handle* h) {
     return MOR_OK;
 }
 
+// The largest dynamic shared memory allocate() gives the frame kernel.
+constexpr size_t kMaxFrameSmem = kSmallK * sizeof(unsigned long long) > kLinkSmem ? kSmallK * sizeof(unsigned long long) : kLinkSmem;
+
 // A handle whose max_clusters exceeds kSmallK runs the frame kernels' LK instantiations (the group-wide large-K steps);
 // every other handle the instantiations without them.
 inline bool large_k(const mor_handle* h) { return h->kmax > (uint32_t)kSmallK; }
@@ -355,6 +368,8 @@ template <bool LK>
 int configure_frame_kernels(mor_handle* h) {
     MOR_CUDA(cudaFuncSetAttribute(k_frame<LK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
     MOR_CUDA(cudaFuncSetAttribute(k_frame_batch<LK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
+    // (a mixed batched step launches with the largest frame_smem of its handles, which any handle's may be)
+    MOR_CUDA(configure_frame_batch_mixed(kMaxFrameSmem));
     MOR_CUDA(cudaFuncSetAttribute(k_frame_pipe<LK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
     MOR_CUDA(cudaFuncSetAttribute(k_frame_pipe_ground<LK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
     MOR_CUDA(cudaFuncSetAttribute(k_frame_pipe_pde<LK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->frame_smem));
@@ -745,6 +760,63 @@ int reset_state(mor_handle* h) {
     return MOR_OK;
 }
 
+// The next of the leader's four argument slots for a batched step, at least `bytes` long (pinned host + device). The H2D
+// copy of a slot runs later on the stream, so a slot is only rewritten once the step that used it four steps ago has
+// consumed it: the caller records batch_ev[*slot] after its copy.
+int batch_ring_slot(mor_handle* h, size_t bytes, uint8_t** host, uint8_t** dev, int* slot) {
+    bytes = align_up(bytes, 256);
+    if (bytes > h->batch_bytes) {
+        MOR_CUDA(cudaStreamSynchronize(h->stream));
+        if (h->d_batch) cudaFree(h->d_batch);
+        if (h->h_batch) cudaFreeHost(h->h_batch);
+        h->d_batch = nullptr; h->h_batch = nullptr; h->batch_bytes = 0;
+        MOR_CUDA(cudaMalloc(&h->d_batch, bytes * 4));
+        MOR_CUDA(cudaMallocHost(&h->h_batch, bytes * 4));
+        for (auto& e : h->batch_ev) if (!e) MOR_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+        h->batch_bytes = bytes;
+    }
+    *slot = h->batch_slot;
+    h->batch_slot = (*slot + 1) & 3;
+    MOR_CUDA(cudaEventSynchronize(h->batch_ev[*slot]));
+    *host = h->h_batch + (size_t)*slot * h->batch_bytes;
+    *dev = h->d_batch + (size_t)*slot * h->batch_bytes;
+    return MOR_OK;
+}
+
+// The CTA groups of a mixed batched step (k_frame_batch_mixed) for frames of n[s] points on C CTAs. S <= C: one group per
+// sequence, sized in proportion to its point count with a floor of one CTA (the CTAs left over by the rounding go to the
+// largest frames). S > C: C groups of one CTA each, longest-processing-time packing: the sequences in descending size,
+// each to the least-loaded group. groups[g] = {first CTA, size, begin, end} into order; G_of[s] = its group's size.
+void plan_mixed_groups(const std::vector<uint32_t>& n, int C, std::vector<int4>& groups, std::vector<int>& order, std::vector<int>& G_of) {
+    const int S = (int)n.size();
+    std::vector<int> by_size(S);
+    for (int s = 0; s < S; s++) by_size[s] = s;
+    std::stable_sort(by_size.begin(), by_size.end(), [&](int a, int b) { return n[a] > n[b]; });
+    groups.clear(); order.clear(); G_of.assign(S, 1);
+    if (S <= C) {
+        uint64_t total = 0;
+        for (int s = 0; s < S; s++) total += n[s] ? n[s] : 1;
+        int used = 0;
+        for (int s = 0; s < S; s++) { G_of[s] = 1 + (int)((uint64_t)(C - S) * (n[s] ? n[s] : 1) / total); used += G_of[s]; }
+        for (int i = 0; used < C; i = (i + 1) % S, used++) G_of[by_size[i]]++;
+        int first = 0;
+        for (int s = 0; s < S; s++) { groups.push_back(make_int4(first, G_of[s], s, s + 1)); order.push_back(s); first += G_of[s]; }
+        return;
+    }
+    std::vector<uint64_t> load(C, 0);
+    std::vector<std::vector<int>> members(C);
+    for (int s : by_size) {
+        int g = 0;
+        for (int k = 1; k < C; k++) if (load[k] < load[g]) g = k;
+        load[g] += n[s] ? n[s] : 1;
+        members[g].push_back(s);
+    }
+    for (int g = 0; g < C; g++) {
+        groups.push_back(make_int4(g, 1, (int)order.size(), (int)(order.size() + members[g].size())));
+        order.insert(order.end(), members[g].begin(), members[g].end());
+    }
+}
+
 }  // namespace
 
 // ============================================================================================ C ABI
@@ -893,23 +965,11 @@ int mor_batch_step_device(mor_handle* const* hs, uint32_t S, const void* const* 
     static_assert(sizeof(FramePtrs) % alignof(GroundPtrs) == 0, "GroundPtrs follow the FramePtrs of a ring slot");
     static_assert((sizeof(FramePtrs) + sizeof(GroundPtrs)) % alignof(RecordPtrs) == 0, "RecordPtrs follow the GroundPtrs of a ring slot");
     const size_t per_seq = sizeof(FramePtrs) + sizeof(GroundPtrs) + sizeof(RecordPtrs);
-    if (S > h->batch_cap) {
-        MOR_CUDA(cudaStreamSynchronize(st));
-        if (h->d_batch) cudaFree(h->d_batch);
-        if (h->h_batch) cudaFreeHost(h->h_batch);
-        h->d_batch = nullptr; h->h_batch = nullptr; h->batch_cap = 0;
-        MOR_CUDA(cudaMalloc(&h->d_batch, per_seq * S * 4));
-        MOR_CUDA(cudaMallocHost(&h->h_batch, per_seq * S * 4));
-        for (auto& e : h->batch_ev) if (!e) MOR_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        h->batch_cap = S;
-    }
-    // ring of 4 argument slots: the H2D copy of a slot runs later on the stream, so a slot is only rewritten once the
-    // step that used it four steps ago has consumed it
-    const int slot = h->batch_slot;
-    h->batch_slot = (slot + 1) & 3;
-    MOR_CUDA(cudaEventSynchronize(h->batch_ev[slot]));
-    FramePtrs* hp = reinterpret_cast<FramePtrs*>(h->h_batch + (size_t)slot * per_seq * h->batch_cap);
-    FramePtrs* dp = reinterpret_cast<FramePtrs*>(h->d_batch + (size_t)slot * per_seq * h->batch_cap);
+    int slot;
+    uint8_t *h_slot, *d_slot;
+    { int rs = batch_ring_slot(h, per_seq * S, &h_slot, &d_slot, &slot); if (rs != MOR_OK) return rs; }
+    FramePtrs* hp = reinterpret_cast<FramePtrs*>(h_slot);
+    FramePtrs* dp = reinterpret_cast<FramePtrs*>(d_slot);
     GroundPtrs* hg = reinterpret_cast<GroundPtrs*>(hp + S);
     const GroundPtrs* dg = reinterpret_cast<const GroundPtrs*>(dp + S);
     RecordPtrs* hr = reinterpret_cast<RecordPtrs*>(hg + S);
@@ -959,6 +1019,128 @@ int mor_batch_step_device(mor_handle* const* hs, uint32_t S, const void* const* 
         h->launches++;
         const cudaError_t e = cudaGetLastError();
         if (e != cudaSuccess) { h->last_error = std::string("k_gather_records_batch: ") + cudaGetErrorString(e); return MOR_ERR_CUDA; }
+    }
+    for (uint32_t s = 0; s < S; s++) {  // push + filter in one call: the frame is committed
+        hs[s]->mo_parity ^= 1;
+        hs[s]->frame.mo_parity = hs[s]->mo_parity;
+        hs[s]->filtered = true;
+    }
+    return MOR_OK;
+}
+
+// One pushRawCloudAndPose + filterCloud for S independent sequences that may differ in everything but their device: frame
+// count, configuration, limits, record layout and output records. One launch of k_frame_batch_mixed (CTA groups sized
+// per frame, plan_mixed_groups) for all S; the nine ground launches over the sequences with ground_mode 1 / 2 only; one
+// gather over the sequences with output records only.
+int mor_batch_step_device_mixed(mor_handle* const* hs, uint32_t S, const mor_batch_frame* frames) {
+    if (!hs || !S || !frames || !hs[0]) return MOR_ERR_ARG;
+    mor_handle* h = hs[0];  // leader: owns the stream and the argument ring of the batch
+    auto fail = [&](int status, uint32_t s, const char* rule) {
+        char msg[200];
+        std::snprintf(msg, sizeof msg, "mixed batched step, sequence %u: %s", s, rule);
+        h->last_error = msg;
+        return status;
+    };
+    // every rule is checked before anything is enqueued or changed: a refused step leaves every handle as it was
+    uint32_t n_ground = 0, n_rec = 0;
+    bool lk = false;
+    size_t smem = 0;
+    for (uint32_t s = 0; s < S; s++) {
+        const mor_handle* g = hs[s];
+        const mor_batch_frame& f = frames[s];
+        if (!g) return fail(MOR_ERR_ARG, s, "null handle");
+        if (g->device != h->device) return fail(MOR_ERR_ARG, s, "all handles must be on one device");
+        if (g->inflight) return fail(MOR_ERR_ARG, s, "the handle has submitted frames in flight: collect them first");
+        if (g->profiling) return fail(MOR_ERR_ARG, s, "the handle has kernel profiling on");
+        if (validate_layout(f.point_step, f.off_x, f.off_y, f.off_z, f.off_i) != MOR_OK)
+            return fail(MOR_ERR_ARG, s, "point_step / field offsets do not describe a record with float32 x, y, z");
+        if ((!f.d_data && f.n) || !f.d_out) return fail(MOR_ERR_ARG, s, "null d_data or d_out");
+        if (f.n > g->nmax) return fail(MOR_ERR_CAPACITY, s, "frame larger than mor_limits.max_points");
+        if (g->out_records && (size_t)f.n * f.point_step > g->d_in_bytes)
+            return fail(MOR_ERR_CAPACITY, s, "output records: n * point_step exceeds the output buffer (32 B x max_points)");
+        n_ground += g->cfg.ground_mode != MOR_GROUND_CROP;
+        n_rec += g->out_records;
+        lk = lk || large_k(g);
+        smem = g->frame_smem > smem ? g->frame_smem : smem;
+    }
+    {
+        std::vector<std::pair<const mor_handle*, uint32_t>> seen(S);
+        for (uint32_t s = 0; s < S; s++) seen[s] = {hs[s], s};
+        std::sort(seen.begin(), seen.end());
+        for (uint32_t s = 1; s < S; s++)
+            if (seen[s].first == seen[s - 1].first) return fail(MOR_ERR_ARG, seen[s].second, "the handle appears twice in the batch");
+    }
+    if (n_ground > 65535u || n_rec > 65535u) { h->last_error = "mixed batched step: at most 65535 sequences with a voxel ground mode and 65535 with output records"; return MOR_ERR_ARG; }
+    MOR_CUDA(cudaSetDevice(h->device));
+    cudaStream_t st = h->stream;
+    for (uint32_t s = 0; s < S; s++) { int fs = flush_back(hs[s]); if (fs != MOR_OK) return fs; }
+    // CTA groups
+    std::vector<uint32_t> n(S);
+    for (uint32_t s = 0; s < S; s++) n[s] = frames[s].n;
+    std::vector<int4> groups;
+    std::vector<int> order, G_of;
+    plan_mixed_groups(n, h->frame_ctas, groups, order, G_of);
+    // ring slot: FramePtrs[S] | ground subset FramePtrs[Sg], GroundPtrs[Sg] | records subset RecordPtrs[Sr], int[Sr] |
+    // group table int4[groups] + int[S]
+    const size_t off_pg = align_up(sizeof(FramePtrs) * S, 16);
+    const size_t off_gg = off_pg + align_up(sizeof(FramePtrs) * n_ground, 16);
+    const size_t off_r = off_gg + align_up(sizeof(GroundPtrs) * n_ground, 16);
+    const size_t off_rn = off_r + align_up(sizeof(RecordPtrs) * n_rec, 16);
+    const size_t off_t = off_rn + align_up(sizeof(int) * n_rec, 16);
+    const size_t bytes = off_t + sizeof(int4) * groups.size() + sizeof(int) * S;
+    int slot;
+    uint8_t *hb, *db;
+    { int rs = batch_ring_slot(h, bytes, &hb, &db, &slot); if (rs != MOR_OK) return rs; }
+    FramePtrs* hp = reinterpret_cast<FramePtrs*>(hb);
+    FramePtrs* hpg = reinterpret_cast<FramePtrs*>(hb + off_pg);
+    GroundPtrs* hgg = reinterpret_cast<GroundPtrs*>(hb + off_gg);
+    RecordPtrs* hr = reinterpret_cast<RecordPtrs*>(hb + off_r);
+    int* hrn = reinterpret_cast<int*>(hb + off_rn);
+    std::memcpy(hb + off_t, groups.data(), sizeof(int4) * groups.size());
+    std::memcpy(hb + off_t + sizeof(int4) * groups.size(), order.data(), sizeof(int) * S);
+    uint32_t ig = 0, ir = 0, n_max_g = 0, n_max_r = 0;
+    for (uint32_t s = 0; s < S; s++) {
+        mor_handle* g = hs[s];
+        const mor_batch_frame& f = frames[s];
+        if (g->last_stream != st) {  // earlier work of this handle ran elsewhere (its own stream or another batch): wait for it once
+            if (g->last_stream) MOR_CUDA(cudaStreamSynchronize(g->last_stream));
+            if (g->stream != st) MOR_CUDA(cudaStreamSynchronize(g->stream));
+        }
+        advance_frame(g, f.n, f.pose7);
+        g->out_cur = g->slot[0].d_out;
+        fill_frame(g, (const uint8_t*)f.d_data, f.n, f.point_step, f.off_x, f.off_y, f.off_z, f.off_i);
+        if (g->frame_rec) {  // the frame kernel's PointXYZI records go to the handle's own buffer, the gather alone writes d_out
+            hr[ir] = record_ptrs(g, g->frame, f.d_out);
+            hrn[ir++] = (int)rec_blocks(f.n);
+            n_max_r = f.n > n_max_r ? f.n : n_max_r;
+            g->rec_out = f.d_out;
+        } else {
+            g->frame.out = (float4*)f.d_out;
+        }
+        set_segments(g, g->frame, G_of[s]);
+        hp[s] = g->frame;
+        if (g->cfg.ground_mode != MOR_GROUND_CROP) {
+            hpg[ig] = g->frame; hgg[ig++] = g->ground;
+            n_max_g = f.n > n_max_g ? f.n : n_max_g;
+        }
+        g->last_stream = st;
+    }
+    MOR_CUDA(cudaMemcpyAsync(db, hb, bytes, cudaMemcpyHostToDevice, st));
+    MOR_CUDA(cudaEventRecord(h->batch_ev[slot], st));
+    if (n_ground) {  // voxel-covariance ground removal of the frames that use it: 9 launches, then the frame kernel takes over
+        int gs = enqueue_ground_batch(h, reinterpret_cast<const FramePtrs*>(db + off_pg), reinterpret_cast<const GroundPtrs*>(db + off_gg), n_ground, n_max_g);
+        if (gs != MOR_OK) return gs;
+    }
+    {
+        const unsigned grid = (unsigned)(groups.back().x + groups.back().y);
+        cudaError_t e = launch_frame_batch_mixed(lk, grid, smem, st, db, db + off_t, (int)groups.size());
+        h->launches++;
+        if (e != cudaSuccess) { h->last_error = std::string("k_frame_batch_mixed: ") + cudaGetErrorString(e); return MOR_ERR_CUDA; }
+    }
+    if (n_rec) {  // one gather launch for the sequences with output records
+        const cudaError_t e = launch_gather_records_mixed(rec_blocks(n_max_r), n_rec, st, db + off_r, db + off_rn);
+        h->launches++;
+        if (e != cudaSuccess) { h->last_error = std::string("k_gather_records_mixed: ") + cudaGetErrorString(e); return MOR_ERR_CUDA; }
     }
     for (uint32_t s = 0; s < S; s++) {  // push + filter in one call: the frame is committed
         hs[s]->mo_parity ^= 1;

@@ -143,6 +143,27 @@ int mor_batch_step_device(mor_handle* const* hs, uint32_t S, const void* const* 
                           uint32_t point_step, uint32_t off_x, uint32_t off_y, uint32_t off_z, uint32_t off_i,
                           const double* poses7, void* const* d_out);
 
+/* Mixed batched step: like mor_batch_step_device, but the S sequences may differ in everything except their device. Per
+ * sequence: the frame count (a handle just created or reset runs its first frame beside handles in steady state), every
+ * configuration key (method_choice, ground_mode, trim, radius, cluster sizes, n_bad / n_good, ...), the limits, the record
+ * layout of frames[s] and mor_set_output_records. Each sequence gets exactly the push + filterCloud its own handle would
+ * do with mor_push_raw_cloud_and_pose_device + mor_filter_cloud_device(d_out). One launch of the frame kernel whose CTA
+ * groups are sized in proportion to each frame's point count (at least one CTA each; more sequences than SMs are packed
+ * longest frame first onto the least-loaded CTA), the nine ground-stage launches over the sequences with ground_mode 1 /
+ * 2 only, and one gather launch over the sequences with output records only.
+ * All handles must be on one device, none may appear twice, have submitted frames in flight or kernel profiling on:
+ * MOR_ERR_ARG, and mor_last_error(hs[0]) names the sequence and the rule. n > max_points of its handle, or with output
+ * records n * point_step above 32 B x max_points, is MOR_ERR_CAPACITY. A refused step changes no handle. At most 65535
+ * sequences with a voxel ground mode and 65535 with output records per step. frames[s].d_out must hold n records of the
+ * handle's output (32-byte PointXYZI, or point_step bytes with output records). Asynchronous on hs[0]'s stream, like
+ * mor_batch_step_device. */
+typedef struct mor_batch_frame {
+    const void* d_data; uint32_t n, point_step, off_x, off_y, off_z, off_i;
+    double pose7[7];
+    void* d_out;
+} mor_batch_frame;
+int mor_batch_step_device_mixed(mor_handle* const* hs, uint32_t S, const mor_batch_frame* frames);
+
 /* ---- pipelined streaming, host buffers (replay of recorded data / throughput) ------------- */
 /* One frame of the callback body of the reference's node (external_sync_test.cpp:9-21: pushRawCloudAndPose, then
  * filterCloud, then publish `output`) as two calls that do not wait for the device in between:
