@@ -147,6 +147,7 @@ struct mor_handle {
     // products of the front half that only the back half of the SAME frame reads: two, by frame parity
     int* scid2[2]; float4* gpts2[2]; int* gsrc2[2]; int* cloud_src2[2]; uint8_t* removed_mask2[2];
     unsigned long long* acc_sum2[2]; unsigned* acc_box2[2];
+    int* slead2[2]; int* hook2[2]; int* rmin2[2]; int* cid_of_pos2[2];  // what the statistics phase resolves every point's cluster from
     // method 1 only: the clustering grid by frame parity (a pipelined back half searches its frame's grid while the front
     // half of the next frame builds the other one); otherwise both are base.table / base.cell_list
     Cell* table2[2]; int* cell_list2[2];
@@ -310,6 +311,8 @@ int allocate(mor_handle* h) {
             h->scid2[f] = f ? carve<int>(p, N) : b.scid; h->gpts2[f] = f ? carve<float4>(p, N) : b.gpts; h->gsrc2[f] = f ? carve<int>(p, N) : b.gsrc;
             h->cloud_src2[f] = f ? carve<int>(p, N) : b.cloud_src; h->removed_mask2[f] = f ? carve<uint8_t>(p, N) : b.removed_mask;
             h->acc_sum2[f] = f ? carve<unsigned long long>(p, K * 6) : b.acc_sum; h->acc_box2[f] = f ? carve<unsigned>(p, K * 6) : b.acc_box;
+            h->slead2[f] = f ? carve<int>(p, N) : b.slead; h->hook2[f] = f ? carve<int>(p, N) : b.hook;
+            h->rmin2[f] = f ? carve<int>(p, N) : b.rmin; h->cid_of_pos2[f] = f ? carve<int>(p, N) : b.cid_of_pos;
             const bool own_grid = f && h->cfg.method_choice == 1;
             h->table2[f] = own_grid ? carve<Cell>(p, tab) : b.table; h->cell_list2[f] = own_grid ? carve<int>(p, N) : b.cell_list;
         }
@@ -450,6 +453,7 @@ void fill_frame(mor_handle* h, const uint8_t* d_points, uint32_t n, uint32_t ste
     const int cur = h->cur, prev = (cur + 2) % 3;
     a.scid = h->scid2[h->fpar]; a.gpts = h->gpts2[h->fpar]; a.gsrc = h->gsrc2[h->fpar]; a.cloud_src = h->cloud_src2[h->fpar]; a.removed_mask = h->removed_mask2[h->fpar];
     a.acc_sum = h->acc_sum2[h->fpar]; a.acc_box = h->acc_box2[h->fpar];
+    a.slead = h->slead2[h->fpar]; a.hook = h->hook2[h->fpar]; a.rmin = h->rmin2[h->fpar]; a.cid_of_pos = h->cid_of_pos2[h->fpar];
     a.table = h->table2[h->fpar]; a.cell_list = h->cell_list2[h->fpar];
     a.in = d_points; a.n = n; a.step = step; a.off_x = ox; a.off_y = oy; a.off_z = oz; a.off_i = oi;
     a.in_mode = input_mode(d_points, step, ox, oy, oz, oi);
@@ -502,17 +506,17 @@ int launch_gather(mor_handle* h, const FramePtrs& a) {
 struct PipeVariant { void (*kernel)(FramePtrs, FramePtrs, int); const char* name; int back32; };
 PipeVariant pipe_variant(const mor_handle* h) {
     const bool ground = h->cfg.ground_mode != MOR_GROUND_CROP, pde = h->cfg.method_choice == 1;
-    // 5/32 (23 of 148 CTAs): measured optimum on C2 (swept 100 ... 140: the front half holds two thirds of a frame's chain of
-    // phases and is tile-granular in its first one, the back half is three short phases over the points plus its
-    // single-CTA steps). The variants, swept with tools/pipe_modes_run.py on C4 / C1 / HDL-64 frames (BASELINE.md): the voxel
-    // ground modes have C2's front half after their ground stage and the same optimum; method 1's back half holds the
-    // point-distance search, one thread per point of the previous frame's clusters, and needs 11/32 (50 CTAs) - at 5/32 a
-    // pipelined HDL-64 frame is 30 % slower than one kernel per frame, at 11/32 it is faster on every configuration measured.
+    // 7/32 (32 of 148 CTAs): measured optimum on C2 (swept 109 ... 125 front CTAs, flat between 113 and 117: the front half
+    // ends at the cluster selection and barely shortens with more CTAs, the back half is four phases over the points - the
+    // cluster statistics among them - plus its single-CTA steps). The variants, swept with tools/pipe_modes_run.py on C4 /
+    // C1 / HDL-64 frames (BASELINE.md): the voxel ground modes have C2's front half after their ground stage and take the
+    // same share; method 1's back half holds the point-distance search, one thread per point of the previous frame's
+    // clusters, and needs 13/32 (60 CTAs) - at 5/32 a pipelined HDL-64 frame is a third slower than one kernel per frame.
     const bool lk = large_k(h);
-    if (ground) return pde ? PipeVariant{lk ? k_frame_pipe_ground_pde<true> : k_frame_pipe_ground_pde<false>, "k_frame_pipe_ground_pde", 11}
-                           : PipeVariant{lk ? k_frame_pipe_ground<true> : k_frame_pipe_ground<false>, "k_frame_pipe_ground", 5};
-    return pde ? PipeVariant{lk ? k_frame_pipe_pde<true> : k_frame_pipe_pde<false>, "k_frame_pipe_pde", 11}
-               : PipeVariant{lk ? k_frame_pipe<true> : k_frame_pipe<false>, "k_frame_pipe", 5};
+    if (ground) return pde ? PipeVariant{lk ? k_frame_pipe_ground_pde<true> : k_frame_pipe_ground_pde<false>, "k_frame_pipe_ground_pde", 13}
+                           : PipeVariant{lk ? k_frame_pipe_ground<true> : k_frame_pipe_ground<false>, "k_frame_pipe_ground", 7};
+    return pde ? PipeVariant{lk ? k_frame_pipe_pde<true> : k_frame_pipe_pde<false>, "k_frame_pipe_pde", 13}
+               : PipeVariant{lk ? k_frame_pipe<true> : k_frame_pipe<false>, "k_frame_pipe", 7};
 }
 // Pipelined launches (k_frame_pipe): the front half of `front` on most CTAs beside the pending back half, or either alone.
 int launch_pipe(mor_handle* h, const FramePtrs* front, const FramePtrs* back) {

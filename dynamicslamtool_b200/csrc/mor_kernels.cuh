@@ -11,10 +11,10 @@
 // that does not exist) and meets at a group barrier in between. One sequence takes the whole GPU (G = #SMs); S
 // sequences per launch (mor_batch_step_device) take G = #SMs / S CTAs each and run independently side by side.
 // The same phase functions can be launched one kernel per phase (k_phase<>, per-phase timing for bench.py), and as
-// k_frame_pipe: the front half of one frame (ingest ... cluster statistics) on most CTAs beside the back half of the
-// frame before it (transform, match, moving test, chain, filter) on the rest - the throughput mode, see the end of the
-// file. Clustering is done on pair lists: an enumerate phase (a warp per cell) and a test phase (a thread per light
-// pair, a warp per heavy pair).
+// k_frame_pipe: the front half of one frame (ingest ... cluster selection) on most CTAs beside the back half of the
+// frame before it (cluster statistics, transform, match, moving test, chain, filter) on the rest - the throughput mode,
+// see the end of the file. Clustering is done on pair lists: an enumerate phase (a warp per cell) and a test phase (a
+// thread per light pair, a warp per heavy pair).
 #pragma once
 #include <cstdio>
 #include "mor_device.cuh"
@@ -101,20 +101,20 @@ struct FramePtrs {
     int* cell_list;            // [n_cells] table slot of every occupied cell, in creation order
     unsigned long long* ckey; int* cstart; int* ccnt;  // [n_cells] compact copies: key, first sorted position, points
     int2* pslot;               // [N_c] (table slot, rank inside the cell) of every cloud point
-    int* slead;                // [N_c] leader position (cell start = the cell's node) of every sorted position
+    int* slead;                // [N_c] leader position (cell start = the cell's node) of every sorted position; per frame parity
     // link lists: cell pairs to test (light: one thread, heavy: one warp; compact lists, a CTA adds its records in one
     // block) and the connected pairs found (node A, node B; one segment per CTA of the group, no shared counter)
     int2* light; int light_cap;
     int4* heavy; int heavy_cap;
     int2* edges; int edge_seg; int* edge_cnt;
-    int* hook;                 // [N_c, at leader positions] union-find over the nodes: parent word (pointers lead to smaller positions)
-    int* rsize; int* rmin;     // [N_c, at root positions] per root: points and minimum cloud index (= canonical label) of its component
+    int* hook;                 // [N_c, at leader positions] union-find over the nodes: parent word (pointers lead to smaller positions); per frame parity
+    int* rsize; int* rmin;     // [N_c, at root positions] per root: points and minimum cloud index (= canonical label) of its component; rmin per frame parity
     int* root_list;            // [n_roots] the roots, in no particular order
     // ---- per-frame scratch
     Scratch* scratch; unsigned long long* st_ingest; unsigned long long* st_out;
     uint8_t* point_class; uint8_t* removed_mask;
     int* cloud_src; float4* gpts; int* gsrc;
-    int* label; int* cid_of_root; int* cid_of_pos;  // cluster id by canonical label / by root position (-1: not a size-valid cluster)
+    int* label; int* cid_of_root; int* cid_of_pos;  // cluster id by canonical label / by root position (-1: not a size-valid cluster); cid_of_pos per frame parity
     int* scid;                 // cluster id per sorted position
     unsigned long long* acc_sum;  // [kmax*6] hi/lo per axis
     unsigned* acc_box;            // [kmax*6] min xyz, max xyz keys
@@ -127,7 +127,7 @@ struct FramePtrs {
     unsigned long long* lattice; unsigned lattice_mask;
     uint8_t* cluster_removed; int* found;
     int* marker_cluster;          // [momax] cluster each mo_vec entry was matched to by the last filterCloud
-    unsigned long long* phase_ts; // [PH__COUNT + 1] %globaltimer at the start of the frame kernel and after every phase (CTA 0)
+    unsigned long long* phase_ts; // [32] %globaltimer at the start of the frame kernel and after every phase (CTA 0); then the pipelined launch's (TS_FRONT, TS_BACK)
     unsigned long long* cta_trace; // [32][256] debug builds (MOR_CTA_TRACE): when every CTA reached the barrier of every phase
     float4* out;
     // ---- ping-pong frame state: cur / prev
@@ -622,30 +622,43 @@ __device__ __forceinline__ void block_cluster_accumulate(unsigned long long* acc
 // pcl_ros::transformPointCloud of every previous-frame cluster (cpp:544-551, A12), the bounding box of the transformed
 // points (getMinMax3D runs after the transform, cpp:272) and, for method 2, their octree leaves (cpp:319-324). Depends
 // on the previous frame only: it runs beside the single-CTA cluster selection, on the CTAs that one does not need.
+// One point's work in steps that each end at a dependent load (load, look-up, finish), so that the pipelined back half
+// can run it beside the cluster statistics with both chains of loads in flight at once (stats_transform).
+struct XformItem { float4 p; int k; float3 t; };
+__device__ __forceinline__ void xform_load(const FramePtrs& a, int s, int hi, XformItem& it) {
+    it.k = -1; it.t = make_float3(0, 0, 0);
+    if (s < hi) it.p = a.p_spts[s];
+}
+__device__ __forceinline__ void xform_lookup(const FramePtrs& a, int s, int hi, XformItem& it) {
+    if (s < hi) it.k = a.p_cid[__float_as_int(it.p.w)];
+}
+__device__ __forceinline__ void xform_finish(const FramePtrs& a, int s, int hi, bool wide, XformItem& it) {
+    if (s >= hi) return;
+    const int c = __float_as_int(it.p.w), k = it.k;
+    if (k >= 0) {
+        it.t = xform(a.M, it.p.x, it.p.y, it.p.z);
+        a.tpts[c] = make_float4(it.t.x, it.t.y, it.t.z, __int_as_float(k));
+        if (a.method == 2) {
+            unsigned long long key;
+            if (lattice_key(a.anchorp + (size_t)k * 3, k, it.t.x, it.t.y, it.t.z, &key, wide)) hset_insert(a.lattice, a.lattice_mask, key);
+            else atomicOr(&a.scratch->err_early, ERR_LATTICE_RANGE);
+        }
+    } else {
+        a.tpts[c] = make_float4(0, 0, 0, __int_as_float(-1));
+    }
+}
+template <bool LK>
+__device__ __forceinline__ bool lattice_wide(const FramePtrs& a) { return LK && a.p_counts[MOR_CNT_K] > kLatticeNarrowK; }
 template <bool LK>
 __device__ __forceinline__ void transform_range(const FramePtrs& a, int lo, int hi) {
-    const bool wide = LK && a.p_counts[MOR_CNT_K] > kLatticeNarrowK;
+    const bool wide = lattice_wide<LK>(a);
     for (int base = lo; base < hi; base += kT) {
         const int s = base + threadIdx.x;
-        int k = -1;
-        float3 t = make_float3(0, 0, 0);
-        if (s < hi) {
-            const float4 p = a.p_spts[s];
-            const int c = __float_as_int(p.w);
-            k = a.p_cid[c];
-            if (k >= 0) {
-                t = xform(a.M, p.x, p.y, p.z);
-                a.tpts[c] = make_float4(t.x, t.y, t.z, __int_as_float(k));
-                if (a.method == 2) {
-                    unsigned long long key;
-                    if (lattice_key(a.anchorp + (size_t)k * 3, k, t.x, t.y, t.z, &key, wide)) hset_insert(a.lattice, a.lattice_mask, key);
-                    else atomicOr(&a.scratch->err_early, ERR_LATTICE_RANGE);
-                }
-            } else {
-                a.tpts[c] = make_float4(0, 0, 0, __int_as_float(-1));
-            }
-        }
-        block_cluster_accumulate<false>(nullptr, a.pacc_box, k, k >= 0, t.x, t.y, t.z);
+        XformItem it;
+        xform_load(a, s, hi, it);
+        xform_lookup(a, s, hi, it);
+        xform_finish(a, s, hi, wide, it);
+        block_cluster_accumulate<false>(nullptr, a.pacc_box, it.k, it.k >= 0, it.t.x, it.t.y, it.t.z);
     }
 }
 template <bool LK>
@@ -1283,29 +1296,69 @@ __device__ __noinline__ void phase_select_large(const FramePtrs& a, int cta, int
 
 // ===================================================================================== phase G: cluster statistics
 // Per-cluster statistics (cpp:221-244): cluster id of every point, exact coordinate sums for
-// compute3DCentroid<double> (A10) and getMinMax3D bounding boxes (cpp:272-275).
+// compute3DCentroid<double> (A10) and getMinMax3D bounding boxes (cpp:272-275). Needs the selection (cid_of_pos) and
+// nothing of the match: a pipelined launch runs it at the start of the back half, so the front half ends at the select.
+// One point's statistics in the same kind of steps: the point and its cell's node, the node's root (hook is flat), the
+// root's label and cluster id, then the stores.
+struct StatsItem { float4 p; int x, lab, k; };
+__device__ __forceinline__ void stats_load(const FramePtrs& a, int s, int hi, StatsItem& it) {
+    it.p = make_float4(0, 0, 0, 0); it.k = -1;
+    if (s < hi) { it.p = a.spts[s]; it.x = a.slead[s]; }
+}
+__device__ __forceinline__ void stats_root(const FramePtrs& a, int s, int hi, StatsItem& it) {
+    if (s < hi) it.x = a.hook[it.x];  // consecutive points share these words
+}
+__device__ __forceinline__ void stats_lookup(const FramePtrs& a, int s, int hi, StatsItem& it) {
+    if (s < hi) { it.lab = a.rmin[it.x]; it.k = a.cid_of_pos[it.x]; }
+}
+__device__ __forceinline__ void stats_finish(const FramePtrs& a, int s, int hi, int nc, const StatsItem& it) {
+    if (s >= hi) return;
+    const int c = __float_as_int(it.p.w);
+    MOR_CHECK(it.lab >= 0 && it.lab < nc, "label", it.lab);
+    a.label[c] = it.lab;
+    a.cid[c] = it.k;
+    a.scid[s] = it.k;
+}
 __device__ __forceinline__ void phase_stats(const FramePtrs& a, int cta, int G) {
     const int nc = frame_vars().nc;
     int lo, hi;
     cta_slice(nc, cta, G, &lo, &hi);
     for (int base = lo; base < hi; base += kT) {
         const int s = base + threadIdx.x;
-        float4 p = make_float4(0, 0, 0, 0);
-        int k = -1;
-        if (s < hi) {
-            p = a.spts[s];
-            const int c = __float_as_int(p.w);
-            const int root = a.hook[a.slead[s]];  // hook is flat: the cell's root; consecutive points share these words
-            const int lab = a.rmin[root];
-            MOR_CHECK(lab >= 0 && lab < nc, "label", lab);
-            a.label[c] = lab;
-            k = a.cid_of_pos[root];
-            a.cid[c] = k;
-            a.scid[s] = k;
-        }
-        block_cluster_accumulate<true>(a.acc_sum, a.acc_box, k, k >= 0, p.x, p.y, p.z);
+        StatsItem it;
+        stats_load(a, s, hi, it);
+        stats_root(a, s, hi, it);
+        stats_lookup(a, s, hi, it);
+        stats_finish(a, s, hi, nc, it);
+        block_cluster_accumulate<true>(a.acc_sum, a.acc_box, it.k, it.k >= 0, it.p.x, it.p.y, it.p.z);
     }
 }
+// The pipelined back half's first phase: the previous clusters' transform (transform_range) and this frame's
+// statistics (phase_stats) in one loop, step by step, so that a round waits for the two chains of dependent loads side
+// by side instead of one after the other.
+template <bool LK>
+__device__ __forceinline__ void stats_transform(const FramePtrs& a, int cta, int G) {
+    const int nc = frame_vars().nc;
+    const bool wide = lattice_wide<LK>(a);
+    int lo_s, hi_s, lo_t = 0, hi_t = 0;
+    cta_slice(nc, cta, G, &lo_s, &hi_s);
+    if (a.two_frames) cta_slice(a.p_counts[MOR_CNT_NC], cta, G, &lo_t, &hi_t);
+    for (int r = 0; lo_s + r < hi_s || lo_t + r < hi_t; r += kT) {  // (uniform over the CTA)
+        const int s = lo_s + r + threadIdx.x, t = lo_t + r + threadIdx.x;
+        StatsItem is;
+        XformItem ix;
+        stats_load(a, s, hi_s, is);
+        xform_load(a, t, hi_t, ix);
+        stats_root(a, s, hi_s, is);
+        xform_lookup(a, t, hi_t, ix);
+        stats_lookup(a, s, hi_s, is);
+        xform_finish(a, t, hi_t, wide, ix);
+        stats_finish(a, s, hi_s, nc, is);
+        block_cluster_accumulate<false>(nullptr, a.pacc_box, ix.k, ix.k >= 0, ix.t.x, ix.t.y, ix.t.z);
+        block_cluster_accumulate<true>(a.acc_sum, a.acc_box, is.k, is.k >= 0, is.p.x, is.p.y, is.p.z);
+    }
+}
+
 
 // Block-wide ordered compaction helper for the single-CTA phases: returns the exclusive rank of `flag` among all
 // threads, *total = number of set flags. kSingle threads.
@@ -2171,12 +2224,14 @@ __device__ __forceinline__ void frame_body(const FramePtrs& a, int cta, int G, F
 
 // ===================================================================================== pipelined launch
 // Throughput mode (mor_set_pipelining; frames are known one ahead - replay, the streaming calls): clustering a frame needs
-// nothing of the frame before it, so ONE launch runs the front half of frame f+1 (ingest ... cluster statistics) on the
-// first Gf CTAs beside the back half of frame f (transform, match, moving test, chain, filter) on the others. The two
-// groups have their own barriers and counters and touch disjoint state: what the back half reads of frame f and f-1 is
-// triple-buffered (points, cluster ids, cluster tables, counts) or double-buffered (ground points, source indices, masks,
-// the clusters' coordinate sums and boxes)
-// on the host side (mor_b200.cu, fill_frame).
+// nothing of the frame before it, so ONE launch runs the front half of frame f+1 (ingest ... cluster selection) on the
+// first Gf CTAs beside the back half of frame f (cluster statistics, transform, match, moving test, chain, filter) on the
+// others. The two groups have their own barriers and counters and touch disjoint state: what the back half reads of
+// frame f and f-1 is triple-buffered (points, sorted points, cluster ids, cluster tables, counts) or double-buffered by
+// frame parity (ground points, source indices, masks, the clusters' coordinate sums and boxes, and what the statistics
+// phase resolves each point's cluster from: slead, hook, rmin, cid_of_pos; scid, which it writes) on the host side
+// (mor_b200.cu, fill_frame). The front half's other per-frame arrays (cells, pair lists, rsize, root_list, cid_of_root)
+// are read by no back half.
 // Four instantiations of the same two bodies, picked per handle by mor_b200.cu (pipe_kernel):
 //  - k_frame_pipe: crop ground mode, method 2.
 //  - k_frame_pipe_ground (GROUND): voxel ground modes. Frame f+1's nine ground launches (mor_ground.cuh) run on the stream
@@ -2200,24 +2255,35 @@ __device__ __forceinline__ void frame_body(const FramePtrs& a, int cta, int G, F
 //    handle keeps the grid (table, cell_list) per frame parity; the front half leaves it standing and hands its cell
 //    count over in counts[CNT_PIPE_CELLS]; the back half empties it after the search.
 //  - k_frame_pipe_ground_pde: both.
+// Timeline of a pipelined launch in the spare words of phase_ts (after frame_body's PH__COUNT + 1): CTA 0 of each half
+// stamps its start and every barrier it passes, the last CTA out of each half stamps the end (tools/quick_bench.py,
+// QB_PIPE=1). Front: start, ingest, cells, link, test, jump, cross, roots + select, end. Back: start, housekeeping,
+// statistics + transform + match, moving test + chain, filter (end).
+enum { TS_FRONT = PH__COUNT + 1, TS_BACK = TS_FRONT + 9 };
+static_assert(TS_BACK + 5 <= 32, "phase_ts holds 32 words");
+__device__ __forceinline__ void pipe_stamp(const FramePtrs& a, int cta, int word) {
+    if (cta == 0 && threadIdx.x == 0) a.phase_ts[word] = global_ns();
+}
+
 template <bool GROUND, bool PDE, bool LK>
 __device__ __forceinline__ void front_body(const FramePtrs& a, int cta, int G, FrameShared& sh, unsigned long long* dyn, unsigned& parity) {
     GroupBarrier bar{&a.scratch->bar, 0u, (unsigned)G};
+    pipe_stamp(a, cta, TS_FRONT);
     if (GROUND) phase_bin_cloud(a, cta, G, /*housekeep=*/false);
     else phase_ingest(a, cta, G, dyn, &sh.mbar, parity, /*housekeep=*/false);
-    bar.sync();
+    bar.sync(); pipe_stamp(a, cta, TS_FRONT + 1);
     load_frame_vars(a);
-    phase_cells(a, cta, G); bar.sync();
-    phase_link(a, cta, G, dyn); bar.sync();
-    phase_test(a, cta, G); bar.sync();
-    phase_jump(a, cta, G); bar.sync();
-    phase_cross(a, cta, G); bar.sync();
+    phase_cells(a, cta, G); bar.sync(); pipe_stamp(a, cta, TS_FRONT + 2);
+    phase_link(a, cta, G, dyn); bar.sync(); pipe_stamp(a, cta, TS_FRONT + 3);
+    phase_test(a, cta, G); bar.sync(); pipe_stamp(a, cta, TS_FRONT + 4);
+    phase_jump(a, cta, G); bar.sync(); pipe_stamp(a, cta, TS_FRONT + 5);
+    phase_cross(a, cta, G); bar.sync(); pipe_stamp(a, cta, TS_FRONT + 6);
     phase_roots(a, cta, G);
     // (the last CTA in selects the clusters: no barrier in front of it; a large-K frame is selected by the whole group)
     if (group_last_arrival(&a.scratch->tail_centroids, (unsigned)G) && !select_large<LK>(a)) phase_select(a, dyn);
     bar.sync();
     if (select_large<LK>(a)) { phase_select_large(a, cta, G, dyn, bar); bar.sync(); }
-    phase_stats(a, cta, G);  // (the sums it accumulates are double-buffered by frame parity: the back half turns them into centroids)
+    pipe_stamp(a, cta, TS_FRONT + 7);
     if (PDE) {  // the grid stays for the back half's search: only the scan states go back to zero here
         for (int t = cta * kT + threadIdx.x; t < a.tiles_pts; t += G * kT) a.st_ingest[t] = 0ull;
         if (cta == 0 && threadIdx.x == 0) a.counts[CNT_PIPE_CELLS] = frame_vars().n_cells;
@@ -2234,6 +2300,7 @@ __device__ __forceinline__ void front_body(const FramePtrs& a, int cta, int G, F
     }
     __syncthreads();
     if (s_last_front && threadIdx.x == 0) {
+        a.phase_ts[TS_FRONT + 8] = global_ns();
         Scratch* sc = a.scratch;
         sc->bar = 0u; sc->blocks_done = 0; sc->n_cells = 0; sc->n_roots = 0; sc->n_light = 0; sc->n_heavy = 0; sc->n_sorted = 0; sc->tail_centroids = 0u;
         sc->ticket_light = 0; sc->ticket_heavy = 0; sc->err_early = 0;
@@ -2252,19 +2319,16 @@ __device__ __forceinline__ void back_body(const FramePtrs& a, int cta, int G, Fr
         v.n_cells = 0; v.nc = __ldcg(&a.counts[MOR_CNT_NC]); v.ng = __ldcg(&a.counts[MOR_CNT_NG]);
     }
     __syncthreads();
+    pipe_stamp(a, cta, TS_BACK);
     frame_housekeeping(a, cta, G);
-    bar.sync();
-    if (a.two_frames) {
-        int lo, hi;
-        cta_slice(a.p_counts[MOR_CNT_NC], cta, G, &lo, &hi);
-        transform_range<LK>(a, lo, hi);
-    }
+    bar.sync(); pipe_stamp(a, cta, TS_BACK + 1);
+    stats_transform<LK>(a, cta, G);
     if (match_large<LK>(a)) { bar.sync(); phase_match_large(a, cta, G, dyn, bar); }
     else if (group_last_arrival(&a.scratch->tail_match_back, (unsigned)G)) phase_match(a, dyn);
-    bar.sync();
+    bar.sync(); pipe_stamp(a, cta, TS_BACK + 2);
     if (a.two_frames) { if (PDE) phase_pde_count(a, cta, G); else phase_lattice_count<LK>(a, cta, G); }
     if (group_last_arrival(&a.scratch->tail_chain, (unsigned)G)) phase_chain_tail(a);
-    bar.sync();
+    bar.sync(); pipe_stamp(a, cta, TS_BACK + 3);
     if (PDE) {  // the search is over: this frame's clustering grid goes back to "all zero" (frame_cleanup's first loop)
         const int n_cells = a.counts[CNT_PIPE_CELLS];
         for (int i = cta * kT + threadIdx.x; i < n_cells; i += G * kT)
@@ -2282,6 +2346,7 @@ __device__ __forceinline__ void back_body(const FramePtrs& a, int cta, int G, Fr
     if (!s_last_back) return;
     for (int t = threadIdx.x; t < a.tiles_pts; t += kT) a.st_out[t] = 0ull;
     if (threadIdx.x == 0) {
+        a.phase_ts[TS_BACK + 4] = global_ns();
         Scratch* sc = a.scratch;
         sc->bar_back = 0u; sc->blocks_done_back = 0; sc->tail_match_back = 0u; sc->tail_chain = 0u;
     }

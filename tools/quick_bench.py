@@ -1,6 +1,8 @@
 """Quick device-resident timing of one build on the C2 sequence (not the bench: no clocks check, no e2e).
-usage: [MOR_PRODUCT_LIB=...] python tools/quick_bench.py [frames=120] [warmup=20]
-Prints frames/s, the mean in-kernel phase times and a crc of the last output (equal across correct builds)."""
+usage: [MOR_PRODUCT_LIB=...] [QB_PIPE=1] python tools/quick_bench.py [frames=120] [warmup=20]
+Prints frames/s, the mean in-kernel phase times and a crc of the last output (equal across correct builds).
+QB_PIPE=1: pipelined launches, and instead of the one-kernel-per-frame phases the mean timeline of each half of a fused
+launch (front half of frame f+1 beside the back half of f; the TS_FRONT / TS_BACK words of phase_ts)."""
 import ctypes as C, sys, zlib, numpy as np
 from pathlib import Path
 sys.path.insert(0, str(Path(__file__).resolve().parent.parent))
@@ -39,6 +41,30 @@ c = m.counts()
 out = np.empty((c["NOUT"], 8), np.float32)
 b.device_download(0, out.ctypes.data_as(C.c_void_p), C.c_void_p(m.output_device()), out.nbytes)
 print(f"{(F - W) / (ms * 1e-3):8.0f} frames/s  {1e3 * ms / (F - W):7.1f} us/frame  crc {zlib.crc32(out.tobytes()):08x} errflags {c['ERRFLAGS']}")
+if os.environ.get("QB_PIPE"):
+    # per-half timeline of the fused launches (CTA 0 of each half at its barriers, the last CTA out at the end), in us,
+    # averaged over the frames after the warm-up, with a sync per frame
+    TS_FRONT, TS_BACK = 12, 21
+    FRONT = ["ingest", "cells", "link", "test", "jump", "cross", "roots+select", "end"]
+    BACK = ["housekeeping", "stats+transform+match", "moving+chain", "filter"]
+    ts = (C.c_ulonglong * 32)()
+    m.reset()
+    acc = np.zeros(len(FRONT) + len(BACK))
+    n = 0
+    for f in range(F):
+        m.push_device(d.value + f * SLOT, len(frames[f][0]), frames[f][1], point_step=STEP)
+        if f > W:  # (this push launched the front half of f beside the back half of f - 1)
+            assert b.lib.mor_debug_phase_ts(m.h, ts) == 0
+            w = np.array(ts[:], np.float64)
+            fr = np.diff(w[TS_FRONT:TS_FRONT + len(FRONT) + 1])
+            bk = np.diff(w[TS_BACK:TS_BACK + len(BACK) + 1])
+            acc += np.concatenate([fr, bk]) * 1e-3
+            n += 1
+        m.filter_device(None, 0, want_count=False)
+    acc /= max(n, 1)
+    print("  front " + "  ".join(f"{k} {v:.1f}" for k, v in zip(FRONT, acc[:len(FRONT)])) + f"  total {acc[:len(FRONT)].sum():.1f}")
+    print("  back  " + "  ".join(f"{k} {v:.1f}" for k, v in zip(BACK, acc[len(FRONT):])) + f"  total {acc[len(FRONT):].sum():.1f}")
+    sys.exit(0)
 # phase timeline, averaged over a second pass with a sync per frame
 m.reset()
 acc = {}
