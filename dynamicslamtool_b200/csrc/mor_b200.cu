@@ -211,6 +211,13 @@ void prof_harvest(mor_handle* h) {  // stream must be idle
     }
     h->prof_ids.clear();
 }
+// Every kernel launch is counted (mor_get_launch_count); one that fails is reported under the kernel's name.
+int launched(mor_handle* h, cudaError_t e, const char* kernel) {
+    h->launches++;
+    if (e == cudaSuccess) return MOR_OK;
+    h->last_error = std::string(kernel) + ": " + cudaGetErrorString(e);
+    return MOR_ERR_CUDA;
+}
 // Launch with the programmatic-stream-serialisation attribute (see pdl_prologue in mor_device.cuh): the chain of
 // short kernels of the voxel ground modes.
 template <typename... KArgs, typename... Args>
@@ -228,8 +235,7 @@ cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t s
         cudaError_t le__;                                                                          \
         if (h->profiling) { prof_begin(h, id); kernel<<<grid, block, smem, st>>>(__VA_ARGS__); le__ = cudaGetLastError(); prof_end(h); } \
         else le__ = launch_pdl(kernel, dim3(grid), dim3(block), smem, st, __VA_ARGS__);           \
-        if (le__ != cudaSuccess) { h->last_error = std::string(#kernel) + ": " + cudaGetErrorString(le__); return MOR_ERR_CUDA; } \
-        h->launches++;                                                                             \
+        if (int ls__ = launched(h, le__, #kernel)) return ls__;                                    \
     } while (0)
 
 // All CTAs of the frame kernel must be resident at once (they meet at group barriers): cooperative launch.
@@ -381,7 +387,6 @@ int configure_frame_kernels(mor_handle* h) {
     if (st == MOR_OK) st = set_phase_smem<PH_FILTER, LK>(h);
     if (st == MOR_OK) st = set_phase_smem<PH_LINK, LK>(h);
     if (st == MOR_OK) st = set_phase_smem<PH_STATS, LK>(h);
-    if (st == MOR_OK) st = set_phase_smem<PH_INGEST, LK>(h);
     return st;
 }
 int configure_kernels(mor_handle* h) {
@@ -427,11 +432,22 @@ void fill_static(mor_handle* h) {
 
 inline unsigned blocks_for(uint32_t n) { return n ? (n + kBlock - 1) / kBlock : 1; }
 
-// pcl::fromPCLPointCloud2 accepts any record layout (cpp:523): float4 records and 4-byte aligned fields are read with
-// vector / word loads, anything else (e.g. the 22-byte velodyne XYZIRT record) byte by byte.
-int validate_layout(uint32_t step, uint32_t ox, uint32_t oy, uint32_t oz, uint32_t oi) {
-    if (step < 12) return MOR_ERR_ARG;
-    if (ox > step - 4 || oy > step - 4 || oz > step - 4 || (oi != 0xFFFFFFFFu && oi > step - 4)) return MOR_ERR_ARG;
+// The rules a frame of n records meets on the handle g that takes it, on every entry point: a record layout with float32
+// x, y, z (pcl::fromPCLPointCloud2 accepts any layout, cpp:523: float4 records and 4-byte aligned fields are read with
+// vector / word loads, anything else, e.g. the 22-byte velodyne XYZIRT record, byte by byte), at most max_points records,
+// and at most 32 B x max_points bytes where the records are staged (host data) or copied out (output records). A broken
+// rule is named in report->last_error.
+int check_frame(mor_handle* report, const mor_handle* g, uint32_t n, uint32_t step, uint32_t ox, uint32_t oy, uint32_t oz, uint32_t oi, bool staged) {
+    if (step < 12 || ox > step - 4 || oy > step - 4 || oz > step - 4 || (oi != 0xFFFFFFFFu && oi > step - 4)) {
+        report->last_error = "point_step / field offsets do not describe a record with float32 x, y, z";
+        return MOR_ERR_ARG;
+    }
+    if (n > g->nmax) { report->last_error = "frame larger than mor_limits.max_points"; return MOR_ERR_CAPACITY; }
+    if ((staged || g->out_records) && (size_t)n * step > g->d_in_bytes) {
+        report->last_error = staged ? "n * point_step exceeds the staging buffer (32 B x max_points)"
+                                    : "output records: n * point_step exceeds the output buffer (32 B x max_points)";
+        return MOR_ERR_CAPACITY;
+    }
     return MOR_OK;
 }
 int input_mode(const void* d_points, uint32_t step, uint32_t ox, uint32_t oy, uint32_t oz, uint32_t oi) {
@@ -471,12 +487,10 @@ void fill_frame(mor_handle* h, const uint8_t* d_points, uint32_t n, uint32_t ste
 template <int PH>
 int launch_phase(mor_handle* h, const FramePtrs& a) {
     prof_begin(h, KID_PHASE0 + PH);
-    const size_t smem = (PH == PH_INGEST || PH == PH_SELECT || PH == PH_LINK || PH == PH_STATS || PH == PH_FILTER) ? h->frame_smem : 0;
+    const size_t smem = (PH == PH_SELECT || PH == PH_LINK || PH == PH_STATS || PH == PH_FILTER) ? h->frame_smem : 0;
     cudaError_t e = launch_coop(large_k(h) ? k_phase<PH, true> : k_phase<PH, false>, (unsigned)h->frame_ctas, smem, h->stream, a);
     prof_end(h);
-    h->launches++;
-    if (e != cudaSuccess) { h->last_error = std::string("k_phase: ") + cudaGetErrorString(e); return MOR_ERR_CUDA; }
-    return MOR_OK;
+    return launched(h, e, "k_phase");
 }
 
 // The gather of output records (mor_records.cuh) for the frame `a`, into its output buffer a.out (a batched step passes
@@ -495,10 +509,7 @@ RecordPtrs record_ptrs(const mor_handle* h, const FramePtrs& a, void* dst) {
 }
 int launch_gather(mor_handle* h, const FramePtrs& a) {
     k_gather_records<<<rec_blocks(a.n), kRecT, 0, h->stream>>>(record_ptrs(h, a, a.out));
-    h->launches++;
-    const cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) { h->last_error = std::string("k_gather_records: ") + cudaGetErrorString(e); return MOR_ERR_CUDA; }
-    return MOR_OK;
+    return launched(h, cudaGetLastError(), "k_gather_records");
 }
 
 // The pipelined launch of a handle's configuration (k_frame_pipe and its variants, mor_kernels.cuh), and the share of the
@@ -522,25 +533,20 @@ PipeVariant pipe_variant(const mor_handle* h) {
 int launch_pipe(mor_handle* h, const FramePtrs* front, const FramePtrs* back) {
     const int G = h->frame_ctas;
     const PipeVariant v = pipe_variant(h);
-    int Gf = G, Gb = 0;
+    int Gf = G;
     if (front && back && G < 8) {  // too few SMs to share: one half after the other
         int s0 = launch_pipe(h, nullptr, back);
         return s0 != MOR_OK ? s0 : launch_pipe(h, front, nullptr);
     }
     if (front && back) {
-        Gb = (G * v.back32) / 32;
-        if (Gb < 4) Gb = 4;
-        Gf = G - Gb;
+        Gf = G - std::max(4, (G * v.back32) / 32);
         if (const char* env = std::getenv("MOR_PIPE_GF")) { const int v = std::atoi(env); if (v > 0 && v < G) Gf = v; }  // (tuning)
-        Gb = G - Gf;
-    } else if (back) { Gf = 0; Gb = G; }
+    } else if (back) {
+        Gf = 0;
+    }
     FramePtrs f = front ? *front : *back, b = back ? *back : *front;
     set_segments(h, f, Gf > 0 ? Gf : G);
-    (void)Gb;
-    cudaError_t e = launch_coop(v.kernel, (unsigned)G, h->frame_smem, h->stream, f, b, Gf);
-    h->launches++;
-    if (e != cudaSuccess) { h->last_error = std::string(v.name) + ": " + cudaGetErrorString(e); return MOR_ERR_CUDA; }
-    return MOR_OK;
+    return launched(h, launch_coop(v.kernel, (unsigned)G, h->frame_smem, h->stream, f, b, Gf), v.name);
 }
 // The back half of the last filtered frame, if it is still waiting for a partner: alone.
 int flush_back(mor_handle* h) {
@@ -589,9 +595,8 @@ int enqueue_push(mor_handle* h, const uint8_t* d_points, uint32_t n, uint32_t st
         h->back_rec = h->frame_rec;
         h->back_pending = true;
     } else {
-        cudaError_t e = launch_coop(large_k(h) ? k_frame<true> : k_frame<false>, (unsigned)h->frame_ctas, h->frame_smem, st, a);
-        h->launches++;
-        if (e != cudaSuccess) { h->last_error = std::string("k_frame: ") + cudaGetErrorString(e); return MOR_ERR_CUDA; }
+        if (int ls = launched(h, launch_coop(large_k(h) ? k_frame<true> : k_frame<false>, (unsigned)h->frame_ctas, h->frame_smem, st, a), "k_frame"))
+            return ls;
         if (h->frame_rec) return launch_gather(h, a);
     }
     return MOR_OK;
@@ -604,22 +609,16 @@ int enqueue_push(mor_handle* h, const uint8_t* d_points, uint32_t n, uint32_t st
 int enqueue_ground_batch(mor_handle* h, const FramePtrs* P, const GroundPtrs* GP, uint32_t S, uint32_t n_max) {
     cudaStream_t st = h->stream;
     const dim3 pts(blocks_for(n_max), S), strided(((unsigned)h->num_sms * 8 + S - 1) / S, S), single(1, S);
-#define MOR_GLAUNCH(kernel, grid, block)                                                                                \
-    do {                                                                                                               \
-        cudaError_t le__ = launch_pdl(kernel, grid, dim3(block), 0, st, P, GP);                                        \
-        if (le__ != cudaSuccess) { h->last_error = std::string(#kernel) + ": " + cudaGetErrorString(le__); return MOR_ERR_CUDA; } \
-        h->launches++;                                                                                                 \
-    } while (0)
-    MOR_GLAUNCH(k_ingest_raw_batch, pts, kBlock);
-    MOR_GLAUNCH(k_ground_keys_batch, pts, kBlock);
-    MOR_GLAUNCH(k_scan_cells_batch, strided, kBlock);
-    MOR_GLAUNCH(k_scan_voxels_batch, strided, kBlock);
-    MOR_GLAUNCH(k_ground_scatter_batch, pts, kBlock);
-    MOR_GLAUNCH(k_voxel_eval_batch, strided, kBlock);
-    MOR_GLAUNCH(k_ground_mode_batch, single, kSingle);
-    MOR_GLAUNCH(k_ground_mark_batch, strided, kBlock);
-    MOR_GLAUNCH(k_ground_partition_batch, pts, kBlock);
-#undef MOR_GLAUNCH
+    // (the handles of a batched step never profile: these are all launch_pdl)
+    MOR_KLAUNCH(KID_G_INGEST, k_ingest_raw_batch, pts, kBlock, 0, P, GP);
+    MOR_KLAUNCH(KID_G_KEYS, k_ground_keys_batch, pts, kBlock, 0, P, GP);
+    MOR_KLAUNCH(KID_G_SCAN_CELLS, k_scan_cells_batch, strided, kBlock, 0, P, GP);
+    MOR_KLAUNCH(KID_G_SCAN_VOX, k_scan_voxels_batch, strided, kBlock, 0, P, GP);
+    MOR_KLAUNCH(KID_G_SCATTER, k_ground_scatter_batch, pts, kBlock, 0, P, GP);
+    MOR_KLAUNCH(KID_G_EVAL, k_voxel_eval_batch, strided, kBlock, 0, P, GP);
+    MOR_KLAUNCH(KID_G_MODE, k_ground_mode_batch, single, kSingle, 0, P, GP);
+    MOR_KLAUNCH(KID_G_MARK, k_ground_mark_batch, strided, kBlock, 0, P, GP);
+    MOR_KLAUNCH(KID_G_PARTITION, k_ground_partition_batch, pts, kBlock, 0, P, GP);
     return MOR_OK;
 }
 
@@ -636,6 +635,21 @@ void advance_frame(mor_handle* h, uint32_t n, const double pose7[7]) {
     h->frame_rec = h->out_records; h->rec_out = nullptr;
 }
 
+// The first filterCloud on a frame (see do_filter): its tracking update is committed, the mo_vec double buffer flips.
+void commit_frame(mor_handle* h) {
+    h->mo_parity ^= 1;
+    h->frame.mo_parity = h->mo_parity;
+    h->filtered = true;
+}
+
+// A device-side capacity was exceeded (the counts' error bits): the frame's results are not reference-exact.
+int device_capacity_error(mor_handle* h, int flags) {
+    char msg[200];
+    std::snprintf(msg, sizeof msg, "device capacity exceeded (error bits 0x%x: 1=clusters 2=moving 4=lattice range 8=ground grid 16=coordinate beyond the grid's range 32=cell pairs)", flags);
+    h->last_error = msg;
+    return MOR_ERR_CAPACITY;
+}
+
 // Work of a handle may have been enqueued on another handle's stream by mor_batch_step_device.
 int join_foreign_stream(mor_handle* h, bool keep_pending_back = false) {
     if (!keep_pending_back) { int fs = flush_back(h); if (fs != MOR_OK) return fs; }
@@ -648,10 +662,8 @@ int join_foreign_stream(mor_handle* h, bool keep_pending_back = false) {
 
 int do_push(mor_handle* h, const void* data, bool on_device, uint32_t n, uint32_t step, uint32_t ox, uint32_t oy, uint32_t oz, uint32_t oi, const double pose7[7]) {
     if (!h || (!data && n) || !pose7) return MOR_ERR_ARG;
-    if (validate_layout(step, ox, oy, oz, oi) != MOR_OK) { h->last_error = "point_step / field offsets do not describe a record with float32 x, y, z"; return MOR_ERR_ARG; }
-    if (n > h->nmax) { h->last_error = "frame larger than mor_limits.max_points"; return MOR_ERR_CAPACITY; }
+    if (int cs = check_frame(h, h, n, step, ox, oy, oz, oi, /*staged=*/!on_device)) return cs;
     if (h->inflight) { h->last_error = "submitted frames are in flight: collect them first"; return MOR_ERR_STATE; }
-    if (h->out_records && (size_t)n * step > h->d_in_bytes) { h->last_error = "output records: n * point_step exceeds the output buffer (32 B x max_points)"; return MOR_ERR_CAPACITY; }
     h->out_cur = h->slot[0].d_out;
     MOR_CUDA(cudaSetDevice(h->device));
     { int js = join_foreign_stream(h, on_device && h->pipelining && !h->profiling); if (js != MOR_OK) return js; }
@@ -660,7 +672,6 @@ int do_push(mor_handle* h, const void* data, bool on_device, uint32_t n, uint32_
     const uint8_t* d_points = (const uint8_t*)data;
     if (!on_device) {
         const size_t bytes = (size_t)n * step;
-        if (bytes > h->d_in_bytes) { h->last_error = "n * point_step exceeds the staging buffer (32 B/point)"; return MOR_ERR_CAPACITY; }
         if (bytes) MOR_CUDA(cudaMemcpyAsync(h->d_in, data, bytes, cudaMemcpyHostToDevice, h->stream));
         d_points = h->d_in;
     }
@@ -698,8 +709,7 @@ int do_filter(mor_handle* h, void* out, bool on_device, uint32_t cap_points, uin
         }
         (large_k(h) ? k_filter_again<true> : k_filter_again<false>)<<<h->n_input ? (h->n_input + kOutTile - 1) / kOutTile : 1, kT, 0, st>>>(a);
         prof_end(h);
-        h->launches++;
-        MOR_CUDA(cudaGetLastError());
+        if (int ls = launched(h, cudaGetLastError(), "k_filter_again")) return ls;
         if (h->frame_rec) {  // (after a batched step this gathers into the handle's own buffer, no longer into d_out[s])
             h->rec_out = nullptr;
             int gs = launch_gather(h, a);
@@ -712,7 +722,7 @@ int do_filter(mor_handle* h, void* out, bool on_device, uint32_t cap_points, uin
     const void* src = h->rec_out ? h->rec_out : a.out;
     if (on_device && !n_out && !h->profiling) {  // fully asynchronous device-resident mode
         if (out && h->n_input) MOR_CUDA(cudaMemcpyAsync(out, src, (size_t)h->n_input * rb, cudaMemcpyDeviceToDevice, st));
-        h->mo_parity ^= 1; a.mo_parity = h->mo_parity; h->filtered = true;
+        commit_frame(h);
         return MOR_OK;
     }
     MOR_CUDA(cudaMemcpyAsync(h->h_counts, a.counts, sizeof(int32_t) * MOR_NCOUNTS, cudaMemcpyDeviceToHost, st));
@@ -731,20 +741,14 @@ int do_filter(mor_handle* h, void* out, bool on_device, uint32_t cap_points, uin
     const uint32_t no = (uint32_t)h->h_counts[CNT_SPEC_NOUT];
     if (n_out) *n_out = no;
     h->spec_out = no;
-    if (h->h_counts[MOR_CNT_ERRFLAGS]) {  // a device-side capacity was exceeded: the frame's results are not reference-exact
-        char msg[200];
-        std::snprintf(msg, sizeof msg, "device capacity exceeded (error bits 0x%x: 1=clusters 2=moving 4=lattice range 8=ground grid 16=coordinate beyond the grid's range 32=cell pairs)",
-                      h->h_counts[MOR_CNT_ERRFLAGS]);
-        h->last_error = msg;
-        return MOR_ERR_CAPACITY;
-    }
+    if (h->h_counts[MOR_CNT_ERRFLAGS]) return device_capacity_error(h, h->h_counts[MOR_CNT_ERRFLAGS]);
     if (no > cap_points && out) return MOR_ERR_CAPACITY;  // not committed: the call can be repeated with a larger buffer
     if (!on_device && out && no > spec) {
         MOR_CUDA(cudaMemcpyAsync((uint8_t*)out + (size_t)spec * rb, (const uint8_t*)src + (size_t)spec * rb, (size_t)(no - spec) * rb, cudaMemcpyDeviceToHost, st));
         MOR_CUDA(cudaStreamSynchronize(st));
     }
     if (on_device && out && no) MOR_CUDA(cudaMemcpyAsync(out, src, (size_t)no * rb, cudaMemcpyDeviceToDevice, st));
-    h->mo_parity ^= 1; a.mo_parity = h->mo_parity; h->filtered = true;  // commit
+    commit_frame(h);
     return MOR_OK;
 }
 
@@ -819,6 +823,39 @@ void plan_mixed_groups(const std::vector<uint32_t>& n, int C, std::vector<int4>&
         groups.push_back(make_int4(g, 1, (int)order.size(), (int)(order.size() + members[g].size())));
         order.insert(order.end(), members[g].begin(), members[g].end());
     }
+}
+
+// The index of the second appearance of a handle in hs[0 .. S), or -1.
+int64_t repeated_handle(mor_handle* const* hs, uint32_t S) {
+    std::vector<std::pair<const mor_handle*, uint32_t>> seen(S);
+    for (uint32_t s = 0; s < S; s++) seen[s] = {hs[s], s};
+    std::sort(seen.begin(), seen.end());
+    for (uint32_t s = 1; s < S; s++)
+        if (seen[s].first == seen[s - 1].first) return seen[s].second;
+    return -1;
+}
+
+// The part of a batched step that is the same for every sequence: handle g takes the frame f, which a group of G CTAs
+// runs on the leader h's stream. Its output goes to f.d_out: the filtered cloud, or with output records the gather's
+// copies of the input records (*rec, the gather's arguments).
+int prepare_batched_frame(mor_handle* h, mor_handle* g, const mor_batch_frame& f, int G, RecordPtrs* rec) {
+    cudaStream_t st = h->stream;
+    if (g->last_stream != st) {  // earlier work of this handle ran elsewhere (its own stream or another batch): wait for it once
+        if (g->last_stream) MOR_CUDA(cudaStreamSynchronize(g->last_stream));
+        if (g->stream != st) MOR_CUDA(cudaStreamSynchronize(g->stream));
+    }
+    advance_frame(g, f.n, f.pose7);
+    g->out_cur = g->slot[0].d_out;
+    fill_frame(g, (const uint8_t*)f.d_data, f.n, f.point_step, f.off_x, f.off_y, f.off_z, f.off_i);
+    if (g->frame_rec) {  // the frame kernel's PointXYZI records go to the handle's own buffer, the gather alone writes d_out
+        *rec = record_ptrs(g, g->frame, f.d_out);
+        g->rec_out = f.d_out;
+    } else {
+        g->frame.out = (float4*)f.d_out;
+    }
+    set_segments(g, g->frame, G);
+    g->last_stream = st;
+    return MOR_OK;
 }
 
 }  // namespace
@@ -940,32 +977,27 @@ int mor_batch_step_device(mor_handle* const* hs, uint32_t S, const void* const* 
                           uint32_t off_y, uint32_t off_z, uint32_t off_i, const double* poses7, void* const* d_out) {
     if (!hs || !S || !d_data || !n || !poses7 || !d_out || !hs[0]) return MOR_ERR_ARG;
     mor_handle* h = hs[0];  // leader: owns the stream and the argument array of the batch
-    if (validate_layout(point_step, off_x, off_y, off_z, off_i) != MOR_OK) return MOR_ERR_ARG;
+    const bool rec = h->out_records;
+    // every rule is checked before anything is enqueued or changed: a refused step leaves every handle as it was
     for (uint32_t s = 0; s < S; s++) {
-        mor_handle* g = hs[s];
+        const mor_handle* g = hs[s];
         // same device, limits, frame count and configuration (every key that reaches the kernels)
         if (!g || g->device != h->device || g->nmax != h->nmax || g->kmax != h->kmax || g->momax != h->momax || g->have_prev != h->have_prev ||
             g->have_cur != h->have_cur || g->profiling || g->inflight || std::memcmp(&g->cfg, &h->cfg, offsetof(mor_config, output_topic)) != 0) {
             h->last_error = "batched handles must share device, limits, config and frame count";
             return MOR_ERR_ARG;
         }
-        { int fs = flush_back(g); if (fs != MOR_OK) return fs; }
-        if (n[s] > g->nmax || (!d_data[s] && n[s]) || !d_out[s]) return n[s] > g->nmax ? MOR_ERR_CAPACITY : MOR_ERR_ARG;
-        for (uint32_t t = 0; t < s; t++) if (hs[t] == g) return MOR_ERR_ARG;
+        if (g->out_records != rec) { h->last_error = "batched handles must agree on mor_set_output_records"; return MOR_ERR_ARG; }
+        if ((!d_data[s] && n[s]) || !d_out[s]) { h->last_error = "null d_data or d_out"; return MOR_ERR_ARG; }
+        if (int cs = check_frame(h, g, n[s], point_step, off_x, off_y, off_z, off_i, /*staged=*/false)) return cs;
     }
+    if (repeated_handle(hs, S) >= 0) { h->last_error = "a handle appears twice in the batch"; return MOR_ERR_ARG; }
     const bool ground = h->cfg.ground_mode != MOR_GROUND_CROP;  // (shared by every handle: part of the config compared above)
-    const bool rec = h->out_records;
     if (rec && S > 65535u) { h->last_error = "output records: at most 65535 sequences per batched step"; return MOR_ERR_ARG; }
-    for (uint32_t s = 0; s < S; s++) {
-        if (hs[s]->out_records != rec) { h->last_error = "batched handles must agree on mor_set_output_records"; return MOR_ERR_ARG; }
-        if (rec && (size_t)n[s] * point_step > hs[s]->d_in_bytes) {
-            h->last_error = "output records: n * point_step exceeds the output buffer (32 B x max_points)";
-            return MOR_ERR_CAPACITY;
-        }
-    }
     if (ground && S > 65535u) { h->last_error = "the voxel ground modes batch at most 65535 sequences per step"; return MOR_ERR_ARG; }
     MOR_CUDA(cudaSetDevice(h->device));
     cudaStream_t st = h->stream;
+    for (uint32_t s = 0; s < S; s++) { int fs = flush_back(hs[s]); if (fs != MOR_OK) return fs; }
     static_assert(sizeof(FramePtrs) % alignof(GroundPtrs) == 0, "GroundPtrs follow the FramePtrs of a ring slot");
     static_assert((sizeof(FramePtrs) + sizeof(GroundPtrs)) % alignof(RecordPtrs) == 0, "RecordPtrs follow the GroundPtrs of a ring slot");
     const size_t per_seq = sizeof(FramePtrs) + sizeof(GroundPtrs) + sizeof(RecordPtrs);
@@ -987,23 +1019,11 @@ int mor_batch_step_device(mor_handle* const* hs, uint32_t S, const void* const* 
     if (groups > (int)S) groups = (int)S;
     for (uint32_t s = 0; s < S; s++) {
         mor_handle* g = hs[s];
-        if (g->last_stream != st) {  // earlier work of this handle ran elsewhere (its own stream or another batch): wait for it once
-            if (g->last_stream) MOR_CUDA(cudaStreamSynchronize(g->last_stream));
-            if (g->stream != st) MOR_CUDA(cudaStreamSynchronize(g->stream));
-        }
-        advance_frame(g, n[s], poses7 + 7 * s);
-        g->out_cur = g->slot[0].d_out;
-        fill_frame(g, (const uint8_t*)d_data[s], n[s], point_step, off_x, off_y, off_z, off_i);
-        if (rec) {  // the frame kernel's PointXYZI records go to the handle's own buffer, the gather alone writes d_out[s]
-            hr[s] = record_ptrs(g, g->frame, d_out[s]);
-            g->rec_out = d_out[s];
-        } else {
-            g->frame.out = (float4*)d_out[s];
-        }
-        set_segments(g, g->frame, G);
+        mor_batch_frame f{d_data[s], n[s], point_step, off_x, off_y, off_z, off_i, {}, d_out[s]};
+        std::memcpy(f.pose7, poses7 + 7 * s, sizeof f.pose7);
+        if (int ps = prepare_batched_frame(h, g, f, G, hr + s)) return ps;
         hp[s] = g->frame;
         if (ground) { hg[s] = g->ground; n_max = n[s] > n_max ? n[s] : n_max; }
-        g->last_stream = st;
     }
     MOR_CUDA(cudaMemcpyAsync(dp, hp, (rec ? per_seq : ground ? sizeof(FramePtrs) + sizeof(GroundPtrs) : sizeof(FramePtrs)) * S, cudaMemcpyHostToDevice, st));
     MOR_CUDA(cudaEventRecord(h->batch_ev[slot], st));
@@ -1011,24 +1031,16 @@ int mor_batch_step_device(mor_handle* const* hs, uint32_t S, const void* const* 
         int gs = enqueue_ground_batch(h, dp, dg, S, n_max);
         if (gs != MOR_OK) return gs;
     }
-    {
-        cudaError_t e = launch_coop(large_k(h) ? k_frame_batch<true> : k_frame_batch<false>, (unsigned)(groups * G), h->frame_smem, st, (const FramePtrs*)dp, (int)S, G);
-        h->launches++;
-        if (e != cudaSuccess) { h->last_error = std::string("k_frame_batch: ") + cudaGetErrorString(e); return MOR_ERR_CUDA; }
-    }
+    if (int ls = launched(h, launch_coop(large_k(h) ? k_frame_batch<true> : k_frame_batch<false>, (unsigned)(groups * G), h->frame_smem, st, (const FramePtrs*)dp, (int)S, G),
+                          "k_frame_batch"))
+        return ls;
     if (rec) {  // one gather launch for all S sequences
         uint32_t nm = 0;
         for (uint32_t s = 0; s < S; s++) nm = n[s] > nm ? n[s] : nm;
         k_gather_records_batch<<<dim3(rec_blocks(nm), S), kRecT, 0, st>>>(reinterpret_cast<const RecordPtrs*>(reinterpret_cast<const GroundPtrs*>(dp + S) + S));
-        h->launches++;
-        const cudaError_t e = cudaGetLastError();
-        if (e != cudaSuccess) { h->last_error = std::string("k_gather_records_batch: ") + cudaGetErrorString(e); return MOR_ERR_CUDA; }
+        if (int ls = launched(h, cudaGetLastError(), "k_gather_records_batch")) return ls;
     }
-    for (uint32_t s = 0; s < S; s++) {  // push + filter in one call: the frame is committed
-        hs[s]->mo_parity ^= 1;
-        hs[s]->frame.mo_parity = hs[s]->mo_parity;
-        hs[s]->filtered = true;
-    }
+    for (uint32_t s = 0; s < S; s++) commit_frame(hs[s]);  // push + filter in one call
     return MOR_OK;
 }
 
@@ -1039,10 +1051,8 @@ int mor_batch_step_device(mor_handle* const* hs, uint32_t S, const void* const* 
 int mor_batch_step_device_mixed(mor_handle* const* hs, uint32_t S, const mor_batch_frame* frames) {
     if (!hs || !S || !frames || !hs[0]) return MOR_ERR_ARG;
     mor_handle* h = hs[0];  // leader: owns the stream and the argument ring of the batch
-    auto fail = [&](int status, uint32_t s, const char* rule) {
-        char msg[200];
-        std::snprintf(msg, sizeof msg, "mixed batched step, sequence %u: %s", s, rule);
-        h->last_error = msg;
+    auto fail = [&](int status, uint32_t s, const std::string& rule) {
+        h->last_error = "mixed batched step, sequence " + std::to_string(s) + ": " + rule;
         return status;
     };
     // every rule is checked before anything is enqueued or changed: a refused step leaves every handle as it was
@@ -1056,24 +1066,14 @@ int mor_batch_step_device_mixed(mor_handle* const* hs, uint32_t S, const mor_bat
         if (g->device != h->device) return fail(MOR_ERR_ARG, s, "all handles must be on one device");
         if (g->inflight) return fail(MOR_ERR_ARG, s, "the handle has submitted frames in flight: collect them first");
         if (g->profiling) return fail(MOR_ERR_ARG, s, "the handle has kernel profiling on");
-        if (validate_layout(f.point_step, f.off_x, f.off_y, f.off_z, f.off_i) != MOR_OK)
-            return fail(MOR_ERR_ARG, s, "point_step / field offsets do not describe a record with float32 x, y, z");
         if ((!f.d_data && f.n) || !f.d_out) return fail(MOR_ERR_ARG, s, "null d_data or d_out");
-        if (f.n > g->nmax) return fail(MOR_ERR_CAPACITY, s, "frame larger than mor_limits.max_points");
-        if (g->out_records && (size_t)f.n * f.point_step > g->d_in_bytes)
-            return fail(MOR_ERR_CAPACITY, s, "output records: n * point_step exceeds the output buffer (32 B x max_points)");
+        if (int cs = check_frame(h, g, f.n, f.point_step, f.off_x, f.off_y, f.off_z, f.off_i, /*staged=*/false)) return fail(cs, s, h->last_error);
         n_ground += g->cfg.ground_mode != MOR_GROUND_CROP;
         n_rec += g->out_records;
         lk = lk || large_k(g);
         smem = g->frame_smem > smem ? g->frame_smem : smem;
     }
-    {
-        std::vector<std::pair<const mor_handle*, uint32_t>> seen(S);
-        for (uint32_t s = 0; s < S; s++) seen[s] = {hs[s], s};
-        std::sort(seen.begin(), seen.end());
-        for (uint32_t s = 1; s < S; s++)
-            if (seen[s].first == seen[s - 1].first) return fail(MOR_ERR_ARG, seen[s].second, "the handle appears twice in the batch");
-    }
+    if (const int64_t s = repeated_handle(hs, S); s >= 0) return fail(MOR_ERR_ARG, (uint32_t)s, "the handle appears twice in the batch");
     if (n_ground > 65535u || n_rec > 65535u) { h->last_error = "mixed batched step: at most 65535 sequences with a voxel ground mode and 65535 with output records"; return MOR_ERR_ARG; }
     MOR_CUDA(cudaSetDevice(h->device));
     cudaStream_t st = h->stream;
@@ -1106,28 +1106,16 @@ int mor_batch_step_device_mixed(mor_handle* const* hs, uint32_t S, const mor_bat
     for (uint32_t s = 0; s < S; s++) {
         mor_handle* g = hs[s];
         const mor_batch_frame& f = frames[s];
-        if (g->last_stream != st) {  // earlier work of this handle ran elsewhere (its own stream or another batch): wait for it once
-            if (g->last_stream) MOR_CUDA(cudaStreamSynchronize(g->last_stream));
-            if (g->stream != st) MOR_CUDA(cudaStreamSynchronize(g->stream));
-        }
-        advance_frame(g, f.n, f.pose7);
-        g->out_cur = g->slot[0].d_out;
-        fill_frame(g, (const uint8_t*)f.d_data, f.n, f.point_step, f.off_x, f.off_y, f.off_z, f.off_i);
-        if (g->frame_rec) {  // the frame kernel's PointXYZI records go to the handle's own buffer, the gather alone writes d_out
-            hr[ir] = record_ptrs(g, g->frame, f.d_out);
+        if (int ps = prepare_batched_frame(h, g, f, G_of[s], hr + ir)) return ps;
+        hp[s] = g->frame;
+        if (g->frame_rec) {
             hrn[ir++] = (int)rec_blocks(f.n);
             n_max_r = f.n > n_max_r ? f.n : n_max_r;
-            g->rec_out = f.d_out;
-        } else {
-            g->frame.out = (float4*)f.d_out;
         }
-        set_segments(g, g->frame, G_of[s]);
-        hp[s] = g->frame;
         if (g->cfg.ground_mode != MOR_GROUND_CROP) {
             hpg[ig] = g->frame; hgg[ig++] = g->ground;
             n_max_g = f.n > n_max_g ? f.n : n_max_g;
         }
-        g->last_stream = st;
     }
     MOR_CUDA(cudaMemcpyAsync(db, hb, bytes, cudaMemcpyHostToDevice, st));
     MOR_CUDA(cudaEventRecord(h->batch_ev[slot], st));
@@ -1135,22 +1123,12 @@ int mor_batch_step_device_mixed(mor_handle* const* hs, uint32_t S, const mor_bat
         int gs = enqueue_ground_batch(h, reinterpret_cast<const FramePtrs*>(db + off_pg), reinterpret_cast<const GroundPtrs*>(db + off_gg), n_ground, n_max_g);
         if (gs != MOR_OK) return gs;
     }
-    {
-        const unsigned grid = (unsigned)(groups.back().x + groups.back().y);
-        cudaError_t e = launch_frame_batch_mixed(lk, grid, smem, st, db, db + off_t, (int)groups.size());
-        h->launches++;
-        if (e != cudaSuccess) { h->last_error = std::string("k_frame_batch_mixed: ") + cudaGetErrorString(e); return MOR_ERR_CUDA; }
-    }
+    const unsigned grid = (unsigned)(groups.back().x + groups.back().y);
+    if (int ls = launched(h, launch_frame_batch_mixed(lk, grid, smem, st, db, db + off_t, (int)groups.size()), "k_frame_batch_mixed")) return ls;
     if (n_rec) {  // one gather launch for the sequences with output records
-        const cudaError_t e = launch_gather_records_mixed(rec_blocks(n_max_r), n_rec, st, db + off_r, db + off_rn);
-        h->launches++;
-        if (e != cudaSuccess) { h->last_error = std::string("k_gather_records_mixed: ") + cudaGetErrorString(e); return MOR_ERR_CUDA; }
+        if (int ls = launched(h, launch_gather_records_mixed(rec_blocks(n_max_r), n_rec, st, db + off_r, db + off_rn), "k_gather_records_mixed")) return ls;
     }
-    for (uint32_t s = 0; s < S; s++) {  // push + filter in one call: the frame is committed
-        hs[s]->mo_parity ^= 1;
-        hs[s]->frame.mo_parity = hs[s]->mo_parity;
-        hs[s]->filtered = true;
-    }
+    for (uint32_t s = 0; s < S; s++) commit_frame(hs[s]);  // push + filter in one call
     return MOR_OK;
 }
 
@@ -1206,10 +1184,7 @@ static int enqueue_slot_d2h(mor_handle* h, mor_handle::StreamSlot& sl) {
 int mor_submit_frame(mor_handle* h, const void* data, uint32_t n, uint32_t step, uint32_t ox, uint32_t oy, uint32_t oz, uint32_t oi,
                      const double pose7[7], void* out, uint32_t cap_points) {
     if (!h || (!data && n) || !pose7 || (!out && cap_points)) return MOR_ERR_ARG;
-    if (validate_layout(step, ox, oy, oz, oi) != MOR_OK) { h->last_error = "point_step / field offsets do not describe a record with float32 x, y, z"; return MOR_ERR_ARG; }
-    if (n > h->nmax) { h->last_error = "frame larger than mor_limits.max_points"; return MOR_ERR_CAPACITY; }
-    const size_t bytes = (size_t)n * step;
-    if (bytes > h->d_in_bytes) { h->last_error = "n * point_step exceeds the staging buffer (32 B/point)"; return MOR_ERR_CAPACITY; }
+    if (int cs = check_frame(h, h, n, step, ox, oy, oz, oi, /*staged=*/true)) return cs;
     if (h->profiling) { h->last_error = "per-phase profiling serialises every frame: not available while streaming"; return MOR_ERR_STATE; }
     if (h->inflight >= MOR_STREAM_DEPTH) { h->last_error = "MOR_STREAM_DEPTH frames are in flight: collect one first"; return MOR_ERR_STATE; }
     MOR_CUDA(cudaSetDevice(h->device));
@@ -1225,7 +1200,7 @@ int mor_submit_frame(mor_handle* h, const void* data, uint32_t n, uint32_t step,
         MOR_CUDA(cudaEventRecord(h->ev_join, h->stream));
         MOR_CUDA(cudaStreamWaitEvent(h->copy_in, h->ev_join, 0));
     }
-    if (bytes) MOR_CUDA(cudaMemcpyAsync(sl.d_in, data, bytes, cudaMemcpyHostToDevice, h->copy_in));
+    if (n) MOR_CUDA(cudaMemcpyAsync(sl.d_in, data, (size_t)n * step, cudaMemcpyHostToDevice, h->copy_in));
     MOR_CUDA(cudaEventRecord(sl.h2d, h->copy_in));
     MOR_CUDA(cudaStreamWaitEvent(h->stream, sl.h2d, 0));
     advance_frame(h, n, pose7);
@@ -1245,7 +1220,7 @@ int mor_submit_frame(mor_handle* h, const void* data, uint32_t n, uint32_t step,
         int es = enqueue_slot_d2h(h, sl);
         if (es != MOR_OK) return es;
     }
-    h->mo_parity ^= 1; h->frame.mo_parity = h->mo_parity; h->filtered = true;  // committed like push + one filterCloud
+    commit_frame(h);  // like push + one filterCloud
     h->inflight++;
     return MOR_OK;
 }
@@ -1264,13 +1239,7 @@ int mor_collect_frame(mor_handle* h, uint32_t* n_out) {
     const uint32_t no = (uint32_t)sl.h_counts[CNT_SPEC_NOUT];
     if (n_out) *n_out = no;
     h->spec_out = no;
-    if (sl.h_counts[MOR_CNT_ERRFLAGS]) {
-        char msg[200];
-        std::snprintf(msg, sizeof msg, "device capacity exceeded (error bits 0x%x: 1=clusters 2=moving 4=lattice range 8=ground grid 16=coordinate beyond the grid's range 32=cell pairs)",
-                      sl.h_counts[MOR_CNT_ERRFLAGS]);
-        h->last_error = msg;
-        return MOR_ERR_CAPACITY;
-    }
+    if (sl.h_counts[MOR_CNT_ERRFLAGS]) return device_capacity_error(h, sl.h_counts[MOR_CNT_ERRFLAGS]);
     if (no > sl.cap) { h->last_error = "output buffer of the submitted frame too small"; return MOR_ERR_CAPACITY; }
     if (no > sl.spec) {  // (the slot's device buffer is not rewritten before the frame after next is submitted)
         const size_t rb = sl.rec_bytes;

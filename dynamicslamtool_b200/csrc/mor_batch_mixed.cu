@@ -22,7 +22,7 @@ namespace mor_mixed_tu {
 template <bool LK>
 __global__ void __launch_bounds__(kT, 1) k_frame_batch_mixed(const FramePtrs* __restrict__ P, const int4* __restrict__ T, int groups) {
     extern __shared__ __align__(128) unsigned long long dyn[];
-    __shared__ FrameShared sh;
+    __shared__ FilterShared sh;
     int lo = 0, hi = groups - 1;  // the last group whose first CTA is at or below this one
     while (lo < hi) {
         const int mid = (lo + hi + 1) >> 1;
@@ -30,10 +30,7 @@ __global__ void __launch_bounds__(kT, 1) k_frame_batch_mixed(const FramePtrs* __
     }
     const int4 grp = T[lo];
     const int* order = reinterpret_cast<const int*>(T + groups);
-    if (threadIdx.x == 0) mbar_init(&sh.mbar, 1);
-    __syncthreads();
-    unsigned parity = 0;
-    for (int i = grp.z; i < grp.w; i++) frame_body<LK>(P[order[i]], (int)blockIdx.x - grp.x, grp.y, sh, dyn, parity);
+    for (int i = grp.z; i < grp.w; i++) frame_body<LK>(P[order[i]], (int)blockIdx.x - grp.x, grp.y, sh, dyn);
 }
 
 // gather_records (mor_records.cuh) for a batch whose handles' limits differ: a sequence's tile states are sized for its own

@@ -67,7 +67,6 @@ struct Scratch {  // all zero between frames: every counter is put back by the f
     int n_cells, n_roots, n_light, n_heavy;  // list lengths of the frame
     int n_sorted, pad1;      // bump allocator of the sorted array (phase B)
     unsigned tail_match, tail_chain;  // arrival counters of the phases that end with a single-CTA step
-    int ticket_light, ticket_heavy;   // next unclaimed record of the pair lists (test phase)
     int ticket_out, out_blocks_done;  // stand-alone filter kernel (repeated filterCloud on one frame)
     int err_early;           // error bits raised before the frame's counts exist
     int n_sel;               // size-valid clusters found by the group-wide select (phase_select_large)
@@ -217,28 +216,6 @@ __device__ __forceinline__ bool group_last_arrival(unsigned* ctr, unsigned G) {
     return s_last_in != 0;
 }
 
-// ------------------------------------------------------------------------------------------------ 1-D bulk copy (TMA)
-__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, unsigned count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void bulk_load(void* dst_smem, const void* src_gmem, unsigned bytes, unsigned long long* bar) {
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // earlier generic-proxy reads of dst are done (WAR across proxies)
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(smem_u32(dst_smem)), "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long* bar, unsigned parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAIT_%=:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@!p bra WAIT_%=;\n"
-        "}\n" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-
 // ------------------------------------------------------------------------------------------------ clustering grid
 constexpr int kCellBias = 1 << 20;  // cell coordinates are stored biased, 21 bits per axis
 __device__ __forceinline__ unsigned long long cell_pack(int cx, int cy, int cz) {
@@ -381,52 +358,22 @@ __device__ __forceinline__ unsigned long long bin_point(const FramePtrs& a, cons
     return cell_pack(cx, cy, cz);
 }
 
-// A float field of a record staged in shared memory (any alignment).
-__device__ __forceinline__ float smem_f32(const uint8_t* p) {
-    if ((smem_u32(p) & 3u) == 0u) return *reinterpret_cast<const float*>(p);
-    return __uint_as_float((unsigned)p[0] | ((unsigned)p[1] << 8) | ((unsigned)p[2] << 16) | ((unsigned)p[3] << 24));
-}
-
-__device__ __forceinline__ void phase_ingest(const FramePtrs& a, int cta, int G, unsigned long long* dyn, unsigned long long* mbar, unsigned& parity, bool housekeep = true) {
+__device__ __forceinline__ void phase_ingest(const FramePtrs& a, int cta, int G, bool housekeep = true) {
     if (housekeep) frame_housekeeping(a, cta, G);
     const int ntiles = a.n ? (int)((a.n + kIngestTile - 1) / kIngestTile) : 1;
     __shared__ int s_created, s_cbase;
-    // Records that are not plain float4 (PCLPointCloud2 layouts with padding or extra fields, e.g. the 22-byte velodyne
-    // XYZIRT record) can be staged: the tile's bytes come into shared memory by ONE bulk copy (TMA, 1-D) and the fields
-    // are picked out there - instead of four strided word loads, or sixteen byte loads, per point from global memory.
-    // Measured on C2 (profiles/README.md): the phase is a latency chain, not load-bound - 13.0 us staged vs 12.4 us direct
-    // for 22-byte records, 13.3 vs 12.1 us for 32-byte records (the copy's round trip and two CTA barriers sit in front
-    // of everything else). Off unless built with -DMOR_INGEST_STAGE.
-#ifdef MOR_INGEST_STAGE
-    const bool staged = a.in_mode != 0 && (size_t)kIngestTile * a.step + 32 <= (size_t)a.frame_smem && (reinterpret_cast<uintptr_t>(a.in) & 15) == 0;
-#else
-    const bool staged = false;
-#endif
-    uint8_t* const stage = reinterpret_cast<uint8_t*>(dyn);
+    // Records that are not plain float4 are read field by field from global memory. The phase is a latency chain, not
+    // load-bound: staging the tile in shared memory by one bulk copy was measured slower (profiles/README.md).
     for (int tile = cta; tile < ntiles; tile += G) {
         const uint32_t i = (uint32_t)tile * kIngestTile + threadIdx.x;
         float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
         int cls = 0;
         if (threadIdx.x == 0) s_created = 0;
-        __syncthreads();  // (also: the previous tile's readers of s_cbase and of the staged bytes are done)
-        size_t stage_skew = 0;
-        if (staged) {
-            const size_t b0 = (size_t)tile * kIngestTile * a.step, b1 = min((size_t)a.n * a.step, b0 + (size_t)kIngestTile * a.step);
-            const size_t c0 = b0 & ~(size_t)15, c1 = max(c0, b1 & ~(size_t)15);  // [c0, c1): 16-byte granules for the bulk copy; [c1, b1): the last bytes
-            stage_skew = b0 - c0;
-            if (threadIdx.x == 0 && c1 > c0) bulk_load(stage, a.in + c0, (unsigned)(c1 - c0), mbar);
-            if (threadIdx.x < b1 - c1) stage[c1 - c0 + threadIdx.x] = a.in[c1 + threadIdx.x];
-            if (c1 > c0) { mbar_wait(mbar, parity); parity ^= 1u; }
-            __syncthreads();
-        }
+        __syncthreads();  // (also: the previous tile's readers of s_cbase are done)
         if (i < a.n) {
             const uint8_t* p = a.in + (size_t)i * a.step;
             if (a.in_mode == 0) {
                 v = __ldg(reinterpret_cast<const float4*>(p));
-            } else if (staged) {
-                const uint8_t* q = stage + stage_skew + (size_t)threadIdx.x * a.step;
-                v.x = smem_f32(q + a.off_x); v.y = smem_f32(q + a.off_y); v.z = smem_f32(q + a.off_z);
-                v.w = a.off_i != 0xFFFFFFFFu ? smem_f32(q + a.off_i) : 0.f;
             } else {
                 v.x = load_f32(p + a.off_x, a.in_mode); v.y = load_f32(p + a.off_y, a.in_mode); v.z = load_f32(p + a.off_z, a.in_mode);
                 v.w = a.off_i != 0xFFFFFFFFu ? load_f32(p + a.off_i, a.in_mode) : 0.f;
@@ -702,13 +649,8 @@ __device__ __forceinline__ void phase_scatter(const FramePtrs& a, int cta, int G
 // samples first (a heavy pair is nearly always connected and nearly any sample shows it), bounding-box pruning and the
 // full scan only when the probe finds nothing. Connected pairs are RECORDED (edges, per-CTA segments) and the larger
 // node of a pair is pointed at the smaller one (atomicMin on its own word): the forest phase E starts from.
-// The frame kernel is 220-290 KB of code, more than an SM's instruction cache holds. Keeping the large once-per-frame
-// steps out of line (-DMOR_OUTLINE_BIG) was measured and is slower (8.6k vs 9.0k frames/s on C2): inlined by default.
-#ifdef MOR_OUTLINE_BIG
-#define MOR_OUTLINE __device__ __noinline__
-#else
-#define MOR_OUTLINE __device__ __forceinline__
-#endif
+// The frame kernel is 220-290 KB of code, more than an SM's instruction cache holds, yet keeping the large once-per-frame
+// steps out of line was measured slower (8.6k vs 9.0k frames/s on C2, profiles/README.md): they are inlined.
 #ifdef MOR_DEBUG_BOUNDS
 #define MOR_CHECK(cond, tag, v) do { if (!(cond)) { printf("BOUNDS %s: %d (line %d, cta %d thread %d)\n", tag, (int)(v), __LINE__, (int)blockIdx.x, (int)threadIdx.x); } } while (0)
 #else
@@ -717,7 +659,7 @@ __device__ __forceinline__ void phase_scatter(const FramePtrs& a, int cta, int G
 struct BoxF { float lx, ly, lz, hx, hy, hz; };
 // Tight bounding box of the n points from sorted position `start`, by the whole warp (only the few heavy pairs whose
 // probe found nothing need boxes, so they are made on demand).
-MOR_OUTLINE BoxF warp_box(const FramePtrs& a, int start, int n, int lane) {
+__device__ __forceinline__ BoxF warp_box(const FramePtrs& a, int start, int n, int lane) {
     unsigned mnx = 0xFFFFFFFFu, mny = 0xFFFFFFFFu, mnz = 0xFFFFFFFFu, mxx = 0u, mxy = 0u, mxz = 0u;
     for (int k = lane; k < n; k += 32) {
         const float4 p = a.spts[start + k];
@@ -761,7 +703,7 @@ __device__ __forceinline__ bool heavy_boxes_apart(const FramePtrs& a, int sA, in
 }
 // (3) Full scan of one chunk of 32 points of B (from b0) against all of A, both pruned by the other cell's box: A in
 // blocks of 32 per coalesced load, four blocks in flight, every candidate point broadcast by shuffle to all lanes.
-MOR_OUTLINE bool heavy_scan_chunk(const FramePtrs& a, const HeavyBoxes& hb, int sA, int cntA, int sB, int cB, int b0, int lane) {
+__device__ __forceinline__ bool heavy_scan_chunk(const FramePtrs& a, const HeavyBoxes& hb, int sA, int cntA, int sB, int cB, int b0, int lane) {
     const float r2 = a.r2, r2_prune = a.r2 * 1.00001f;
     const float4* A = a.spts + sA;
     const int b = b0 + lane;
@@ -1005,9 +947,9 @@ __device__ __forceinline__ void phase_test(const FramePtrs& a, int cta, int G) {
             }
         }
     };
-#ifndef MOR_TEST_TICKETS
     // Equal shares per CTA: the light pairs packed into the first warps (a warp issues the same instructions whether 12 or 32
     // of its lanes hold a pair: spreading them over all warps was 2x slower), the heavy pairs on the others, side by side.
+    // (Dealing both lists out by ticket evens out the CTAs but queues every chunk on one word: 22.9 vs 16.1 us.)
     const int lper = (TL + G - 1) / G, llo = min(TL, cta * lper), lhi = min(TL, llo + lper);
     const int hper = (TH + G - 1) / G, hlo = min(TH, cta * hper), hhi = min(TH, hlo + hper);
     const int light_warps = min(kWarps, (lhi - llo + 31) >> 5);
@@ -1017,31 +959,6 @@ __device__ __forceinline__ void phase_test(const FramePtrs& a, int cta, int G) {
     const int hwarp = kWarps - 1 - warp;
     if (hwarp < heavy_warps)
         for (int w = hlo + hwarp; w < hhi; w += 2 * heavy_warps) heavy_pairs(w, w + heavy_warps, w + heavy_warps < hhi);
-#else
-    // Measurement variant (-DMOR_TEST_TICKETS): both lists dealt out by ticket over the whole group, a chunk per warp and
-    // step (32 light pairs or 2 heavy pairs), half of the warps starting on either list. It evens out the CTAs but puts a
-    // round trip - and 4,700 warps queueing on two words - in front of every chunk: 22.9 vs 16.1 us for the phase.
-    auto run_light = [&]() {
-        while (true) {
-            int t = 0;
-            if (lane == 0) t = atomicAdd(&a.scratch->ticket_light, 32);
-            t = __shfl_sync(kFull, t, 0);
-            if (t >= TL) break;
-            light_chunk(t, TL);
-        }
-    };
-    auto run_heavy = [&]() {
-        while (true) {
-            int t = 0;
-            if (lane == 0) t = atomicAdd(&a.scratch->ticket_heavy, 2);
-            t = __shfl_sync(kFull, t, 0);
-            if (t >= TH) break;
-            heavy_pairs(t, t + 1, t + 1 < TH);
-        }
-    };
-    if (warp < kWarps / 2) { run_light(); MOR_TRACE_NOSYNC(17); run_heavy(); }
-    else { run_heavy(); run_light(); }
-#endif
     __syncthreads();
     MOR_TRACE(18);
     const int nhard = min(s_nhard, kHardCap);
@@ -1155,7 +1072,7 @@ __device__ __forceinline__ void bitonic_sort_smem(unsigned long long* keys, int 
     }
 }
 
-MOR_OUTLINE void phase_select(const FramePtrs& a, unsigned long long* keys) {
+__device__ __forceinline__ void phase_select(const FramePtrs& a, unsigned long long* keys) {
     __shared__ int s_k;
     const int n_roots = __ldcg(&a.scratch->n_roots);
     if (threadIdx.x == 0) s_k = 0;
@@ -1543,7 +1460,7 @@ __device__ __forceinline__ void phase_match_impl(const FramePtrs& a, unsigned lo
     }
 }
 
-MOR_OUTLINE void phase_match(const FramePtrs& a, unsigned long long* dyn) {
+__device__ __forceinline__ void phase_match(const FramePtrs& a, unsigned long long* dyn) {
     const int K = a.counts[MOR_CNT_K];
     const int Kp = a.two_frames ? a.p_counts[MOR_CNT_K] : 0;
     const int cap = (a.frame_smem - kSingle * 12) / kMatchBytesPerCluster;
@@ -1705,7 +1622,7 @@ __device__ __forceinline__ void phase_lattice_count(const FramePtrs& a, int cta,
 // count, so the search is bounded by sqrt(pde_ub) on the clustering grid. Shells of growing Chebyshev distance around
 // the query's cell: a point in shell r is at least (r-1)*h away, so the search stops as soon as that bound exceeds the
 // best distance (or pde_ub: farther neighbours never count), and a neighbour at d2 <= pde_lb settles the answer.
-MOR_OUTLINE void phase_pde_count(const FramePtrs& a, int cta, int G) {
+__device__ __forceinline__ void phase_pde_count(const FramePtrs& a, int cta, int G) {
     const int ncp = a.p_counts[MOR_CNT_NC];
     const int ring = a.pde_ring;
     const float h = (float)a.cell_h;
@@ -1750,7 +1667,7 @@ MOR_OUTLINE void phase_pde_count(const FramePtrs& a, int cta, int G) {
 // Detection flags (cpp:580-606) and the N-frame consistency chain: checkMovingClusterChain (cpp:478-514),
 // recurseFindClusterChain (cpp:415-453), pushCentroid (cpp:455-476). corrs_vec / res_vec are device-resident ring
 // buffers; a correspondence map is stored as match_of_prev[].
-MOR_OUTLINE void phase_chain(const FramePtrs& a) {
+__device__ __forceinline__ void phase_chain(const FramePtrs& a) {
     const int K = a.counts[MOR_CNT_K], Kp = a.p_counts[MOR_CNT_K], M = a.counts[MOR_CNT_M];
     const int D = a.ring_depth, kmax = a.kmax;
     TrackState* ts = a.track;
@@ -2146,7 +2063,7 @@ __device__ __forceinline__ void frame_epilogue(const FramePtrs& a, int G) {
     for (int t = threadIdx.x; t < a.tiles_pts; t += kT) a.st_out[t] = 0ull;
     if (threadIdx.x == 0) {
         Scratch* sc = a.scratch;
-        sc->bar = 0u; sc->blocks_done = 0; sc->n_cells = 0; sc->n_roots = 0; sc->n_light = 0; sc->n_heavy = 0; sc->n_sorted = 0; sc->tail_match = 0u; sc->tail_chain = 0u; sc->ticket_light = 0; sc->ticket_heavy = 0; sc->err_early = 0;
+        sc->bar = 0u; sc->blocks_done = 0; sc->n_cells = 0; sc->n_roots = 0; sc->n_light = 0; sc->n_heavy = 0; sc->n_sorted = 0; sc->tail_match = 0u; sc->tail_chain = 0u; sc->err_early = 0;
         if (LK) sc->n_sel = 0;
         sc->ticket_ingest = 0; sc->ticket_cells = 0;  // voxel ground modes (k_ground_partition leaves its tile tickets behind)
         for (int q = 0; q < 3; q++) { sc->box_inv_min[q] = 0u; sc->box_max[q] = 0u; }
@@ -2156,14 +2073,9 @@ __device__ __forceinline__ void frame_epilogue(const FramePtrs& a, int G) {
 // ===================================================================================== the frame kernel
 enum Phase { PH_INGEST = 0, PH_CELLS, PH_LINK, PH_TEST, PH_JUMP, PH_CROSS, PH_ROOTS, PH_SELECT, PH_STATS, PH_MOVING, PH_FILTER, PH__COUNT };
 
-struct FrameShared {
-    unsigned long long mbar;
-    FilterShared filter;
-};
-
 template <int PH, bool LK>
-__device__ __forceinline__ void run_phase(const FramePtrs& a, int cta, int G, FrameShared& sh, unsigned long long* dyn, unsigned& parity, GroupBarrier& bar) {
-    if (PH == PH_INGEST) { if (a.skip_ingest) phase_bin_cloud(a, cta, G); else phase_ingest(a, cta, G, dyn, &sh.mbar, parity); }
+__device__ __forceinline__ void run_phase(const FramePtrs& a, int cta, int G, FilterShared& sh, unsigned long long* dyn, GroupBarrier& bar) {
+    if (PH == PH_INGEST) { if (a.skip_ingest) phase_bin_cloud(a, cta, G); else phase_ingest(a, cta, G); }
     if (PH == PH_CELLS) phase_cells(a, cta, G);
     if (PH == PH_LINK) phase_link(a, cta, G, dyn);
     if (PH == PH_TEST) phase_test(a, cta, G);
@@ -2188,13 +2100,13 @@ __device__ __forceinline__ void run_phase(const FramePtrs& a, int cta, int G, Fr
         if (a.two_frames) { if (a.method == 2) phase_lattice_count<LK>(a, cta, G); else phase_pde_count(a, cta, G); }
         if (group_last_arrival(&a.scratch->tail_chain, (unsigned)G)) phase_chain_tail(a);
     }
-    if (PH == PH_FILTER) phase_filter<LK>(a, cta, G, sh.filter, dyn, bar);
+    if (PH == PH_FILTER) phase_filter<LK>(a, cta, G, sh, dyn, bar);
 }
 
 
 template <int PH, bool LK>
-__device__ __forceinline__ void frame_step(const FramePtrs& a, int cta, int G, FrameShared& sh, unsigned long long* dyn, unsigned& parity, GroupBarrier& bar) {
-    run_phase<PH, LK>(a, cta, G, sh, dyn, parity, bar);
+__device__ __forceinline__ void frame_step(const FramePtrs& a, int cta, int G, FilterShared& sh, unsigned long long* dyn, GroupBarrier& bar) {
+    run_phase<PH, LK>(a, cta, G, sh, dyn, bar);
 #ifdef MOR_CTA_TRACE
     __syncthreads();
     if (threadIdx.x == 0 && cta < 256) a.cta_trace[PH * 256 + cta] = global_ns();
@@ -2204,21 +2116,21 @@ __device__ __forceinline__ void frame_step(const FramePtrs& a, int cta, int G, F
 }
 
 template <bool LK>
-__device__ __forceinline__ void frame_body(const FramePtrs& a, int cta, int G, FrameShared& sh, unsigned long long* dyn, unsigned& parity) {
+__device__ __forceinline__ void frame_body(const FramePtrs& a, int cta, int G, FilterShared& sh, unsigned long long* dyn) {
     GroupBarrier bar{&a.scratch->bar, 0u, (unsigned)G};
     if (cta == 0 && threadIdx.x == 0) a.phase_ts[0] = global_ns();
-    frame_step<PH_INGEST, LK>(a, cta, G, sh, dyn, parity, bar);
+    frame_step<PH_INGEST, LK>(a, cta, G, sh, dyn, bar);
     load_frame_vars(a);
-    frame_step<PH_CELLS, LK>(a, cta, G, sh, dyn, parity, bar);
-    frame_step<PH_LINK, LK>(a, cta, G, sh, dyn, parity, bar);
-    frame_step<PH_TEST, LK>(a, cta, G, sh, dyn, parity, bar);
-    frame_step<PH_JUMP, LK>(a, cta, G, sh, dyn, parity, bar);
-    frame_step<PH_CROSS, LK>(a, cta, G, sh, dyn, parity, bar);
-    frame_step<PH_ROOTS, LK>(a, cta, G, sh, dyn, parity, bar);
-    frame_step<PH_SELECT, LK>(a, cta, G, sh, dyn, parity, bar);
-    frame_step<PH_STATS, LK>(a, cta, G, sh, dyn, parity, bar);
-    frame_step<PH_MOVING, LK>(a, cta, G, sh, dyn, parity, bar);
-    frame_step<PH_FILTER, LK>(a, cta, G, sh, dyn, parity, bar);
+    frame_step<PH_CELLS, LK>(a, cta, G, sh, dyn, bar);
+    frame_step<PH_LINK, LK>(a, cta, G, sh, dyn, bar);
+    frame_step<PH_TEST, LK>(a, cta, G, sh, dyn, bar);
+    frame_step<PH_JUMP, LK>(a, cta, G, sh, dyn, bar);
+    frame_step<PH_CROSS, LK>(a, cta, G, sh, dyn, bar);
+    frame_step<PH_ROOTS, LK>(a, cta, G, sh, dyn, bar);
+    frame_step<PH_SELECT, LK>(a, cta, G, sh, dyn, bar);
+    frame_step<PH_STATS, LK>(a, cta, G, sh, dyn, bar);
+    frame_step<PH_MOVING, LK>(a, cta, G, sh, dyn, bar);
+    frame_step<PH_FILTER, LK>(a, cta, G, sh, dyn, bar);
     frame_epilogue<LK>(a, G);
 }
 
@@ -2232,7 +2144,7 @@ __device__ __forceinline__ void frame_body(const FramePtrs& a, int cta, int G, F
 // phase resolves each point's cluster from: slead, hook, rmin, cid_of_pos; scid, which it writes) on the host side
 // (mor_b200.cu, fill_frame). The front half's other per-frame arrays (cells, pair lists, rsize, root_list, cid_of_root)
 // are read by no back half.
-// Four instantiations of the same two bodies, picked per handle by mor_b200.cu (pipe_kernel):
+// Four instantiations of the same two bodies, picked per handle by mor_b200.cu (pipe_variant):
 //  - k_frame_pipe: crop ground mode, method 2.
 //  - k_frame_pipe_ground (GROUND): voxel ground modes. Frame f+1's nine ground launches (mor_ground.cuh) run on the stream
 //    before this launch, i.e. after the launch that ran f's front half and before f's back half. What they write, against
@@ -2266,11 +2178,11 @@ __device__ __forceinline__ void pipe_stamp(const FramePtrs& a, int cta, int word
 }
 
 template <bool GROUND, bool PDE, bool LK>
-__device__ __forceinline__ void front_body(const FramePtrs& a, int cta, int G, FrameShared& sh, unsigned long long* dyn, unsigned& parity) {
+__device__ __forceinline__ void front_body(const FramePtrs& a, int cta, int G, unsigned long long* dyn) {
     GroupBarrier bar{&a.scratch->bar, 0u, (unsigned)G};
     pipe_stamp(a, cta, TS_FRONT);
     if (GROUND) phase_bin_cloud(a, cta, G, /*housekeep=*/false);
-    else phase_ingest(a, cta, G, dyn, &sh.mbar, parity, /*housekeep=*/false);
+    else phase_ingest(a, cta, G, /*housekeep=*/false);
     bar.sync(); pipe_stamp(a, cta, TS_FRONT + 1);
     load_frame_vars(a);
     phase_cells(a, cta, G); bar.sync(); pipe_stamp(a, cta, TS_FRONT + 2);
@@ -2303,7 +2215,7 @@ __device__ __forceinline__ void front_body(const FramePtrs& a, int cta, int G, F
         a.phase_ts[TS_FRONT + 8] = global_ns();
         Scratch* sc = a.scratch;
         sc->bar = 0u; sc->blocks_done = 0; sc->n_cells = 0; sc->n_roots = 0; sc->n_light = 0; sc->n_heavy = 0; sc->n_sorted = 0; sc->tail_centroids = 0u;
-        sc->ticket_light = 0; sc->ticket_heavy = 0; sc->err_early = 0;
+        sc->err_early = 0;
         if (LK) sc->n_sel = 0;
         if (GROUND) sc->ticket_ingest = 0;  // (drawn by k_ground_partition; frame_epilogue resets it in one kernel per frame)
     }
@@ -2312,7 +2224,7 @@ __device__ __forceinline__ void front_body(const FramePtrs& a, int cta, int G, F
 // (GROUND does not change the back half; it keeps every kernel's instantiations of the two bodies its own, so that their
 // static shared variables stay local to one kernel and k_frame_pipe's shared layout is what it was before the variants)
 template <bool GROUND, bool PDE, bool LK>
-__device__ __forceinline__ void back_body(const FramePtrs& a, int cta, int G, FrameShared& sh, unsigned long long* dyn) {
+__device__ __forceinline__ void back_body(const FramePtrs& a, int cta, int G, FilterShared& sh, unsigned long long* dyn) {
     GroupBarrier bar{&a.scratch->bar_back, 0u, (unsigned)G};
     if (threadIdx.x == 0) {  // (the cell count belongs to the front half, which is busy with the next frame)
         FrameVars& v = frame_vars();
@@ -2334,7 +2246,7 @@ __device__ __forceinline__ void back_body(const FramePtrs& a, int cta, int G, Fr
         for (int i = cta * kT + threadIdx.x; i < n_cells; i += G * kT)
             *reinterpret_cast<uint4*>(a.table + a.cell_list[i]) = make_uint4(0u, 0u, 0u, 0u);
     }
-    phase_filter<LK>(a, cta, G, sh.filter, dyn, bar, /*cleanup=*/false);
+    phase_filter<LK>(a, cta, G, sh, dyn, bar, /*cleanup=*/false);
     __shared__ int s_last_back;
     __syncthreads();
     if (threadIdx.x == 0) {
@@ -2357,27 +2269,16 @@ __device__ __forceinline__ void back_body(const FramePtrs& a, int cta, int G, Fr
 // every other handle, with no trace of them (mor_b200.cu picks the instantiation per handle).
 //
 // Front half of `f` on the CTAs [0, Gf), back half of `b` on the rest; Gf = gridDim.x: front only, Gf = 0: back only.
-template <bool LK>
-__global__ void __launch_bounds__(kT, 1) k_frame_pipe(const __grid_constant__ FramePtrs f, const __grid_constant__ FramePtrs b, int Gf) {
-    extern __shared__ __align__(128) unsigned long long dyn[];
-    __shared__ FrameShared sh;
-    if (threadIdx.x == 0) mbar_init(&sh.mbar, 1);
-    __syncthreads();
-    unsigned parity = 0;
-    if ((int)blockIdx.x < Gf) front_body<false, false, LK>(f, blockIdx.x, Gf, sh, dyn, parity);
-    else back_body<false, false, LK>(b, (int)blockIdx.x - Gf, (int)gridDim.x - Gf, sh, dyn);
-}
-
-// The other configurations: the same launch with the variants of the two bodies described above.
 template <bool GROUND, bool PDE, bool LK>
 __device__ __forceinline__ void frame_pipe_variant(const FramePtrs& f, const FramePtrs& b, int Gf) {
     extern __shared__ __align__(128) unsigned long long dyn[];
-    __shared__ FrameShared sh;
-    if (threadIdx.x == 0) mbar_init(&sh.mbar, 1);
-    __syncthreads();
-    unsigned parity = 0;
-    if ((int)blockIdx.x < Gf) front_body<GROUND, PDE, LK>(f, blockIdx.x, Gf, sh, dyn, parity);
+    __shared__ FilterShared sh;
+    if ((int)blockIdx.x < Gf) front_body<GROUND, PDE, LK>(f, blockIdx.x, Gf, dyn);
     else back_body<GROUND, PDE, LK>(b, (int)blockIdx.x - Gf, (int)gridDim.x - Gf, sh, dyn);
+}
+template <bool LK>
+__global__ void __launch_bounds__(kT, 1) k_frame_pipe(const __grid_constant__ FramePtrs f, const __grid_constant__ FramePtrs b, int Gf) {
+    frame_pipe_variant<false, false, LK>(f, b, Gf);
 }
 template <bool LK>
 __global__ void __launch_bounds__(kT, 1) k_frame_pipe_ground(const __grid_constant__ FramePtrs f, const __grid_constant__ FramePtrs b, int Gf) {
@@ -2396,11 +2297,8 @@ __global__ void __launch_bounds__(kT, 1) k_frame_pipe_ground_pde(const __grid_co
 template <bool LK>
 __global__ void __launch_bounds__(kT, 1) k_frame(const __grid_constant__ FramePtrs a) {
     extern __shared__ __align__(128) unsigned long long dyn[];
-    __shared__ FrameShared sh;
-    if (threadIdx.x == 0) mbar_init(&sh.mbar, 1);
-    __syncthreads();
-    unsigned parity = 0;
-    frame_body<LK>(a, blockIdx.x, gridDim.x, sh, dyn, parity);
+    __shared__ FilterShared sh;
+    frame_body<LK>(a, blockIdx.x, gridDim.x, sh, dyn);
 }
 
 // S sequences per launch: grid = groups x G CTAs; group g steps sequences g, g + groups, ... (each through all
@@ -2408,25 +2306,19 @@ __global__ void __launch_bounds__(kT, 1) k_frame(const __grid_constant__ FramePt
 template <bool LK>
 __global__ void __launch_bounds__(kT, 1) k_frame_batch(const FramePtrs* __restrict__ P, int S, int G) {
     extern __shared__ __align__(128) unsigned long long dyn[];
-    __shared__ FrameShared sh;
+    __shared__ FilterShared sh;
     const int group = blockIdx.x / G, cta = blockIdx.x % G, groups = gridDim.x / G;
-    if (threadIdx.x == 0) mbar_init(&sh.mbar, 1);
-    __syncthreads();
-    unsigned parity = 0;
-    for (int seq = group; seq < S; seq += groups) frame_body<LK>(P[seq], cta, G, sh, dyn, parity);
+    for (int seq = group; seq < S; seq += groups) frame_body<LK>(P[seq], cta, G, sh, dyn);
 }
 
 // One phase per launch (per-phase timing; the kernel boundary is the barrier). Same grid, same striding.
 template <int PH, bool LK>
 __global__ void __launch_bounds__(kT, 1) k_phase(const __grid_constant__ FramePtrs a) {
     extern __shared__ __align__(128) unsigned long long dyn[];
-    __shared__ FrameShared sh;
-    if (threadIdx.x == 0) mbar_init(&sh.mbar, 1);
-    __syncthreads();
-    unsigned parity = 0;
+    __shared__ FilterShared sh;
     GroupBarrier bar{&a.scratch->bar, 0u, gridDim.x};  // (the large-K steps of select, match and filter)
     if (PH != PH_INGEST) load_frame_vars(a);
-    run_phase<PH, LK>(a, blockIdx.x, gridDim.x, sh, dyn, parity, bar);
+    run_phase<PH, LK>(a, blockIdx.x, gridDim.x, sh, dyn, bar);
     if (PH == PH_FILTER) frame_epilogue<LK>(a, gridDim.x);
     if (LK && (PH == PH_SELECT || PH == PH_STATS)) {  // last CTA out: the barrier back to zero for the next launch
         __shared__ int s_last;

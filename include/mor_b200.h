@@ -138,7 +138,8 @@ int mor_sync(mor_handle* h);
  * d_data[s] / d_out[s] are device pointers (d_out[s] must hold n[s] records), poses7 = S x 7 doubles. Asynchronous on
  * hs[0]'s stream; mor_sync / mor_tap on any of the handles waits for it. With output records (mor_set_output_records,
  * which all handles must agree on, else MOR_ERR_ARG) d_out[s] must hold n[s] * point_step bytes, S <= 65535, and d_data[s]
- * must stay untouched until the step has completed. */
+ * must stay untouched until the step has completed. Every rule is checked for every sequence before anything is
+ * enqueued: a refused step changes no handle. */
 int mor_batch_step_device(mor_handle* const* hs, uint32_t S, const void* const* d_data, const uint32_t* n,
                           uint32_t point_step, uint32_t off_x, uint32_t off_y, uint32_t off_z, uint32_t off_i,
                           const double* poses7, void* const* d_out);

@@ -202,6 +202,63 @@ def test_batched_step_matches_oracle_per_sequence(product, oracle, cfg_dir):
         product.device_free(0, p)
 
 
+def test_refused_batched_step_launches_nothing(product, oracle, cfg_dir):
+    """A lockstep batched step that a later sequence's frame refuses (n > max_points) launches nothing, not even the
+    pending back half of an earlier, pipelined sequence; the step after it equals the oracle in every sequence."""
+    import ctypes as C
+    from dynamicslamtool_b200 import MorError, SequenceBatch, Synth
+    cfg = cfg_dir / "MOR_config.txt"
+    S = 3
+    syn = [Synth(1, 50 + s) for s in range(S)]
+    maxp = syn[0].max_points
+    gpus = [MovingObjectRemoval(cfg, 4, 3, binding=product, max_points=maxp) for _ in range(S)]
+    orcs = [MovingObjectRemoval(cfg, 4, 3, binding=oracle) for _ in range(S)]
+    gpus[0].set_pipelining(True)
+    d_in, d_out = [], []
+    for s in range(S):
+        a, b = C.c_void_p(), C.c_void_p()
+        assert product.device_alloc(0, (maxp + 1) * 16, C.byref(a)) == 0 and product.device_alloc(0, maxp * 32, C.byref(b)) == 0
+        d_in.append(a); d_out.append(b)
+    try:
+        for s in range(S):  # frame 0 alone; sequence 0's back half stays pending (pipelined push, filter that asks for nothing)
+            pts, pose = syn[s].frame(0)
+            assert product.device_upload(0, d_in[s], pts.ctypes.data_as(C.c_void_p), pts.nbytes) == 0
+            gpus[s].push_device(d_in[s].value, len(pts), pose)
+            if s == 0:
+                gpus[s].filter_device(None, 0, want_count=False)
+            else:
+                gpus[s].filter_device(d_out[s].value, maxp)
+            orcs[s].push_raw_cloud_and_pose(pts, pose)
+            orcs[s].filter_cloud()
+        data = [syn[s].frame(1) for s in range(S)]
+        big = np.zeros((maxp + 1, 4), np.float32)
+        big[: len(data[2][0])] = data[2][0]
+        assert product.device_upload(0, d_in[2], big.ctypes.data_as(C.c_void_p), big.nbytes) == 0
+        launches = [g.launch_count() for g in gpus]
+        with pytest.raises(MorError) as e:
+            SequenceBatch(gpus).step_device([p.value for p in d_in], [len(data[0][0]), len(data[1][0]), maxp + 1],
+                                            [d[1] for d in data], [p.value for p in d_out])
+        assert e.value.status == 6
+        assert [g.launch_count() for g in gpus] == launches
+        for s in range(S):
+            pts = data[s][0]
+            assert product.device_upload(0, d_in[s], pts.ctypes.data_as(C.c_void_p), pts.nbytes) == 0
+        SequenceBatch(gpus).step_device([p.value for p in d_in], [len(d[0]) for d in data], [d[1] for d in data], [p.value for p in d_out])
+        for s in range(S):
+            orcs[s].push_raw_cloud_and_pose(*data[s])
+            oo = orcs[s].filter_cloud().copy()
+            gpus[s].sync()
+            n_out = gpus[s].counts()["NOUT"]
+            og = np.empty((n_out, 8), np.float32)
+            if n_out:
+                assert product.device_download(0, og.ctypes.data_as(C.c_void_p), d_out[s], n_out * 32) == 0
+            bad = compare_frame(gpus[s], orcs[s], og, oo)
+            assert not bad, f"sequence {s}: {bad}"
+    finally:
+        for p in d_in + d_out:
+            product.device_free(0, p)
+
+
 @pytest.mark.parametrize("n_bad,n_good", [(1, 0), (2, 1), (3, 5), (6, 2)])
 def test_confidence_parameters(product, oracle, tmp_path, n_bad, n_good):
     """moving_confidence / static_confidence other than the node's 4, 3 (external_sync_test.cpp:37): ring-buffer depth,
